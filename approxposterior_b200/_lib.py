@@ -78,6 +78,7 @@ _SIGNATURES = {
     "apgp_get_chol": (C.c_int, [C.c_void_p, C.c_void_p]),
     "apgp_set_variant": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_set_group": (C.c_int, [C.c_void_p, C.c_int]),
+    "apgp_set_var_engine": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_set_predict_few": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_debug_exp_neg": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "apgp_debug_exp_neg256": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),

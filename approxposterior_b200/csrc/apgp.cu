@@ -56,6 +56,8 @@ struct apgp_handle {
   int variant_eff = 2;   // tiling the current factorisation was packed for
   int group = -1;        // CTAs per query tile in the variance kernel: 0 = one tile per CTA, -1 = automatic, G = fixed
   bool predict_few = true;   // calls of at most PREDICT_FEW_MAX queries: one CTA per query (APGP_PREDICT_FEW=0: tiled kernels)
+  bool var_i8 = true;        // variance engine of grouped calls: int8 tensor cores where they apply (predict_i8.cu), else DMMA
+  bool i8_packed = false;    // LinvI8 / i8scale hold the current factorisation's digits
   bool has_training = false, has_hyper = false, factored = false;
   double mean = 0, amp = 1, white_noise = -12;
   double log_metric[APGP_MAX_DIM];
@@ -75,7 +77,8 @@ struct apgp_handle {
   DevBuf o_in, o_x, o_f, o_stats;      // device optimiser staging
   DevBuf g_arrive, g_part, g_plan;     // grouped variance kernel: barrier counters, partial sums, work-split tables
   DevBuf few_ws;                       // few-query predict: per-split partial sums, means, arrival counters
-  int plan_Npad = -1, plan_G = -1, plan_d = -1;   // what g_plan currently holds
+  int plan_Npad = -1, plan_G = -1, plan_d = -1, plan_i8 = -1;   // what g_plan currently holds
+  DevBuf LinvI8, i8scale;              // int8 engine operands (pack_linv_i8)
 };
 
 namespace {
@@ -126,6 +129,7 @@ int apgp_create(apgp_handle** out, int device) {
   const char* gv = getenv("APGP_PREDICT_GROUP");
   if (gv) h->group = atoi(gv);
   if (const char* fv = getenv("APGP_PREDICT_FEW")) h->predict_few = atoi(fv) != 0;
+  if (const char* ev = getenv("APGP_PREDICT_VAR_ENGINE")) h->var_i8 = strcmp(ev, "dmma") != 0;
   *out = h;
   return APGP_OK;
 }
@@ -137,7 +141,7 @@ int apgp_destroy(apgp_handle* h) {
   DevBuf* bufs[] = {&h->X, &h->y, &h->K, &h->Dinv, &h->r, &h->Linv, &h->work, &h->scal, &h->info, &h->hyper, &h->Xs,
                     &h->alphaA, &h->alpha, &h->LinvF, &h->scratch, &h->qscale, &h->stage_in, &h->stage_out, &h->ap_k, &h->ap_l, &h->ap_u, &h->ap_x, &h->bK,
                     &h->bDinv, &h->br, &h->bscal, &h->binfo, &h->bhyper, &h->bll, &h->bgrad, &h->s_p0, &h->s_chain, &h->s_logp,
-                    &h->s_blob, &h->s_nacc, &h->s_ri, &h->s_rz, &h->s_rr, &h->s_rl, &h->o_in, &h->o_x, &h->o_f, &h->o_stats, &h->g_arrive, &h->g_part, &h->g_plan, &h->few_ws, &h->gws, &h->ac_part, &h->ac_f, &h->ac_stage, &h->c_hdr, &h->c_send, &h->c_recv};
+                    &h->s_blob, &h->s_nacc, &h->s_ri, &h->s_rz, &h->s_rr, &h->s_rl, &h->o_in, &h->o_x, &h->o_f, &h->o_stats, &h->g_arrive, &h->g_part, &h->g_plan, &h->few_ws, &h->LinvI8, &h->i8scale, &h->gws, &h->ac_part, &h->ac_f, &h->ac_stage, &h->c_hdr, &h->c_send, &h->c_recv};
   for (DevBuf* b : bufs) b->release();
   if (h->comm) comm_destroy(h->comm);
   if (h->pin) cudaFreeHost(h->pin);
@@ -161,11 +165,13 @@ int apgp_reset(apgp_handle* h) {
   h->N = h->d = h->Np = h->Npad = 0;
   h->has_training = h->has_hyper = h->factored = false;
   h->mean = 0; h->amp = 1; h->white_noise = -12; h->logdet = 0; h->loglik = 0;
-  h->plan_Npad = h->plan_G = h->plan_d = -1;
-  h->variant = 2; h->variant_eff = 2; h->group = -1; h->predict_few = true;   // tuning knobs back to their defaults (as apgp_create)
+  h->plan_Npad = h->plan_G = h->plan_d = h->plan_i8 = -1;
+  h->i8_packed = false;
+  h->variant = 2; h->variant_eff = 2; h->group = -1; h->predict_few = true; h->var_i8 = true;   // tuning knobs back to their defaults (as apgp_create)
   if (const char* v = getenv("APGP_PREDICT_VARIANT")) { int vv = atoi(v); h->variant = (vv >= 0 && vv <= 2) ? vv : 2; }
   if (const char* gv = getenv("APGP_PREDICT_GROUP")) h->group = atoi(gv);
   if (const char* fv = getenv("APGP_PREDICT_FEW")) h->predict_few = atoi(fv) != 0;
+  if (const char* ev = getenv("APGP_PREDICT_VAR_ENGINE")) h->var_i8 = strcmp(ev, "dmma") != 0;
   if (h->comm) { comm_destroy(h->comm); h->comm = nullptr; h->comm_rank = 0; h->comm_world = 1; }
   return APGP_OK;
 }
@@ -194,6 +200,12 @@ long long apgp_launch_count(const apgp_handle* h) { return h ? h->launches : 0; 
 int apgp_set_group(apgp_handle* h, int group) {
   if (!h || group < -1 || group > 64) return fail(APGP_ERR_ARG, "apgp_set_group");
   h->group = group;
+  return APGP_OK;
+}
+
+int apgp_set_var_engine(apgp_handle* h, int engine) {
+  if (!h || (engine != APGP_VAR_ENGINE_DMMA && engine != APGP_VAR_ENGINE_I8)) return fail(APGP_ERR_ARG, "apgp_set_var_engine");
+  h->var_i8 = engine == APGP_VAR_ENGINE_I8;
   return APGP_OK;
 }
 
@@ -234,6 +246,21 @@ int apgp_set_hyper(apgp_handle* h, double mean, double amp, const double* log_me
   return APGP_OK;
 }
 
+// int8 variance engine: grouped calls from Npad = I8_MIN_NPAD, where it measured 1.5x (N = 1024) to 1.9x (N = 8192)
+// faster than the DMMA kernel (profiles/r03_var_engine.jsonl); smaller N, mostly not grouped, stays on DMMA
+constexpr int I8_MIN_NPAD = 1024;
+static bool i8_applies(const apgp_handle* h) {
+  return h->var_i8 && h->group != 0 && h->variant_eff == 2 && h->Npad >= I8_MIN_NPAD && predict_i8_fits(h->Npad, h->d);
+}
+static int pack_i8_operands(apgp_handle* h, cudaStream_t st, int* nl) {
+  CUI(h->LinvI8.reserve(linv_i8_bytes(h->Npad)));
+  CUI(h->i8scale.reserve((size_t)h->Npad * 8));
+  CUI(launch_pack_linv_i8(h->Linv.as<double>(), h->Np, h->N, h->Npad, h->amp, h->LinvI8.as<unsigned char>(),
+                          h->i8scale.as<double>(), st)); ++*nl;
+  h->i8_packed = true;
+  return APGP_OK;
+}
+
 static int pack_predict_operands(apgp_handle* h, int* nl) {
   const int N = h->N, d = h->d, Np = h->Np;
   const int BN = predict_variant_bn(h->variant_eff);
@@ -244,6 +271,8 @@ static int pack_predict_operands(apgp_handle* h, int* nl) {
   CU(cudaMemcpyAsync(h->qscale.p, qs, d * 8, cudaMemcpyHostToDevice, h->stream));
   CUI(launch_pack_xs(h->X.as<double>(), N, d, h->Npad, h->qscale.as<double>(), h->Xs.as<double>(), h->stream)); ++*nl;
   CUI(launch_pack_linv(h->Linv.as<double>(), Np, N, h->Npad, BN, h->amp, h->LinvF.as<double>(), h->stream)); ++*nl;
+  h->i8_packed = false;
+  if (i8_applies(h)) { int st_ = pack_i8_operands(h, h->stream, nl); if (st_ != APGP_OK) return st_; }
   return APGP_OK;
 }
 
@@ -375,22 +404,31 @@ static int predict_launch(apgp_handle* h, PredictParams& p, int want_var, cudaSt
     CUI(launch_predict_few(p, h->Linv.as<double>(), h->Np, h->few_ws.p, st, nl));
     return APGP_OK;
   }
-  const int G = (h->group == 0) ? 1 : predict_group_size(h->Npad, h->num_sms, h->variant_eff, h->group, d, Qplan);
+  const bool i8 = i8_applies(h);
+  int G = (h->group == 0) ? 1 : predict_group_size(h->Npad, h->num_sms, h->variant_eff, h->group, d, Qplan, i8);
+  if (i8 && G > 1) {
+    // packed with the factorisation; here only when the engine was switched to i8 after it
+    if (!h->i8_packed) { int st_ = pack_i8_operands(h, st, nl); if (st_ != APGP_OK) return st_; }
+    p.LinvI8 = h->LinvI8.as<unsigned char>(); p.i8scale = h->i8scale.as<double>();
+  } else if (i8) {
+    G = (h->group == 0) ? 1 : predict_group_size(h->Npad, h->num_sms, h->variant_eff, h->group, d, Qplan);
+  }
+  const bool use_i8 = i8 && p.LinvI8 != nullptr;
   if (G > 1) {
-    CUI(h->scratch.reserve(predict_group_scratch_bytes(h->Npad, h->num_sms, G)));
+    CUI(h->scratch.reserve(predict_group_scratch_bytes(h->Npad, h->num_sms, G, use_i8)));
     CUI(h->g_arrive.reserve(sizeof(int) * ((h->num_sms + G - 1) / G)));
     CUI(h->g_part.reserve(predict_group_part_bytes(h->Npad, h->num_sms, G)));
     CUI(h->g_plan.reserve(4 * 128 * sizeof(int)));
     p.scratch = h->scratch.as<double>();
     p.grp_arrive = h->g_arrive.as<int>(); p.grp_part = h->g_part.as<double>(); p.grp_plan = h->g_plan.as<int>();
-    if (h->plan_Npad != h->Npad || h->plan_G != G || h->plan_d != d) {      // re-plan only when the shape changes
+    if (h->plan_Npad != h->Npad || h->plan_G != G || h->plan_d != d || h->plan_i8 != (int)use_i8) {   // re-plan on a new shape
       int tab[4 * 128];
-      predict_group_plan(h->Npad, h->num_sms, G, d, tab);
+      predict_group_plan(h->Npad, h->num_sms, G, d, tab, use_i8);
       CU(cudaMemcpyAsync(h->g_plan.p, tab, sizeof(tab), cudaMemcpyHostToDevice, st));
       CU(cudaStreamSynchronize(st));
-      h->plan_Npad = h->Npad; h->plan_G = G; h->plan_d = d;
+      h->plan_Npad = h->Npad; h->plan_G = G; h->plan_d = d; h->plan_i8 = (int)use_i8;
     }
-    const int ge = launch_predict_var_grouped(p, h->num_sms, G, st, nl);
+    const int ge = use_i8 ? launch_predict_var_i8(p, h->num_sms, G, st, nl) : launch_predict_var_grouped(p, h->num_sms, G, st, nl);
     if (ge == (int)cudaErrorCooperativeLaunchTooLarge) {
       // the GPU is shared (fewer SMs free than the grid needs for its spin barriers): one tile per CTA instead
       (void)cudaGetLastError();

@@ -44,6 +44,8 @@ struct PredictParams {
   int* grp_arrive;         // grouped kernel: [ngroups] arrival counters (zeroed per launch)
   double* grp_part;        // grouped kernel: [ngroups][2 (mu, ss)][2 buffers][Npad/64][256] per-block partial sums
   int* grp_plan;           // grouped kernel: work-split tables (plan_group_split), 4 x 128 ints
+  const unsigned char* LinvI8;   // int8 engine: digit planes of A * L^{-1} (predict_i8.cu)
+  const double* i8scale;   // int8 engine: [Npad] per-row scale of those digits
 };
 
 int predict_variant_bn(int variant);   // block-row height BN of the LinvF tiling used by a kernel variant
@@ -59,11 +61,18 @@ int launch_predict_mean(const PredictParams& p, int num_sms, cudaStream_t st, in
 size_t predict_scratch_bytes(int Npad, int num_sms, int variant);
 // grouped 256x64 kernel: G CTAs share one query tile so the K* panels in flight stay in L2 (predict.cu).
 // requested < 0: automatic choice; returns 1 when grouping is off / not applicable
-int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q);
-void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab /*[4*128]*/);
-size_t predict_group_scratch_bytes(int Npad, int num_sms, int G);
+// i8: plan for the int8 engine's 128-query tile (predict_i8.cu) instead of the DMMA kernel's 256-query tile
+int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q, bool i8 = false);
+void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab /*[4*128]*/, bool i8 = false);
+size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, bool i8 = false);
 size_t predict_group_part_bytes(int Npad, int num_sms, int G);
 int launch_predict_var_grouped(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches);
+// int8 tensor-core variance engine (grouped launch only): exact-integer split of the triangular product
+bool predict_i8_fits(int Npad, int d);
+size_t linv_i8_bytes(int Npad);
+int launch_pack_linv_i8(const double* Linv, int ld, int N, int Npad, double amp, unsigned char* out, double* rowscale,
+                        cudaStream_t st);
+int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches);
 int launch_pack_linv(const double* Linv, int ld, int N, int Npad, int BN, double amp, double* LinvF, cudaStream_t st);
 int launch_pack_xs(const double* X, int N, int d, int Npad, const double* qscale_dev, double* Xs, cudaStream_t st);
 

@@ -834,7 +834,9 @@ size_t predict_scratch_bytes(int Npad, int num_sms, int variant) {
 // of DMMA for the 256x64 tile); longest-first onto the least loaded rank.  Phase 1: building one 64-column block of
 // the panel costs (2d + 12)/64 of a unit (exp + distances on the same FP64 pipe); the blocks go, one by one, to the
 // rank with the least combined load, which also evens out what phase 2 could not.  Returns max load / mean load.
-double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1) {
+// i8: the int8 engine's unit is a 128-query tile on the int8 pipe, and its panel block costs the same FP64 exponentials
+// for half the queries, ~0.86 of its units at d = 5 (estimated from the DMMA rate and the int8 kernel's shared-memory bound)
+double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, bool i8 = false) {
   double load[64];
   for (int r = 0; r < gs; ++r) load[r] = 0.0;
   for (int ib = nblk - 1; ib >= 0; --ib) {
@@ -842,7 +844,7 @@ double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1) {
     for (int r = 1; r < gs; ++r) if (load[r] < load[best]) best = r;
     owner2[ib] = best; load[best] += ib + 1;
   }
-  const double c1 = (2.0 * d + 12.0) / 64.0;
+  const double c1 = (2.0 * d + 12.0) / 64.0 * (i8 ? 2.5 : 1.0);
   for (int cb = 0; cb < nblk; ++cb) {
     int best = 0;
     for (int r = 1; r < gs; ++r) if (load[r] < load[best]) best = r;
@@ -853,8 +855,9 @@ double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1) {
   return mx * gs / tot;
 }
 
-int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q) {
+int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q, bool i8) {
   if (variant != 2 || Npad / 64 > GROUP_MAX_BLOCKS) return 1;
+  const int BM = i8 ? 128 : 256, EB = i8 ? 7 : 8;      // queries per tile, panel bytes per (query, training point)
   // the grouped kernel carries 4.6 KB of static shared memory (ownership tables, kept means) on top of the one-tile
   // kernel's dynamic layout: from d = 28 the staged queries no longer fit beside the ring -> one tile per CTA
   if (VarCfg<256, 64, 4, 8>::smem_bytes(d) > 220 * 1024) return 1;
@@ -871,11 +874,11 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
     int Gmin = 1;
     if (Npad >= 1024) {
       Gmin = 2;
-      while (Gmin < 64 && (size_t)((num_sms + Gmin - 1) / Gmin) * 256 * Npad * 8 > ((size_t)80 << 20)) ++Gmin;
+      while (Gmin < 64 && (size_t)((num_sms + Gmin - 1) / Gmin) * BM * Npad * EB > ((size_t)80 << 20)) ++Gmin;
       for (int g = (Gmin / 2 > 2 ? Gmin / 2 : 2); g <= 64 && 2 * g <= nblk; ++g) {
-        double imb = plan_group_split(nblk, g, d, o2, o1);
+        double imb = plan_group_split(nblk, g, d, o2, o1, i8);
         const int tail = num_sms % g;               // a smaller last group: weigh its imbalance by its share of the SMs
-        if (tail > 1) imb = (imb * (num_sms - tail) + plan_group_split(nblk, tail, d, o2, o1) * tail) / num_sms;
+        if (tail > 1) imb = (imb * (num_sms - tail) + plan_group_split(nblk, tail, d, o2, o1, i8) * tail) / num_sms;
         else if (tail == 1) imb += 1.0 / num_sms;   // a lone CTA does whole tiles: fine, but it cannot share a panel
         const double score = imb + (g < Gmin ? 0.005 : 0.0) + 1e-4 * g;   // L2 fit is worth 0.5 % of balance; then small G
         if (score < bestS) { bestS = score; bestG = g; }
@@ -884,14 +887,14 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
     // (b) latency regime: a call with fewer query tiles than would fill half the GPU (optimiser rounds, refinement
     // passes: a handful of queries) spreads each tile over as many CTAs as the balance allows -- one 256-query tile
     // at N = 2048 is 32 block-rows for ONE CTA otherwise.
-    const long long ntiles = (Q + 255) / 256;
+    const long long ntiles = (Q + BM - 1) / BM;
     if (ntiles * bestG * 2 <= num_sms && nblk >= 4) {
       long long cap = num_sms / ntiles;
       if (cap > 64) cap = 64;
       if (cap > nblk / 2) cap = nblk / 2;
-      int fillG = bestG; double fillS = (bestG > 1) ? plan_group_split(nblk, bestG, d, o2, o1) / bestG : 1.0;
+      int fillG = bestG; double fillS = (bestG > 1) ? plan_group_split(nblk, bestG, d, o2, o1, i8) / bestG : 1.0;
       for (int g = bestG + 1; g <= (int)cap; ++g) {
-        const double t = plan_group_split(nblk, g, d, o2, o1) / g;      // time per tile ~ imbalance / ranks
+        const double t = plan_group_split(nblk, g, d, o2, o1, i8) / g;      // time per tile ~ imbalance / ranks
         if (t < fillS * 0.97) { fillS = t; fillG = g; }
       }
       bestG = fillG;
@@ -904,14 +907,14 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
   return G < 1 ? 1 : G;
 }
 // work-split tables for the kernel: [full group | last (smaller) group] x [phase-2 owner | phase-1 owner] x 128
-void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab) {
+void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab, bool i8) {
   const int nblk = Npad / 64, tail = num_sms % G;
   for (int i = 0; i < 4 * GROUP_MAX_BLOCKS; ++i) tab[i] = 0;
-  plan_group_split(nblk, G, d, tab, tab + GROUP_MAX_BLOCKS);
-  plan_group_split(nblk, tail > 0 ? tail : G, d, tab + 2 * GROUP_MAX_BLOCKS, tab + 3 * GROUP_MAX_BLOCKS);
+  plan_group_split(nblk, G, d, tab, tab + GROUP_MAX_BLOCKS, i8);
+  plan_group_split(nblk, tail > 0 ? tail : G, d, tab + 2 * GROUP_MAX_BLOCKS, tab + 3 * GROUP_MAX_BLOCKS, i8);
 }
-size_t predict_group_scratch_bytes(int Npad, int num_sms, int G) {
-  return (size_t)2 * ((num_sms + G - 1) / G) * 256 * Npad * 8;
+size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, bool i8) {
+  return (size_t)2 * ((num_sms + G - 1) / G) * (i8 ? 128 * 7 : 256 * 8) * Npad;
 }
 size_t predict_group_part_bytes(int Npad, int num_sms, int G) { return (size_t)((num_sms + G - 1) / G) * 4 * (Npad / 64) * 256 * 8; }
 

@@ -1,0 +1,458 @@
+// Grouped variance predict on the int8 tensor cores (tcgen05.mma.kind::i8): the triangular product
+// W = E . (A L^{-1})^T of predict.cu's grouped kernel, computed exactly in integer arithmetic (Ozaki split).
+//
+//   E[q,k] in [0,1]  -> fixed 2^-55 grid, 7 unsigned base-256 digits e_p (top digit <= 128)
+//   B = A L^{-1}     -> per row i a power-of-two scale 2^(ex_i - 55), 7 balanced signed digits b_r in [-127,127]
+//                       at the top, [-128,127] below
+//   W[q,i] = 2^(ex_i - 14) * sum_{s=0..7} 2^(-8 s) * acc_s,   acc_s = sum_k sum_{p+r=s} e_p[q,k] b_r[i,k]
+// The 34 digit products with p + r <= 7 are kept (the dropped levels 8..12 weigh 2^-64 and less against level 0).
+// Each level accumulates in int32 in tensor memory: <= 7 pairs x N x 255 x 128 < 2^31 for N <= 8192.  The integer sums are exact, so a
+// query's variance does not depend on the accumulation order, its position in the batch or the group size.
+//
+// Tile: 128 queries x 64 rows of B per block-row, K staged 64 at a time; 8 levels x 64 int32 columns fill the 512
+// TMEM columns.  Operands use the no-swizzle K-major canonical layout: 8-row x 16-byte core matrices, stored
+// [plane][k16 chunk][8-row group][8 rows][16 bytes].  Inside a 16-wide k chunk byte c holds k = c/4 + 4 (c%4): one
+// phase-1 thread builds k = l, l+4, l+8, l+12 (the DMMA kernel's order, so the mean is bit-identical) and stores
+// them as one 32-bit word.  A and B use the same permutation; an exact integer sum does not see it.
+//
+// Warps: 0-7 build the panel (phase 1) and run the per-block-row epilogue (tcgen05.ld, combine, W^2 row sums);
+// warp 8 lane 0 streams digit tiles with 1-D bulk TMA; warp 9 owns the TMEM allocation and its lane 0 issues MMAs.
+#include "apgp_internal.h"
+
+namespace apgp {
+
+namespace {
+
+constexpr int I8_BM = 128, I8_BN = 64, I8_BK = 64, I8_NST = 2, I8_GROUP_MAX_BLOCKS = 128;
+constexpr int I8_DIG = 7, I8_LEVELS = 8;
+constexpr int I8_A_STAGE = I8_DIG * I8_BM * I8_BK;      // bytes: 57344
+constexpr int I8_B_STAGE = I8_DIG * I8_BN * I8_BK;      // bytes: 28672
+constexpr int I8_STAGE = I8_A_STAGE + I8_B_STAGE;
+constexpr int I8_RING = I8_NST * I8_STAGE;
+constexpr int I8_NTHREADS = 10 * 32;
+
+size_t i8_smem_bytes(int d) { return (size_t)I8_RING + (size_t)d * I8_BM * 8 + 64 * 8 + 8 * 8 + 128; }
+
+__device__ __forceinline__ int ld_acquire_gpu_i8(const int* p) {
+  int v;
+  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+
+// no-swizzle K-major shared-memory matrix descriptor (sm_100: version bits 46-48 = 0b001)
+__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
+  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
+         (1ull << 46);
+}
+// kind::i8 instruction descriptor: D s32, A u8, B s8, both K-major, M = 128, N = 64
+constexpr uint32_t I8_IDESC = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(I8_BN >> 3) << 17) |
+                              ((uint32_t)(I8_BM >> 4) << 24);
+
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t acc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
+      :: "r"(tmem_d), "l"(da), "l"(db), "r"(I8_IDESC), "r"(acc) : "memory");
+}
+__device__ __forceinline__ void umma_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n"
+               :: "r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory"); }
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+               : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory"); }
+
+// round(e * 2^55) for 0 <= e <= 1 from the bits of e (integer pipe only); ties round up
+__device__ __forceinline__ unsigned long long fixed55(double e) {
+  const unsigned long long b = (unsigned long long)__double_as_longlong(e);
+  const int ex = (int)(b >> 52);
+  const int sh = 1023 - ex;
+  if (ex == 0 || sh > 56) return 0ull;
+  const unsigned long long m = ((b & 0xFFFFFFFFFFFFFull) | (1ull << 52)) << 3;
+  return sh <= 0 ? m : ((m >> (sh - 1)) + 1ull) >> 1;
+}
+// byte `byte` (0 = least significant) of four 64-bit values, packed into one word (value j -> byte j)
+__device__ __forceinline__ uint32_t gather_byte(const uint32_t (&lo)[4], const uint32_t (&hi)[4], int byte) {
+  const uint32_t* w = byte >= 4 ? hi : lo;
+  const uint32_t bb = (uint32_t)(byte & 3);
+  const uint32_t sel = bb | ((bb + 4u) << 4);
+  return __byte_perm(__byte_perm(w[0], w[1], sel), __byte_perm(w[2], w[3], sel), 0x5410);
+}
+
+__global__ void __launch_bounds__(I8_NTHREADS, 1)
+predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
+  constexpr int BM = I8_BM, BN = I8_BN, NCW = 8, NCONS = NCW * 32;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  unsigned char* ring = smem_raw;
+  double* qs = reinterpret_cast<double*>(smem_raw + I8_RING);   // [d][BM] scaled queries
+  double* etab = qs + (size_t)p.d * BM;                          // [64]
+  uint64_t* full = reinterpret_cast<uint64_t*>(etab + 64);
+  uint64_t* empty = full + I8_NST;
+  uint64_t* stagebar = empty + I8_NST;
+  uint64_t* accfull = stagebar + 1;
+  uint64_t* accempty = accfull + 1;
+  __shared__ int owner_s[I8_GROUP_MAX_BLOCKS];
+  __shared__ int myblk_s[I8_GROUP_MAX_BLOCKS];
+  __shared__ int nmine_s;
+  __shared__ double mu_keep[2][BM];
+  __shared__ double ss_s[BM];
+  __shared__ uint32_t tmem_base_s;
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int d = p.d, Npad = p.Npad, nblk = Npad / BN;
+  const int grp = blockIdx.x / G, rank = blockIdx.x % G;
+  const int gs = min(G, (int)gridDim.x - grp * G);
+  const long long ntiles = (p.Q + BM - 1) / BM;
+  const long long t_begin = (ntiles * (long long)(grp * G) + gridDim.x - 1) / gridDim.x;
+  const long long t_end = (ntiles * (long long)(grp * G + gs) + gridDim.x - 1) / gridDim.x;
+  const int sl0 = BM * rank / gs, sl1 = BM * (rank + 1) / gs;
+  int* arrive = p.grp_arrive + grp;
+  double* part_mu = p.grp_part + (size_t)grp * 4 * nblk * BM;       // [2 buffers][nblk][BM]
+  double* part_ss = part_mu + (size_t)2 * nblk * BM;                // [2 buffers][nblk][BM]
+  unsigned char* scratch8 = reinterpret_cast<unsigned char*>(p.scratch);
+
+  if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
+  if (tid == 0) {
+    for (int s = 0; s < I8_NST; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
+    mbar_init(stagebar, 1);
+    mbar_init(accfull, 1);
+    mbar_init(accempty, NCONS);
+    mbar_fence_init();
+  }
+  if (warp == 9) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n"
+                 :: "r"(smem_u32(&tmem_base_s)) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
+  }
+  {
+    const int* tab = p.grp_plan + (gs == G ? 0 : 2 * I8_GROUP_MAX_BLOCKS);
+    for (int e = tid; e < nblk; e += blockDim.x) owner_s[e] = tab[e];
+    if (tid == 0) {
+      int n = 0;
+      for (int e = 0; e < nblk; ++e) if (tab[I8_GROUP_MAX_BLOCKS + e] == rank) myblk_s[n++] = e;
+      nmine_s = n;
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const int nmine = nmine_s;
+  const uint32_t tmem = tmem_base_s;
+
+  uint32_t it = 0, nstaged = 0, nacc = 0;
+  int nbar = 0;
+
+  for (long long tile = t_begin; tile <= t_end; ++tile) {
+    const int b = (int)((tile - t_begin) & 1);
+    const long long q0 = tile * BM;
+    const bool live = tile < t_end;
+    unsigned char* panel = scratch8 + ((size_t)grp * 2 + b) * BM * (size_t)Npad * I8_DIG;
+
+    // ------------------------------------------------------------ phase 1: my column blocks of the digit panel
+    if (live && warp < NCW) {
+      for (int e = tid; e < d * BM; e += NCONS) {
+        int i = e / BM, m = e - i * BM;
+        long long q = q0 + m;
+        qs[e] = (q < p.Q) ? p.Xq[q * d + i] * p.qscale[i] : 0.0;
+      }
+      double* stg = reinterpret_cast<double*>(ring);
+      const int CAPB = min(8, (I8_RING / 8 / (d + 1)) / BN);
+      const int JCHT = CAPB * BN;
+      constexpr int R = BM / (8 * NCW);
+      const int l = lane & 3, row = lane >> 2;
+      for (int s0 = 0; s0 < nmine; s0 += CAPB) {
+        const int ns = min(CAPB, nmine - s0);
+        named_bar_sync(1, NCONS);
+        if (tid == 0) {
+          mbar_arrive_expect_tx(stagebar, (uint32_t)((d + 1) * ns * BN * 8));
+          for (int sl = 0; sl < ns; ++sl) {
+            const int j0 = myblk_s[s0 + sl] * BN;
+            for (int i = 0; i < d; ++i) bulk_g2s(stg + i * JCHT + sl * BN, p.Xs + (size_t)i * Npad + j0, BN * 8, stagebar);
+            bulk_g2s(stg + d * JCHT + sl * BN, p.alphaA + j0, BN * 8, stagebar);
+          }
+        }
+        mbar_wait(stagebar, nstaged & 1u);
+        ++nstaged;
+        for (int sl = 0; sl < ns; ++sl) {
+          const int cb = myblk_s[s0 + sl];
+          const double* al = stg + d * JCHT + sl * BN;
+          unsigned char* pstage = panel + (size_t)cb * I8_A_STAGE;
+          double macc[R] = {};
+          for (int jb = 0; jb < BN; jb += 16) {
+            const int jj = jb + l;
+            double s[R][4] = {};
+            for (int i = 0; i < d; ++i) {
+              const double* xr = stg + i * JCHT + sl * BN + jj;
+              const double x0 = xr[0], x1 = xr[4], x2 = xr[8], x3 = xr[12];
+#pragma unroll
+              for (int r = 0; r < R; ++r) {
+                const double qv = qs[i * BM + (warp + r * NCW) * 8 + row];
+                const double d0 = x0 - qv, d1 = x1 - qv, d2 = x2 - qv, d3 = x3 - qv;
+                s[r][0] = fma(d0, d0, s[r][0]); s[r][1] = fma(d1, d1, s[r][1]);
+                s[r][2] = fma(d2, d2, s[r][2]); s[r][3] = fma(d3, d3, s[r][3]);
+              }
+            }
+            const double a0 = al[jj], a1 = al[jj + 4], a2 = al[jj + 8], a3 = al[jj + 12];
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+              const int mg = warp + r * NCW;
+              double ev[4];
+              ev[0] = exp_neg(s[r][0], etab); ev[1] = exp_neg(s[r][1], etab);
+              ev[2] = exp_neg(s[r][2], etab); ev[3] = exp_neg(s[r][3], etab);
+              macc[r] = fma(ev[0], a0, macc[r]); macc[r] = fma(ev[1], a1, macc[r]);
+              macc[r] = fma(ev[2], a2, macc[r]); macc[r] = fma(ev[3], a3, macc[r]);
+              uint32_t lo[4], hi[4];
+#pragma unroll
+              for (int j = 0; j < 4; ++j) {
+                const unsigned long long v = fixed55(ev[j]);
+                lo[j] = (uint32_t)v; hi[j] = (uint32_t)(v >> 32);
+              }
+              uint32_t* dst = reinterpret_cast<uint32_t*>(pstage + ((size_t)(jb >> 4) * 16 + mg) * 128 + row * 16 + l * 4);
+#pragma unroll
+              for (int pl = 0; pl < I8_DIG; ++pl) dst[pl * (4 * 16 * 128 / 4)] = gather_byte(lo, hi, 6 - pl);
+            }
+          }
+#pragma unroll
+          for (int r = 0; r < R; ++r) {
+            double v = macc[r];
+            v += __shfl_xor_sync(0xffffffffu, v, 1);
+            v += __shfl_xor_sync(0xffffffffu, v, 2);
+            if (l == 0) part_mu[((size_t)b * nblk + cb) * BM + (warp + r * NCW) * 8 + row] = v;
+          }
+        }
+      }
+      __threadfence();
+    }
+    __syncthreads();
+
+    // ------------------------------------------------------------ group barrier (one per tile)
+    if (tid == 0) {
+      ++nbar;
+      __threadfence();
+      atomicAdd(arrive, 1);
+      const int target = nbar * gs;
+      while (ld_acquire_gpu_i8(arrive) < target) __nanosleep(40);
+      __threadfence();
+    }
+    __syncthreads();
+    fence_proxy_async();
+
+    // ------------------------------------------------------------ finalise the previous tile, keep this tile's means
+    if (warp < NCW) {
+      const int m = sl0 + tid;
+      if (tid < sl1 - sl0) {
+        if (live) {
+          double mu = 0.0;
+          for (int cb = 0; cb < nblk; ++cb) mu += __ldcg(part_mu + ((size_t)b * nblk + cb) * BM + m);
+          mu_keep[b][tid] = mu;
+        }
+        if (tile > t_begin) {
+          const long long q = (tile - 1) * BM + m;
+          if (q < p.Q) {
+            double tot = 0.0;
+            for (int ib = 0; ib < nblk; ++ib) tot += __ldcg(part_ss + ((size_t)(b ^ 1) * nblk + ib) * BM + m);
+            const double mu = p.mean + mu_keep[b ^ 1][tid];
+            const double var = p.amp - tot;
+            if (p.mu) p.mu[q] = mu;
+            if (p.var) p.var[q] = var;
+            if (p.util) {
+              bool ok = true;
+              if (p.has_box) {
+                for (int i = 0; i < d; ++i) {
+                  const double x = p.Xq[q * d + i];
+                  ok = ok && (x >= p.lo[i]) && (x <= p.hi[i]);
+                }
+              }
+              p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
+            }
+          }
+        }
+      }
+    }
+    if (!live) break;
+
+    // ------------------------------------------------------------ phase 2: my block-rows on the int8 tensor cores
+    if (warp == NCW) {
+      if (lane == 0) {
+        for (int ib = 0; ib < nblk; ++ib) {
+          if (owner_s[ib] != rank) continue;
+          const unsigned char* bsrc = p.LinvI8 + ((size_t)ib * (ib + 1) / 2) * I8_B_STAGE;
+          for (int kb = 0; kb <= ib; ++kb, ++it) {
+            const int s = it % I8_NST;
+            const uint32_t ph = (it / I8_NST) & 1u;
+            mbar_wait(&empty[s], ph ^ 1u);
+            unsigned char* dst = ring + (size_t)s * I8_STAGE;
+            mbar_arrive_expect_tx(&full[s], I8_STAGE);
+            bulk_g2s(dst, panel + (size_t)kb * I8_A_STAGE, I8_A_STAGE, &full[s]);
+            bulk_g2s(dst + I8_A_STAGE, bsrc + (size_t)kb * I8_B_STAGE, I8_B_STAGE, &full[s]);
+          }
+        }
+      }
+    } else if (warp == NCW + 1) {
+      if (lane == 0) {
+        for (int ib = 0; ib < nblk; ++ib) {
+          if (owner_s[ib] != rank) continue;
+          mbar_wait(accempty, (nacc & 1u) ^ 1u);         // the epilogue has read the previous block-row
+          tc_fence_after();
+          for (int kb = 0; kb <= ib; ++kb, ++it) {
+            const int s = it % I8_NST;
+            const uint32_t ph = (it / I8_NST) & 1u;
+            mbar_wait(&full[s], ph);
+            tc_fence_after();
+            const uint32_t sa = smem_u32(ring + (size_t)s * I8_STAGE);
+            const uint32_t sb = sa + I8_A_STAGE;
+#pragma unroll
+            for (int kk = 0; kk < I8_BK / 32; ++kk) {
+#pragma unroll
+              for (int pa = 0; pa < I8_DIG; ++pa) {
+                const uint64_t da = umma_desc(sa + (pa * 4 + 2 * kk) * 2048, 2048, 128);
+#pragma unroll
+                for (int rb = 0; rb < I8_DIG; ++rb) {
+                  if (pa + rb >= I8_LEVELS) continue;
+                  const int lev = pa + rb;
+                  const uint64_t db = umma_desc(sb + (rb * 4 + 2 * kk) * 1024, 1024, 128);
+                  const bool first = (kb == 0 && kk == 0 && pa == (lev > 6 ? lev - 6 : 0));
+                  umma_i8(tmem + lev * BN, da, db, first ? 0u : 1u);
+                }
+              }
+            }
+            umma_commit(&empty[s]);                       // stage free once these MMAs have read it
+          }
+          umma_commit(accfull);
+          ++nacc;
+        }
+      }
+    } else {
+      // epilogue: warp w reads TMEM lanes 32 (w % 4) .. + 31 (its queries), columns 32 (w / 4) .. + 31 of each level
+      const int quarter = warp & 3, half = warp >> 2;
+      const int m = quarter * 32 + lane;
+      const uint32_t tl = tmem + ((uint32_t)(quarter * 32) << 16) + half * 32;
+      for (int ib = 0; ib < nblk; ++ib) {
+        if (owner_s[ib] != rank) continue;
+        mbar_wait(accfull, nacc & 1u);
+        ++nacc;
+        tc_fence_after();
+        const double* sc = p.i8scale + ib * BN + half * 32;
+        double ss = 0.0;
+#pragma unroll 1
+        for (int c0 = 0; c0 < 32; c0 += 8) {
+          uint32_t v[I8_LEVELS][8];
+#pragma unroll
+          for (int lev = 0; lev < I8_LEVELS; ++lev) tmem_ld8(tl + lev * BN + c0, v[lev]);
+          tmem_wait_ld();
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            long long hi = (int)v[0][j], lo = (int)v[4][j];
+#pragma unroll
+            for (int lev = 1; lev < 4; ++lev) {
+              hi = hi * 256 + (int)v[lev][j];
+              lo = lo * 256 + (int)v[4 + lev][j];
+            }
+            const double w = fma((double)lo, 0x1p-32, (double)hi) * __ldg(sc + c0 + j);
+            ss = fma(w, w, ss);
+          }
+        }
+        tc_fence_before();
+        if (half == 1) ss_s[m] = ss;
+        named_bar_sync(1, NCONS);
+        if (half == 0) part_ss[((size_t)b * nblk + ib) * BM + m] = ss + ss_s[m];
+        mbar_arrive(accempty);
+      }
+      __threadfence();
+    }
+    __syncthreads();
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 9) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;\n" :: "r"(tmem) : "memory");
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Operand pack: one CTA per padded row i of B = A L^{-1}.  Row scale 2^(ex_i - 38) (the combine's 2^(ex_i - 14) and
+// the hi/lo split's 2^-24), zero for padding rows; digits of round(B[i,k] 2^(55 - ex_i)) with |.| <= 127 * 2^48.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+pack_linv_i8_kernel(const double* __restrict__ Linv, int ld, int N, double amp, unsigned char* __restrict__ out,
+                    double* __restrict__ rowscale) {
+  __shared__ double red[8];
+  const int i = blockIdx.x, tid = threadIdx.x;
+  const int ib = i / I8_BN, ng = (i / 8) % 8, row = i % 8;
+  double mx = 0.0;
+  if (i < N)
+    for (int k = tid; k <= i; k += blockDim.x) mx = fmax(mx, fabs(amp * Linv[(size_t)i * ld + k]));
+  for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if ((tid & 31) == 0) red[tid >> 5] = mx;
+  __syncthreads();
+  mx = 0.0;
+  for (int w = 0; w < 8; ++w) mx = fmax(mx, red[w]);
+  int ex = 0;
+  if (mx > 0.0) {
+    ex = ilogb(mx) + 1;                                  // mx < 2^ex
+    if (mx > ldexp(127.0 / 128.0, ex)) ++ex;             // top digit <= 127 after balanced rounding
+  }
+  if (tid == 0) rowscale[i] = mx > 0.0 ? ldexp(1.0, ex - 38) : 0.0;
+  unsigned char* tile0 = out + ((size_t)ib * (ib + 1) / 2) * I8_B_STAGE;
+  for (int kk = tid; kk < (ib + 1) * I8_BK; kk += blockDim.x) {
+    const int kb = kk / I8_BK, kc = (kk / 16) % 4, c = kk % 16;
+    const int k = kb * I8_BK + kc * 16 + (c >> 2) + 4 * (c & 3);
+    long long X = 0;
+    if (i < N && k <= i && mx > 0.0) X = llrint(ldexp(amp * Linv[(size_t)i * ld + k], 55 - ex));
+    unsigned char* t = tile0 + (size_t)kb * I8_B_STAGE + (kc * 8 + ng) * 128 + row * 16 + c;
+    for (int r = I8_DIG - 1; r >= 1; --r) {
+      const int dg = (int)(signed char)(X & 0xff);
+      X = (X - dg) >> 8;
+      t[r * (4 * 8 * 128)] = (unsigned char)dg;
+    }
+    t[0] = (unsigned char)(signed char)X;
+  }
+}
+
+}  // namespace
+
+size_t linv_i8_bytes(int Npad) {
+  const size_t nblk = (size_t)Npad / I8_BN;
+  return nblk * (nblk + 1) / 2 * I8_B_STAGE;
+}
+
+int launch_pack_linv_i8(const double* Linv, int ld, int N, int Npad, double amp, unsigned char* out, double* rowscale,
+                        cudaStream_t st) {
+  pack_linv_i8_kernel<<<Npad, 256, 0, st>>>(Linv, ld, N, amp, out, rowscale);
+  return (int)cudaGetLastError();
+}
+
+bool predict_i8_fits(int Npad, int d) {
+  return Npad % I8_BN == 0 && Npad / I8_BN <= I8_GROUP_MAX_BLOCKS && i8_smem_bytes(d) <= 200 * 1024;
+}
+
+int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches) {
+  if (p.Q <= 0) return 0;
+  const size_t smem = i8_smem_bytes(p.d);
+  static PerDeviceOnce attr;
+  if (attr.needed()) {
+    cudaError_t e = cudaFuncSetAttribute(predict_var_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         200 * 1024);
+    if (e != cudaSuccess) return (int)e;
+    attr.mark();
+  }
+  const int ngroups = (num_sms + G - 1) / G;
+  cudaError_t e = cudaMemsetAsync(p.grp_arrive, 0, sizeof(int) * ngroups, st);
+  if (e != cudaSuccess) return (int)e;
+  PredictParams pc = p;
+  int Gc = G;
+  void* args[] = {(void*)&pc, (void*)&Gc};
+  e = cudaLaunchCooperativeKernel((const void*)predict_var_i8_kernel, dim3(num_sms), dim3(I8_NTHREADS), args, smem, st);
+  if (launches) ++*launches;
+  return (int)e;
+}
+
+}  // namespace apgp

@@ -132,6 +132,14 @@ class GP(object):
         with groups the K* panels in flight stay in L2 instead of streaming through HBM."""
         _lib.check(self._lib.apgp_set_group(self._h, int(group)), "apgp_set_group")
 
+    def set_var_engine(self, engine):
+        """Engine of the variance product in grouped predict calls: ``"i8"`` (default; int8 tensor cores, exact-integer
+        split of the FP64 operands, used from N = 1024) or ``"dmma"`` (FP64 tensor cores)."""
+        codes = {"dmma": 0, "i8": 1}
+        if engine not in codes:
+            raise ValueError("engine must be 'i8' or 'dmma'")
+        _lib.check(self._lib.apgp_set_var_engine(self._h, codes[engine]), "apgp_set_var_engine")
+
     def set_predict_few(self, enable=True):
         """Calls of at most 16 queries use the few-query kernel (default) or, with ``enable=False``, the tiled kernels."""
         _lib.check(self._lib.apgp_set_predict_few(self._h, 1 if enable else 0), "apgp_set_predict_few")

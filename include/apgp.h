@@ -225,6 +225,13 @@ int apgp_set_variant(apgp_handle* h, int variant);
  * through HBM): 0 = one tile per CTA, -1 = automatic (by training-set size, and by the number of query tiles of the
  * call: a few-tile call is spread over more CTAs for latency), 2..64 = fixed group size.  Default -1. */
 int apgp_set_group(apgp_handle* h, int group);
+/* engine of the variance product in grouped predict calls: APGP_VAR_ENGINE_I8 (default) runs it on the int8 tensor
+ * cores as an exact-integer split of the FP64 operands, at N >= 1024 where that is faster; APGP_VAR_ENGINE_DMMA keeps
+ * the FP64 tensor-core kernel everywhere.  The mean is bit-identical between the two.  Environment:
+ * APGP_PREDICT_VAR_ENGINE=i8|dmma, read by apgp_create / apgp_reset. */
+#define APGP_VAR_ENGINE_DMMA 0
+#define APGP_VAR_ENGINE_I8 1
+int apgp_set_var_engine(apgp_handle* h, int engine);
 /* predict calls of at most 16 queries (the reference asks for ONE point per call: utility.py:131,178,224) run a few-query
  * kernel -- several CTAs per query against the explicit inverse -- instead of a 256-query tile of the DMMA kernels:
  * enable != 0 (default) / 0 = always the tiled kernels.  Environment: APGP_PREDICT_FEW, read by apgp_create / apgp_reset. */
