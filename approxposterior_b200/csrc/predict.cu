@@ -834,8 +834,10 @@ size_t predict_scratch_bytes(int Npad, int num_sms, int variant) {
 // of DMMA for the 256x64 tile); longest-first onto the least loaded rank.  Phase 1: building one 64-column block of
 // the panel costs (2d + 12)/64 of a unit (exp + distances on the same FP64 pipe); the blocks go, one by one, to the
 // rank with the least combined load, which also evens out what phase 2 could not.  Returns max load / mean load.
-// i8: the int8 engine's unit is a 128-query tile on the int8 pipe, and its panel block costs the same FP64 exponentials
-// for half the queries, ~0.86 of its units at d = 5 (estimated from the DMMA rate and the int8 kernel's shared-memory bound)
+// i8: the int8 engine's unit is one 64-wide k-stage of a 128-query block-row on the int8 pipe; its panel block is
+// estimated at ~0.86 units at d = 5.  The -DAPGP_PROF phase profile (profiles/r04_i8_phases_after.txt, cfg3) measures
+// 3.5 units (a factor of 10 here); that value moves G at many padded sizes that are not powers of two and has not
+// been timed there, so the estimate stays until it has (DESIGN 4.1a)
 double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, bool i8 = false) {
   double load[64];
   for (int r = 0; r < gs; ++r) load[r] = 0.0;

@@ -10,14 +10,20 @@
 // query's variance does not depend on the accumulation order, its position in the batch or the group size.
 //
 // Tile: 128 queries x 64 rows of B per block-row, K staged 64 at a time; 8 levels x 64 int32 columns fill the 512
-// TMEM columns.  Operands use the no-swizzle K-major canonical layout: 8-row x 16-byte core matrices, stored
-// [plane][k16 chunk][8-row group][8 rows][16 bytes].  Inside a 16-wide k chunk byte c holds k = c/4 + 4 (c%4): one
+// TMEM columns, level s at columns 64 s.  Operands use the no-swizzle K-major canonical layout of 8-row x 16-byte
+// core matrices.  A (panel) stages are [plane][k16 chunk][8-row group][8 rows][16 bytes]; B (LinvI8) stages are
+// [k16 chunk][plane][8-row group][8 rows][16 bytes], so B's planes r0, r0+1, ... follow each other along N and one
+// MMA of N = 64 n multiplies A plane p by n of them into n adjacent levels (i8_sched: 11 MMAs per 32-wide k-step
+// instead of one 128 x 64 x 32 MMA per digit pair, which read the 4 KB A tile once per 64 output columns and left
+// the MMAs bound by shared-memory operand reads).  Inside a 16-wide k chunk byte c holds k = c/4 + 4 (c%4): one
 // phase-1 thread builds k = l, l+4, l+8, l+12 (the DMMA kernel's order, so the mean is bit-identical) and stores
 // them as one 32-bit word.  A and B use the same permutation; an exact integer sum does not see it.
 //
 // Warps: 0-7 build the panel (phase 1) and run the per-block-row epilogue (tcgen05.ld, combine, W^2 row sums);
 // warp 8 lane 0 streams digit tiles with 1-D bulk TMA; warp 9 owns the TMEM allocation and its lane 0 issues MMAs.
 #include "apgp_internal.h"
+#include <stdio.h>
+#include <stdlib.h>
 
 namespace apgp {
 
@@ -30,6 +36,26 @@ constexpr int I8_B_STAGE = I8_DIG * I8_BN * I8_BK;      // bytes: 28672
 constexpr int I8_STAGE = I8_A_STAGE + I8_B_STAGE;
 constexpr int I8_RING = I8_NST * I8_STAGE;
 constexpr int I8_NTHREADS = 10 * 32;
+
+// -DAPGP_PROF: SM cycles per phase for the first I8_PROF_CTAS CTAs, summed over the tiles of a call and printed by
+// launch_predict_var_i8 when APGP_PROF_PRINT is set (tools/profile_var_i8_phases.py).  Thread 0: 0 phase 1 (panel
+// build, to the end-of-phase barrier), 1 group-barrier wait, 2 finaliser, 7 phase 2 (epilogue warps' view, to the
+// end-of-tile barrier), 8 whole kernel.  MMA lane: 3 waiting on full[] (operands late), 4 waiting on accempty (the
+// epilogue still reads the previous block-row), 5 MMA issue, 6 waiting for the last block-row's epilogue.  Counts:
+// 9 tiles, 10 panel blocks built, 11 phase-2 units (64-wide k-stages) issued.
+#ifdef APGP_PROF
+constexpr int I8_PROF_CTAS = 4, I8_PROF_SLOTS = 12;
+__device__ long long g_i8prof[I8_PROF_CTAS][I8_PROF_SLOTS];
+#define I8P_T(var) long long var = clock64()
+#define I8P_SET(var) ((var) = clock64())
+#define I8P_CNT(slot, n) do { if (blockIdx.x < I8_PROF_CTAS) g_i8prof[blockIdx.x][slot] += (n); } while (0)
+#define I8P_ADD(slot, t0) do { if (blockIdx.x < I8_PROF_CTAS) { const long long _n = clock64(); g_i8prof[blockIdx.x][slot] += _n - (t0); (t0) = _n; } } while (0)
+#else
+#define I8P_T(var) do {} while (0)
+#define I8P_SET(var) do {} while (0)
+#define I8P_CNT(slot, n) do {} while (0)
+#define I8P_ADD(slot, t0) do {} while (0)
+#endif
 
 size_t i8_smem_bytes(int d) { return (size_t)I8_RING + (size_t)d * I8_BM * 8 + 64 * 8 + 8 * 8 + 128; }
 
@@ -44,16 +70,63 @@ __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint
   return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
          (1ull << 46);
 }
-// kind::i8 instruction descriptor: D s32, A u8, B s8, both K-major, M = 128, N = 64
-constexpr uint32_t I8_IDESC = (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(I8_BN >> 3) << 17) |
-                              ((uint32_t)(I8_BM >> 4) << 24);
+// kind::i8 instruction descriptor: D s32, A u8, B s8, both K-major, M = 128, N = n
+__host__ __device__ constexpr uint32_t i8_idesc(int n) {
+  return (2u << 4) | (0u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(I8_BM >> 4) << 24);
+}
 
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t acc) {
+// The MMAs of one 32-wide k-step.  B's digit planes are stacked along N inside a k16 chunk, so one MMA multiplies A
+// plane p by B planes r0 .. r0 + n - 1 (N = 64 n) into the contiguous level accumulators p + r0 .. p + r0 + n - 1,
+// TMEM columns 64 (p + r0) onward: 11 MMAs for the 34 digit products with p + r <= 7, each 4 KB A tile read once per
+// up to 256 output columns.  The accumulate flag covers a whole MMA, so the order is chosen such that on a
+// block-row's first k-step each MMA either writes only levels no earlier MMA has written (it overwrites: level 7
+// first comes from {3, 4, 1}) or only levels some earlier MMA has (it accumulates).
+struct I8Mma { int p, r0, n; };
+constexpr int I8_NMMA = 11;
+__host__ __device__ constexpr I8Mma i8_sched(int j) {
+  constexpr I8Mma t[I8_NMMA] = {{0, 0, 4}, {0, 4, 3}, {3, 4, 1}, {1, 0, 4}, {1, 4, 3}, {2, 0, 4},
+                                {2, 4, 2}, {3, 0, 4}, {4, 0, 4}, {5, 0, 3}, {6, 0, 2}};
+  return t[j];
+}
+
+// how many of the levels of MMA j an earlier MMA of the step has written
+__host__ __device__ constexpr int i8_levels_written_before(int j) {
+  const I8Mma m = i8_sched(j);
+  int cnt = 0;
+  for (int l = m.p + m.r0; l < m.p + m.r0 + m.n; ++l) {
+    bool w = false;
+    for (int i = 0; i < j; ++i) {
+      const I8Mma e = i8_sched(i);
+      w = w || (l >= e.p + e.r0 && l < e.p + e.r0 + e.n);
+    }
+    cnt += w;
+  }
+  return cnt;
+}
+__host__ __device__ constexpr bool i8_sched_ok() {
+  int covered[I8_DIG][I8_DIG] = {};
+  for (int j = 0; j < I8_NMMA; ++j) {
+    const I8Mma m = i8_sched(j);
+    if (m.p < 0 || m.p >= I8_DIG || m.r0 < 0 || m.n < 1 || m.n > 4 || m.r0 + m.n > I8_DIG) return false;
+    if ((m.p + m.r0 + m.n) * I8_BN > 512) return false;                        // inside the TMEM allocation
+    const int w = i8_levels_written_before(j);
+    if (w != 0 && w != m.n) return false;                                       // one accumulate flag serves all its levels
+    for (int r = m.r0; r < m.r0 + m.n; ++r) ++covered[m.p][r];
+  }
+  for (int pa = 0; pa < I8_DIG; ++pa)
+    for (int rb = 0; rb < I8_DIG; ++rb)
+      if (covered[pa][rb] != (pa + rb < I8_LEVELS ? 1 : 0)) return false;       // every kept product exactly once
+  return true;
+}
+static_assert(i8_sched_ok(), "i8_sched must cover each digit product with p + r <= 7 exactly once, inside 512 TMEM "
+                             "columns, with all of an MMA's levels fresh or all already written");
+
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t acc) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
-      :: "r"(tmem_d), "l"(da), "l"(db), "r"(I8_IDESC), "r"(acc) : "memory");
+      :: "r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(acc) : "memory");
 }
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n"
@@ -105,6 +178,9 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   __shared__ uint32_t tmem_base_s;
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  I8P_T(tk);
+  I8P_T(tp);
+  I8P_T(tm);
   const int d = p.d, Npad = p.Npad, nblk = Npad / BN;
   const int grp = blockIdx.x / G, rank = blockIdx.x % G;
   const int gs = min(G, (int)gridDim.x - grp * G);
@@ -153,6 +229,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
     const long long q0 = tile * BM;
     const bool live = tile < t_end;
     unsigned char* panel = scratch8 + ((size_t)grp * 2 + b) * BM * (size_t)Npad * I8_DIG;
+    if (tid == 0 && live) { I8P_CNT(9, 1); I8P_CNT(10, nmine); }
 
     // ------------------------------------------------------------ phase 1: my column blocks of the digit panel
     if (live && warp < NCW) {
@@ -230,6 +307,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
       __threadfence();
     }
     __syncthreads();
+    if (tid == 0) I8P_ADD(0, tp);
 
     // ------------------------------------------------------------ group barrier (one per tile)
     if (tid == 0) {
@@ -239,6 +317,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
       const int target = nbar * gs;
       while (ld_acquire_gpu_i8(arrive) < target) __nanosleep(40);
       __threadfence();
+      I8P_ADD(1, tp);
     }
     __syncthreads();
     fence_proxy_async();
@@ -275,6 +354,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
         }
       }
     }
+    if (tid == 0) I8P_ADD(2, tp);
     if (!live) break;
 
     // ------------------------------------------------------------ phase 2: my block-rows on the int8 tensor cores
@@ -296,37 +376,39 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
       }
     } else if (warp == NCW + 1) {
       if (lane == 0) {
+        I8P_SET(tm);
         for (int ib = 0; ib < nblk; ++ib) {
           if (owner_s[ib] != rank) continue;
           mbar_wait(accempty, (nacc & 1u) ^ 1u);         // the epilogue has read the previous block-row
+          I8P_ADD(4, tm);
           tc_fence_after();
           for (int kb = 0; kb <= ib; ++kb, ++it) {
             const int s = it % I8_NST;
             const uint32_t ph = (it / I8_NST) & 1u;
             mbar_wait(&full[s], ph);
+            I8P_ADD(3, tm);
             tc_fence_after();
             const uint32_t sa = smem_u32(ring + (size_t)s * I8_STAGE);
             const uint32_t sb = sa + I8_A_STAGE;
 #pragma unroll
             for (int kk = 0; kk < I8_BK / 32; ++kk) {
 #pragma unroll
-              for (int pa = 0; pa < I8_DIG; ++pa) {
-                const uint64_t da = umma_desc(sa + (pa * 4 + 2 * kk) * 2048, 2048, 128);
-#pragma unroll
-                for (int rb = 0; rb < I8_DIG; ++rb) {
-                  if (pa + rb >= I8_LEVELS) continue;
-                  const int lev = pa + rb;
-                  const uint64_t db = umma_desc(sb + (rb * 4 + 2 * kk) * 1024, 1024, 128);
-                  const bool first = (kb == 0 && kk == 0 && pa == (lev > 6 ? lev - 6 : 0));
-                  umma_i8(tmem + lev * BN, da, db, first ? 0u : 1u);
-                }
+              for (int j = 0; j < I8_NMMA; ++j) {
+                const I8Mma m = i8_sched(j);
+                const uint64_t da = umma_desc(sa + (m.p * 4 + 2 * kk) * 2048, 2048, 128);
+                const uint64_t db = umma_desc(sb + (2 * kk * I8_DIG + m.r0) * 1024, I8_DIG * 1024, 128);
+                const bool first = kb == 0 && kk == 0 && i8_levels_written_before(j) == 0;
+                umma_i8(tmem + (m.p + m.r0) * BN, da, db, i8_idesc(m.n * BN), first ? 0u : 1u);
               }
             }
             umma_commit(&empty[s]);                       // stage free once these MMAs have read it
+            I8P_ADD(5, tm);
+            I8P_CNT(11, 1);
           }
           umma_commit(accfull);
           ++nacc;
         }
+        I8P_ADD(5, tm);
       }
     } else {
       // epilogue: warp w reads TMEM lanes 32 (w % 4) .. + 31 (its queries), columns 32 (w / 4) .. + 31 of each level
@@ -367,8 +449,11 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
       __threadfence();
     }
     __syncthreads();
+    if (tid == 0) I8P_ADD(7, tp);
+    if (warp == NCW + 1 && lane == 0) I8P_ADD(6, tm);
   }
 
+  if (tid == 0) I8P_ADD(8, tk);
   tc_fence_before();
   __syncthreads();
   if (warp == 9) {
@@ -407,11 +492,11 @@ pack_linv_i8_kernel(const double* __restrict__ Linv, int ld, int N, double amp, 
     const int k = kb * I8_BK + kc * 16 + (c >> 2) + 4 * (c & 3);
     long long X = 0;
     if (i < N && k <= i && mx > 0.0) X = llrint(ldexp(amp * Linv[(size_t)i * ld + k], 55 - ex));
-    unsigned char* t = tile0 + (size_t)kb * I8_B_STAGE + (kc * 8 + ng) * 128 + row * 16 + c;
+    unsigned char* t = tile0 + (size_t)kb * I8_B_STAGE + ((kc * I8_DIG) * 8 + ng) * 128 + row * 16 + c;
     for (int r = I8_DIG - 1; r >= 1; --r) {
       const int dg = (int)(signed char)(X & 0xff);
       X = (X - dg) >> 8;
-      t[r * (4 * 8 * 128)] = (unsigned char)dg;
+      t[r * (8 * 128)] = (unsigned char)dg;
     }
     t[0] = (unsigned char)(signed char)X;
   }
@@ -452,6 +537,20 @@ int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream
   void* args[] = {(void*)&pc, (void*)&Gc};
   e = cudaLaunchCooperativeKernel((const void*)predict_var_i8_kernel, dim3(num_sms), dim3(I8_NTHREADS), args, smem, st);
   if (launches) ++*launches;
+#ifdef APGP_PROF
+  if (getenv("APGP_PROF_PRINT")) {
+    cudaStreamSynchronize(st);
+    long long h[I8_PROF_CTAS][I8_PROF_SLOTS];
+    cudaMemcpyFromSymbol(h, g_i8prof, sizeof(h));
+    for (int c = 0; c < I8_PROF_CTAS; ++c) {
+      fprintf(stderr, "[i8prof] Npad=%d Q=%lld G=%d cta=%d cycles:", p.Npad, p.Q, G, c);
+      for (int i = 0; i < I8_PROF_SLOTS; ++i) fprintf(stderr, " %lld", h[c][i]);
+      fprintf(stderr, "\n");
+    }
+    long long z[I8_PROF_CTAS][I8_PROF_SLOTS] = {};
+    cudaMemcpyToSymbol(g_i8prof, z, sizeof(z));
+  }
+#endif
   return (int)e;
 }
 
