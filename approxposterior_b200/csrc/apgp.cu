@@ -79,6 +79,7 @@ struct apgp_handle {
   DevBuf few_ws;                       // few-query predict: per-split partial sums, means, arrival counters
   int plan_Npad = -1, plan_G = -1, plan_d = -1, plan_i8 = -1;   // what g_plan currently holds
   DevBuf LinvI8, i8scale;              // int8 engine operands (pack_linv_i8)
+  int last_var_path = 0;               // kernel of the last variance launch (apgp_debug_last_var_path)
 };
 
 namespace {
@@ -167,6 +168,7 @@ int apgp_reset(apgp_handle* h) {
   h->mean = 0; h->amp = 1; h->white_noise = -12; h->logdet = 0; h->loglik = 0;
   h->plan_Npad = h->plan_G = h->plan_d = h->plan_i8 = -1;
   h->i8_packed = false;
+  h->last_var_path = 0;
   h->variant = 2; h->variant_eff = 2; h->group = -1; h->predict_few = true; h->var_i8 = true;   // tuning knobs back to their defaults (as apgp_create)
   if (const char* v = getenv("APGP_PREDICT_VARIANT")) { int vv = atoi(v); h->variant = (vv >= 0 && vv <= 2) ? vv : 2; }
   if (const char* gv = getenv("APGP_PREDICT_GROUP")) h->group = atoi(gv);
@@ -402,6 +404,7 @@ static int predict_launch(apgp_handle* h, PredictParams& p, int want_var, cudaSt
       CU(cudaMemsetAsync(h->few_ws.p, 0, predict_few_ws_bytes(), st));
     }
     CUI(launch_predict_few(p, h->Linv.as<double>(), h->Np, h->few_ws.p, st, nl));
+    h->last_var_path = 1;
     return APGP_OK;
   }
   const bool i8 = i8_applies(h);
@@ -436,13 +439,16 @@ static int predict_launch(apgp_handle* h, PredictParams& p, int want_var, cudaSt
       CUI(h->scratch.reserve(predict_scratch_bytes(h->Npad, h->num_sms, h->variant_eff)));
       p.scratch = h->scratch.as<double>();
       CUI(launch_predict_var(p, h->num_sms, st, h->variant_eff, nl));
+      h->last_var_path = 2;
     } else {
       CUI(ge);
+      h->last_var_path = use_i8 ? 4 : 3;
     }
   } else {
     CUI(h->scratch.reserve(predict_scratch_bytes(h->Npad, h->num_sms, h->variant_eff)));
     p.scratch = h->scratch.as<double>();
     CUI(launch_predict_var(p, h->num_sms, st, h->variant_eff, nl));
+    h->last_var_path = 2;
   }
   return APGP_OK;
 }
@@ -1093,5 +1099,45 @@ int apgp_debug_group_plan(int N, int num_sms, int d, long long Q, int requested,
 int apgp_debug_read_prof(long long* out16) { return out16 ? read_prof(out16) : APGP_ERR_ARG; }
 int apgp_get_linv(apgp_handle* h, double* linv) { return get_square(h, h->Linv, linv); }
 int apgp_get_chol(apgp_handle* h, double* L) { return get_square(h, h->K, L); }
+
+int apgp_debug_last_var_path(const apgp_handle* h, int* path) {
+  if (!h || !path) return fail(APGP_ERR_ARG, "apgp_debug_last_var_path");
+  *path = h->last_var_path;
+  return APGP_OK;
+}
+
+int apgp_debug_i8_operands(apgp_handle* h, unsigned char* linv_i8, double* rowscale, unsigned char* panel, int* npad) {
+  if (!h || !h->factored || !h->i8_packed) return fail(APGP_ERR_ARG, "apgp_debug_i8_operands: int8 operands not packed");
+  if (panel && h->last_var_path != 4) return fail(APGP_ERR_ARG, "apgp_debug_i8_operands: last variance call was not int8");
+  Guard g(h->device);
+  if (npad) *npad = h->Npad;
+  if (linv_i8) CU(cudaMemcpyAsync(linv_i8, h->LinvI8.p, linv_i8_bytes(h->Npad), cudaMemcpyDeviceToHost, h->stream));
+  if (rowscale) CU(cudaMemcpyAsync(rowscale, h->i8scale.p, (size_t)h->Npad * 8, cudaMemcpyDeviceToHost, h->stream));
+  // group 0, buffer 0 of the grouped kernel's scratch: the first 128-query tile of the last call
+  if (panel) CU(cudaMemcpyAsync(panel, h->scratch.p, (size_t)128 * 7 * h->Npad, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return APGP_OK;
+}
+
+int apgp_debug_pack_linv_i8(apgp_handle* h, const double* M, int n, double amp, unsigned char* out, double* rowscale) {
+  if (!h || !M || !out || !rowscale || n < 1 || n > 8192) return fail(APGP_ERR_ARG, "apgp_debug_pack_linv_i8");
+  Guard g(h->device);
+  const int Npad = (n + 63) / 64 * 64;
+  const size_t nb = linv_i8_bytes(Npad);
+  void *dm = nullptr, *dout = nullptr, *dsc = nullptr;
+  cudaError_t e = cudaMalloc(&dm, (size_t)n * n * 8);
+  if (e == cudaSuccess) e = cudaMalloc(&dout, nb);
+  if (e == cudaSuccess) e = cudaMalloc(&dsc, (size_t)Npad * 8);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(dm, M, (size_t)n * n * 8, cudaMemcpyHostToDevice, h->stream);
+  if (e == cudaSuccess)
+    e = (cudaError_t)launch_pack_linv_i8((const double*)dm, n, n, Npad, amp, (unsigned char*)dout, (double*)dsc, h->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, nb, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(rowscale, dsc, (size_t)Npad * 8, cudaMemcpyDeviceToHost, h->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+  cudaFree(dm); cudaFree(dout); cudaFree(dsc);
+  if (e != cudaSuccess) return fail(APGP_ERR_CUDA, "apgp_debug_pack_linv_i8", e);
+  h->launches += 1;
+  return APGP_OK;
+}
 
 }  // extern "C"

@@ -337,7 +337,8 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
             double tot = 0.0;
             for (int ib = 0; ib < nblk; ++ib) tot += __ldcg(part_ss + ((size_t)(b ^ 1) * nblk + ib) * BM + m);
             const double mu = p.mean + mu_keep[b ^ 1][tid];
-            const double var = p.amp - tot;
+            // a NaN query has NaN kernel values, which reach the mean but not the panel (fixed55 has no NaN digits)
+            const double var = isnan(mu) ? mu : p.amp - tot;
             if (p.mu) p.mu[q] = mu;
             if (p.var) p.var[q] = var;
             if (p.util) {

@@ -216,6 +216,18 @@ int apgp_debug_exp_neg256(apgp_handle* h, const double* s, int n, double* out);
  * call of Q queries: *G_out = CTAs per query tile (requested: -1 automatic, else as apgp_set_group); tab512 (may be NULL)
  * receives [full group | last group] x [owner of block-row ib | owner of panel column block cb] x 128 ints. */
 int apgp_debug_group_plan(int N, int num_sms, int d, long long Q, int requested, int* G_out, int* tab512);
+/* kernel of the handle's last predict call with variances: 0 none yet, 1 few-query kernel, 2 one-tile DMMA kernel (also
+ * the fallback when the cooperative grouped launch does not fit), 3 grouped DMMA kernel, 4 grouped int8 kernel */
+int apgp_debug_last_var_path(const apgp_handle* h, int* path);
+/* the int8 engine's operands as the kernel reads them (host outputs, each may be NULL): linv_i8 the digit planes of
+ * amp * L^-1 (nblk (nblk + 1) / 2 * 28672 bytes, nblk = Npad / 64), rowscale the Npad row scales 2^(ex_i - 38) (0 for
+ * padding rows), panel the digit panel of the first 128-query tile of the last call (128 * 7 * Npad bytes; only when
+ * that call ran on the int8 kernel), *npad the padded training-set size.  APGP_ERR_ARG when the operands are not
+ * packed, or a panel is asked for and the last variance call did not run on the int8 kernel. */
+int apgp_debug_i8_operands(apgp_handle* h, unsigned char* linv_i8, double* rowscale, unsigned char* panel, int* npad);
+/* run the int8 engine's operand pack on the lower triangle of the host n x n matrix M (n <= 8192, padded to a multiple
+ * of 64 as Npad): out and rowscale receive what apgp_debug_i8_operands returns for a factorisation with L^-1 = M */
+int apgp_debug_pack_linv_i8(apgp_handle* h, const double* M, int n, double amp, unsigned char* out, double* rowscale);
 /* profiling builds (-DAPGP_PROF): read and reset 16 per-phase SM-cycle counters of the log-likelihood objective */
 int apgp_debug_read_prof(long long* out16);
 /* select the variance-kernel tiling (queries x L^-1 rows per CTA tile): 0 = 64x256, 1 = 128x128,

@@ -29,6 +29,15 @@ def _queries(X, Q, d, seed):
     return torch.as_tensor(q, device="cuda")
 
 
+def _path(gp):
+    """Kernel of the last variance call: 2 one-tile DMMA, 3 grouped DMMA, 4 grouped int8."""
+    import ctypes
+    from approxposterior_b200 import _lib
+    p = ctypes.c_int()
+    _lib.check(_lib.load().apgp_debug_last_var_path(gp._h, ctypes.byref(p)), "apgp_debug_last_var_path")
+    return p.value
+
+
 def _both(gp, q):
     import torch
     out = {}
@@ -37,6 +46,7 @@ def _both(gp, q):
         l0 = gp.launch_count
         r1 = gp._predict_raw(q, True, utility="bape", bounds=[(-5.0, 5.0)] * q.shape[1])
         assert gp.launch_count == l0 + 1                             # operands were packed with the factorisation
+        assert _path(gp) == (4 if eng == "i8" else 3)                # the grouped kernel of that engine ran
         r2 = gp._predict_raw(q, True, utility="bape", bounds=[(-5.0, 5.0)] * q.shape[1])
         for a, b in zip(r1, r2):                                     # repeatable launch to launch
             assert torch.equal(a, b)
@@ -53,7 +63,6 @@ def test_i8_engine_matches_dmma(N, d, Q):
     out = _both(gp, q)
     mu0, var0, u0 = out["dmma"]
     mu1, var1, u1 = out["i8"]
-    assert not torch.equal(var0, var1)                                # a different product ran
     assert torch.equal(mu0, mu1)
     assert float((var1 - var0).abs().max()) <= 1e-12          # as the grouped-vs-one-tile DMMA comparison
     fin = torch.isfinite(u0)
@@ -80,6 +89,7 @@ def test_i8_engine_error_against_extended_truth(N, d):
     for eng in ("dmma", "i8"):
         gp.set_var_engine(eng)
         _, var = gp.predict(y, Xq, return_cov=False, return_var=True)
+        assert _path(gp) == (4 if eng == "i8" else 3)
         errs[eng] = float(np.abs(var[:64] - var_t).max())
     gp.set_var_engine("i8")
     assert errs["i8"] <= 2.0 * errs["dmma"] + 1e-16, errs
