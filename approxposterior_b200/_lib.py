@@ -76,7 +76,6 @@ _SIGNATURES = {
     "apgp_get_alpha": (C.c_int, [C.c_void_p, C.c_void_p]),
     "apgp_get_linv": (C.c_int, [C.c_void_p, C.c_void_p]),
     "apgp_get_chol": (C.c_int, [C.c_void_p, C.c_void_p]),
-    "apgp_set_variant": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_set_group": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_set_var_engine": (C.c_int, [C.c_void_p, C.c_int]),
     "apgp_set_predict_few": (C.c_int, [C.c_void_p, C.c_int]),

@@ -52,8 +52,6 @@ struct apgp_handle {
   cudaStream_t copy_in = nullptr, copy_out = nullptr;   // H2D / D2H streams of the pipelined host-buffer predict
   cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_k[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
   int N = 0, d = 0, Np = 0, Npad = 0;
-  int variant = 2;       // requested tiling: 2 = 256x64 (fastest measured, profiles/), 1 = 128x128, 0 = 64x256
-  int variant_eff = 2;   // tiling the current factorisation was packed for
   int group = -1;        // CTAs per query tile in the variance kernel: 0 = one tile per CTA, -1 = automatic, G = fixed
   bool predict_few = true;   // calls of at most PREDICT_FEW_MAX queries: one CTA per query (APGP_PREDICT_FEW=0: tiled kernels)
   bool var_i8 = true;        // variance engine of grouped calls: int8 tensor cores where they apply (predict_i8.cu), else DMMA
@@ -79,7 +77,7 @@ struct apgp_handle {
   DevBuf few_ws;                       // few-query predict: per-split partial sums, means, arrival counters
   int plan_Npad = -1, plan_G = -1, plan_d = -1, plan_i8 = -1;   // what g_plan currently holds
   DevBuf LinvI8, i8scale;              // int8 engine operands (pack_linv_i8)
-  int last_var_path = 0;               // kernel of the last variance launch (apgp_debug_last_var_path)
+  int last_var_path = 0;               // VarPath of the last variance launch (apgp_debug_last_var_path)
 };
 
 namespace {
@@ -93,6 +91,13 @@ struct Guard {  // select the handle's device for the duration of a call
   explicit Guard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
   ~Guard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+// the tuning knobs' environment overrides, read by apgp_create and apgp_reset
+void read_env_knobs(apgp_handle* h) {
+  if (const char* gv = getenv("APGP_PREDICT_GROUP")) h->group = atoi(gv);
+  if (const char* fv = getenv("APGP_PREDICT_FEW")) h->predict_few = atoi(fv) != 0;
+  if (const char* ev = getenv("APGP_PREDICT_VAR_ENGINE")) h->var_i8 = strcmp(ev, "dmma") != 0;
+}
 
 void fill_hyper_row(double* row, double mean, double amp, double wn, const double* logM, int d) {
   row[0] = mean; row[1] = amp; row[2] = exp(wn) + TINY2;
@@ -125,12 +130,7 @@ int apgp_create(apgp_handle** out, int device) {
   h->own_stream = true;
   e = cudaHostAlloc((void**)&h->pin, apgp_handle::PIN_DOUBLES * 8, cudaHostAllocDefault);
   if (e != cudaSuccess) { cudaStreamDestroy(h->stream); delete h; return fail(APGP_ERR_CUDA, "apgp_create: cudaHostAlloc", e); }
-  const char* v = getenv("APGP_PREDICT_VARIANT");
-  if (v) { int vv = atoi(v); h->variant = (vv >= 0 && vv <= 2) ? vv : 2; }
-  const char* gv = getenv("APGP_PREDICT_GROUP");
-  if (gv) h->group = atoi(gv);
-  if (const char* fv = getenv("APGP_PREDICT_FEW")) h->predict_few = atoi(fv) != 0;
-  if (const char* ev = getenv("APGP_PREDICT_VAR_ENGINE")) h->var_i8 = strcmp(ev, "dmma") != 0;
+  read_env_knobs(h);
   *out = h;
   return APGP_OK;
 }
@@ -169,11 +169,8 @@ int apgp_reset(apgp_handle* h) {
   h->plan_Npad = h->plan_G = h->plan_d = h->plan_i8 = -1;
   h->i8_packed = false;
   h->last_var_path = 0;
-  h->variant = 2; h->variant_eff = 2; h->group = -1; h->predict_few = true; h->var_i8 = true;   // tuning knobs back to their defaults (as apgp_create)
-  if (const char* v = getenv("APGP_PREDICT_VARIANT")) { int vv = atoi(v); h->variant = (vv >= 0 && vv <= 2) ? vv : 2; }
-  if (const char* gv = getenv("APGP_PREDICT_GROUP")) h->group = atoi(gv);
-  if (const char* fv = getenv("APGP_PREDICT_FEW")) h->predict_few = atoi(fv) != 0;
-  if (const char* ev = getenv("APGP_PREDICT_VAR_ENGINE")) h->var_i8 = strcmp(ev, "dmma") != 0;
+  h->group = -1; h->predict_few = true; h->var_i8 = true;   // tuning knobs back to their defaults (as apgp_create)
+  read_env_knobs(h);
   if (h->comm) { comm_destroy(h->comm); h->comm = nullptr; h->comm_rank = 0; h->comm_world = 1; }
   return APGP_OK;
 }
@@ -217,12 +214,6 @@ int apgp_set_predict_few(apgp_handle* h, int enable) {
   return APGP_OK;
 }
 
-int apgp_set_variant(apgp_handle* h, int variant) {
-  if (!h || variant < 0 || variant > 2) return fail(APGP_ERR_ARG, "apgp_set_variant");
-  h->variant = variant; h->factored = false;
-  return APGP_OK;
-}
-
 int apgp_set_training(apgp_handle* h, const double* X, const double* y, int N, int d, int on_host) {
   if (!h || !X || !y) return fail(APGP_ERR_ARG, "apgp_set_training: null argument");
   if (N < 1 || d < 1 || d > APGP_MAX_DIM) return fail(APGP_ERR_ARG, "apgp_set_training: need N>=1, 1<=d<=32");
@@ -252,7 +243,7 @@ int apgp_set_hyper(apgp_handle* h, double mean, double amp, const double* log_me
 // faster than the DMMA kernel (profiles/r03_var_engine.jsonl); smaller N, mostly not grouped, stays on DMMA
 constexpr int I8_MIN_NPAD = 1024;
 static bool i8_applies(const apgp_handle* h) {
-  return h->var_i8 && h->group != 0 && h->variant_eff == 2 && h->Npad >= I8_MIN_NPAD && predict_i8_fits(h->Npad, h->d);
+  return h->var_i8 && h->group != 0 && h->Npad >= I8_MIN_NPAD && predict_i8_fits(h->Npad, h->d);
 }
 static int pack_i8_operands(apgp_handle* h, cudaStream_t st, int* nl) {
   CUI(h->LinvI8.reserve(linv_i8_bytes(h->Npad)));
@@ -265,7 +256,7 @@ static int pack_i8_operands(apgp_handle* h, cudaStream_t st, int* nl) {
 
 static int pack_predict_operands(apgp_handle* h, int* nl) {
   const int N = h->N, d = h->d, Np = h->Np;
-  const int BN = predict_variant_bn(h->variant_eff);
+  const int BN = predict_tile_bn(d);
   scale_pad_kernel<<<(h->Npad + 255) / 256, 256, 0, h->stream>>>(h->alpha.as<double>(), N, h->Npad, h->amp,
                                                                  h->alphaA.as<double>()); ++*nl;
   double qs[APGP_MAX_DIM];
@@ -283,9 +274,7 @@ int apgp_factorize(apgp_handle* h, double* logdet, double* loglik, int* info) {
   if (!h->has_training || !h->has_hyper) return fail(APGP_ERR_ARG, "apgp_factorize: training set and hyper-parameters required");
   Guard g(h->device);
   const int N = h->N, d = h->d, Np = h->Np;
-  // the 256x64 tiling stages d x 256 scaled queries in shared memory: beyond d = 31 fall back to 128x128
-  h->variant_eff = (h->variant == 2 && d > 31) ? 1 : h->variant;
-  const int BN = predict_variant_bn(h->variant_eff);
+  const int BN = predict_tile_bn(d);
   h->Npad = (N + BN - 1) / BN * BN;
   h->factored = false;
   if (info) *info = 0;
@@ -351,7 +340,7 @@ int apgp_append_point(apgp_handle* h, const double* x_new, double y_new, double*
   if (!h || !x_new) return fail(APGP_ERR_ARG, "apgp_append_point: null argument");
   if (!h->factored) return fail(APGP_NOT_COMPUTED, "apgp_append_point: GP not computed");
   const int N = h->N, d = h->d, Np = h->Np;
-  const int BN = predict_variant_bn(h->variant_eff);
+  const int BN = predict_tile_bn(d);
   if (N + 1 > Np || (N + BN) / BN * BN != h->Npad) return APGP_NEEDS_REFACTOR;   // padded buffers are full
   Guard g(h->device);
   CUI(h->X.reserve_keep((size_t)(N + 1) * d * 8, (size_t)N * d * 8, h->stream));
@@ -391,65 +380,74 @@ static void fill_predict_params(apgp_handle* h, PredictParams& p) {
   p.mean = h->mean; p.amp = h->amp;
 }
 
+// the variance kernels, as apgp_debug_last_var_path reports them
+enum VarPath { VAR_FEW = 1, VAR_TILE = 2, VAR_GROUP_DMMA = 3, VAR_GROUP_I8 = 4 };
+
+// The variance kernel of a call of Qplan queries (of which this launch is p.Q) and its group size G: a handful of
+// queries go one CTA per query (APGP_PREDICT_FEW=0 keeps them on the tiled kernels); then the int8 engine where it
+// applies and its plan groups the tiles, else the grouped DMMA kernel where its plan does, else one tile per CTA.
+static VarPath choose_var_path(const apgp_handle* h, long long Q, long long Qplan, int* G) {
+  *G = 1;
+  if (Qplan <= PREDICT_FEW_MAX && Q == Qplan && (size_t)h->N * 8 <= 96 * 1024 && h->predict_few) return VAR_FEW;
+  if (h->group == 0) return VAR_TILE;
+  if (i8_applies(h) && (*G = predict_group_size(h->Npad, h->num_sms, h->group, h->d, Qplan, I8_GROUP_TILE)) > 1)
+    return VAR_GROUP_I8;
+  if ((*G = predict_group_size(h->Npad, h->num_sms, h->group, h->d, Qplan, DMMA_GROUP_TILE)) > 1) return VAR_GROUP_DMMA;
+  *G = 1;
+  return VAR_TILE;
+}
+
 // one launch of the predict kernels for the queries described by p (device pointers), on stream st
 // Qplan: the size of the WHOLE call this launch is a slice of -- the group size (hence the summation order of the mean)
 // must not depend on how a host call was sliced
 static int predict_launch(apgp_handle* h, PredictParams& p, int want_var, cudaStream_t st, int* nl, long long Qplan) {
   const int d = h->d;
   if (!want_var) { CUI(launch_predict_mean(p, h->num_sms, st, nl)); return APGP_OK; }
-  // a handful of queries in the whole call: one CTA per query (APGP_PREDICT_FEW=0 keeps them on the tiled kernels)
-  if (Qplan <= PREDICT_FEW_MAX && p.Q == Qplan && (size_t)h->N * 8 <= 96 * 1024 && h->predict_few) {
+  int G = 1;
+  VarPath path = choose_var_path(h, p.Q, Qplan, &G);
+  if (path == VAR_FEW) {
     if (h->few_ws.cap < predict_few_ws_bytes()) {
       CUI(h->few_ws.reserve(predict_few_ws_bytes()));
       CU(cudaMemsetAsync(h->few_ws.p, 0, predict_few_ws_bytes(), st));
     }
     CUI(launch_predict_few(p, h->Linv.as<double>(), h->Np, h->few_ws.p, st, nl));
-    h->last_var_path = 1;
-    return APGP_OK;
-  }
-  const bool i8 = i8_applies(h);
-  int G = (h->group == 0) ? 1 : predict_group_size(h->Npad, h->num_sms, h->variant_eff, h->group, d, Qplan, i8);
-  if (i8 && G > 1) {
-    // packed with the factorisation; here only when the engine was switched to i8 after it
-    if (!h->i8_packed) { int st_ = pack_i8_operands(h, st, nl); if (st_ != APGP_OK) return st_; }
-    p.LinvI8 = h->LinvI8.as<unsigned char>(); p.i8scale = h->i8scale.as<double>();
-  } else if (i8) {
-    G = (h->group == 0) ? 1 : predict_group_size(h->Npad, h->num_sms, h->variant_eff, h->group, d, Qplan);
-  }
-  const bool use_i8 = i8 && p.LinvI8 != nullptr;
-  if (G > 1) {
-    CUI(h->scratch.reserve(predict_group_scratch_bytes(h->Npad, h->num_sms, G, use_i8)));
+  } else if (path != VAR_TILE) {
+    const bool i8 = path == VAR_GROUP_I8;
+    const GroupTile& tile = i8 ? I8_GROUP_TILE : DMMA_GROUP_TILE;
+    if (i8) {
+      // packed with the factorisation; here only when the engine was switched to i8 after it
+      if (!h->i8_packed) { int st_ = pack_i8_operands(h, st, nl); if (st_ != APGP_OK) return st_; }
+      p.LinvI8 = h->LinvI8.as<unsigned char>(); p.i8scale = h->i8scale.as<double>();
+    }
+    CUI(h->scratch.reserve(predict_group_scratch_bytes(h->Npad, h->num_sms, G, tile)));
     CUI(h->g_arrive.reserve(sizeof(int) * ((h->num_sms + G - 1) / G)));
     CUI(h->g_part.reserve(predict_group_part_bytes(h->Npad, h->num_sms, G)));
-    CUI(h->g_plan.reserve(4 * 128 * sizeof(int)));
+    CUI(h->g_plan.reserve(4 * GROUP_MAX_BLOCKS * sizeof(int)));
     p.scratch = h->scratch.as<double>();
     p.grp_arrive = h->g_arrive.as<int>(); p.grp_part = h->g_part.as<double>(); p.grp_plan = h->g_plan.as<int>();
-    if (h->plan_Npad != h->Npad || h->plan_G != G || h->plan_d != d || h->plan_i8 != (int)use_i8) {   // re-plan on a new shape
-      int tab[4 * 128];
-      predict_group_plan(h->Npad, h->num_sms, G, d, tab, use_i8);
+    if (h->plan_Npad != h->Npad || h->plan_G != G || h->plan_d != d || h->plan_i8 != (int)i8) {   // re-plan on a new shape
+      int tab[4 * GROUP_MAX_BLOCKS];
+      predict_group_plan(h->Npad, h->num_sms, G, d, tab, tile);
       CU(cudaMemcpyAsync(h->g_plan.p, tab, sizeof(tab), cudaMemcpyHostToDevice, st));
       CU(cudaStreamSynchronize(st));
-      h->plan_Npad = h->Npad; h->plan_G = G; h->plan_d = d; h->plan_i8 = (int)use_i8;
+      h->plan_Npad = h->Npad; h->plan_G = G; h->plan_d = d; h->plan_i8 = (int)i8;
     }
-    const int ge = use_i8 ? launch_predict_var_i8(p, h->num_sms, G, st, nl) : launch_predict_var_grouped(p, h->num_sms, G, st, nl);
+    const int ge = i8 ? launch_predict_var_i8(p, h->num_sms, G, st, nl) : launch_predict_var_grouped(p, h->num_sms, G, st, nl);
     if (ge == (int)cudaErrorCooperativeLaunchTooLarge) {
       // the GPU is shared (fewer SMs free than the grid needs for its spin barriers): one tile per CTA instead
       (void)cudaGetLastError();
       --*nl;
-      CUI(h->scratch.reserve(predict_scratch_bytes(h->Npad, h->num_sms, h->variant_eff)));
-      p.scratch = h->scratch.as<double>();
-      CUI(launch_predict_var(p, h->num_sms, st, h->variant_eff, nl));
-      h->last_var_path = 2;
+      path = VAR_TILE;
     } else {
       CUI(ge);
-      h->last_var_path = use_i8 ? 4 : 3;
     }
-  } else {
-    CUI(h->scratch.reserve(predict_scratch_bytes(h->Npad, h->num_sms, h->variant_eff)));
-    p.scratch = h->scratch.as<double>();
-    CUI(launch_predict_var(p, h->num_sms, st, h->variant_eff, nl));
-    h->last_var_path = 2;
   }
+  if (path == VAR_TILE) {
+    CUI(h->scratch.reserve(predict_scratch_bytes(h->Npad, h->num_sms, d)));
+    p.scratch = h->scratch.as<double>();
+    CUI(launch_predict_var(p, h->num_sms, st, nl));
+  }
+  h->last_var_path = path;
   return APGP_OK;
 }
 
@@ -813,7 +811,7 @@ int apgp_comm_destroy(apgp_handle* h) {
 
 // header of a broadcast factorisation: everything host-side that apgp_factorize leaves in the handle
 struct FactorHeader {
-  int N, d, Np, Npad, variant_eff, factored;
+  int N, d, Np, Npad, factored;
   double mean, amp, white_noise, logdet, loglik;
   double log_metric[APGP_MAX_DIM];
 };
@@ -827,7 +825,7 @@ int apgp_comm_broadcast_factor(apgp_handle* h, int root) {
   FactorHeader hd;
   memset(&hd, 0, sizeof(hd));
   if (is_root) {
-    hd.N = h->N; hd.d = h->d; hd.Np = h->Np; hd.Npad = h->Npad; hd.variant_eff = h->variant_eff; hd.factored = 1;
+    hd.N = h->N; hd.d = h->d; hd.Np = h->Np; hd.Npad = h->Npad; hd.factored = 1;
     hd.mean = h->mean; hd.amp = h->amp; hd.white_noise = h->white_noise; hd.logdet = h->logdet; hd.loglik = h->loglik;
     for (int i = 0; i < h->d; ++i) hd.log_metric[i] = h->log_metric[i];
   }
@@ -839,7 +837,7 @@ int apgp_comm_broadcast_factor(apgp_handle* h, int root) {
   if (!hd.factored || hd.N < 1 || hd.d < 1 || hd.d > APGP_MAX_DIM) return fail(APGP_ERR_COMM, "apgp_comm_broadcast_factor: bad header");
   const int N = hd.N, d = hd.d, Np = hd.Np;
   if (!is_root) {
-    h->N = N; h->d = d; h->Np = Np; h->Npad = hd.Npad; h->variant_eff = hd.variant_eff;
+    h->N = N; h->d = d; h->Np = Np; h->Npad = hd.Npad;
     h->mean = hd.mean; h->amp = hd.amp; h->white_noise = hd.white_noise; h->logdet = hd.logdet; h->loglik = hd.loglik;
     for (int i = 0; i < d; ++i) h->log_metric[i] = hd.log_metric[i];
     h->has_training = true; h->has_hyper = true; h->factored = false;
@@ -848,7 +846,7 @@ int apgp_comm_broadcast_factor(apgp_handle* h, int root) {
     CUI(h->Linv.reserve((size_t)Np * Np * 8)); CUI(h->work.reserve((size_t)Np * Np * 8));
     CUI(h->alpha.reserve((size_t)Np * 8)); CUI(h->alphaA.reserve((size_t)h->Npad * 8)); CUI(h->Xs.reserve((size_t)d * h->Npad * 8));
     CUI(h->scal.reserve(4 * 8)); CUI(h->info.reserve(4)); CUI(h->hyper.reserve((3 + APGP_MAX_DIM) * 8)); CUI(h->qscale.reserve(APGP_MAX_DIM * 8));
-    const int BN = predict_variant_bn(h->variant_eff);
+    const int BN = predict_tile_bn(d);
     CUI(h->LinvF.reserve((size_t)linvf_total_tiles(h->Npad, BN) * BN * 16 * 8));
   }
   struct { DevBuf* b; size_t bytes; } parts[] = {
@@ -1091,9 +1089,9 @@ int apgp_debug_group_plan(int N, int num_sms, int d, long long Q, int requested,
   // host-only: the work split the grouped variance kernel would use (no device needed; exercised by the CPU tests)
   if (!G_out || N < 1 || num_sms < 1 || d < 1) return fail(APGP_ERR_ARG, "apgp_debug_group_plan");
   const int Npad = (N + 63) / 64 * 64;
-  const int G = predict_group_size(Npad, num_sms, 2, requested, d, Q);
+  const int G = predict_group_size(Npad, num_sms, requested, d, Q, DMMA_GROUP_TILE);
   *G_out = G;
-  if (tab512 && G > 1) predict_group_plan(Npad, num_sms, G, d, tab512);
+  if (tab512 && G > 1) predict_group_plan(Npad, num_sms, G, d, tab512, DMMA_GROUP_TILE);
   return APGP_OK;
 }
 int apgp_debug_read_prof(long long* out16) { return out16 ? read_prof(out16) : APGP_ERR_ARG; }
@@ -1114,7 +1112,9 @@ int apgp_debug_i8_operands(apgp_handle* h, unsigned char* linv_i8, double* rowsc
   if (linv_i8) CU(cudaMemcpyAsync(linv_i8, h->LinvI8.p, linv_i8_bytes(h->Npad), cudaMemcpyDeviceToHost, h->stream));
   if (rowscale) CU(cudaMemcpyAsync(rowscale, h->i8scale.p, (size_t)h->Npad * 8, cudaMemcpyDeviceToHost, h->stream));
   // group 0, buffer 0 of the grouped kernel's scratch: the first 128-query tile of the last call
-  if (panel) CU(cudaMemcpyAsync(panel, h->scratch.p, (size_t)128 * 7 * h->Npad, cudaMemcpyDeviceToHost, h->stream));
+  if (panel)
+    CU(cudaMemcpyAsync(panel, h->scratch.p, (size_t)I8_GROUP_TILE.bm * I8_GROUP_TILE.panel_bytes * h->Npad,
+                       cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return APGP_OK;
 }

@@ -43,28 +43,39 @@ struct PredictParams {
   double ybest, zeta;
   int* grp_arrive;         // grouped kernel: [ngroups] arrival counters (zeroed per launch)
   double* grp_part;        // grouped kernel: [ngroups][2 (mu, ss)][2 buffers][Npad/64][256] per-block partial sums
-  int* grp_plan;           // grouped kernel: work-split tables (plan_group_split), 4 x 128 ints
+  int* grp_plan;           // grouped kernel: work-split tables (plan_group_split), 4 x GROUP_MAX_BLOCKS ints
   const unsigned char* LinvI8;   // int8 engine: digit planes of A * L^{-1} (predict_i8.cu)
   const double* i8scale;   // int8 engine: [Npad] per-row scale of those digits
 };
 
-int predict_variant_bn(int variant);   // block-row height BN of the LinvF tiling used by a kernel variant
+// grouped variance kernels: at most GROUP_MAX_BLOCKS 64-column blocks, Npad <= 8192
+constexpr int GROUP_MAX_BLOCKS = 128;
+
+// one-tile-per-CTA variance kernel: block-row height BN of its LinvF tiling (and the padding of Npad), from d
+int predict_tile_bn(int d);
 
 // returns cudaError_t as int; *launches incremented by the number of kernel launches issued
-int launch_predict_var(const PredictParams& p, int num_sms, cudaStream_t st, int variant, int* launches);
+int launch_predict_var(const PredictParams& p, int num_sms, cudaStream_t st, int* launches);
 // at most PREDICT_FEW_MAX queries: one CTA per query against the explicit row-major inverse (pure latency path)
 constexpr long long PREDICT_FEW_MAX = 16;
 size_t predict_few_ws_bytes();
 int launch_predict_few(const PredictParams& p, const double* Linv, int ld, void* ws, cudaStream_t st, int* launches);
 int launch_exp_neg_test(const double* s, int n, double* out, cudaStream_t st, int variant = 0);
 int launch_predict_mean(const PredictParams& p, int num_sms, cudaStream_t st, int* launches);
-size_t predict_scratch_bytes(int Npad, int num_sms, int variant);
-// grouped 256x64 kernel: G CTAs share one query tile so the K* panels in flight stay in L2 (predict.cu).
+size_t predict_scratch_bytes(int Npad, int num_sms, int d);
+// What the group planner needs to know about a grouped kernel's tile
+struct GroupTile {
+  int bm;                  // queries per tile
+  int panel_bytes;         // panel bytes per (query, training point)
+  double phase1_scale;     // cost of building a 64-column panel block, relative to the DMMA tile's (plan_group_split)
+};
+extern const GroupTile DMMA_GROUP_TILE;   // predict_var_group_kernel, 256 x 64 (predict.cu)
+extern const GroupTile I8_GROUP_TILE;     // predict_var_i8_kernel, 128 x 64 (predict_i8.cu)
+// grouped kernels: G CTAs share one query tile so the K* panels in flight stay in L2 (predict.cu).
 // requested < 0: automatic choice; returns 1 when grouping is off / not applicable
-// i8: plan for the int8 engine's 128-query tile (predict_i8.cu) instead of the DMMA kernel's 256-query tile
-int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q, bool i8 = false);
-void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab /*[4*128]*/, bool i8 = false);
-size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, bool i8 = false);
+int predict_group_size(int Npad, int num_sms, int requested, int d, long long Q, const GroupTile& tile);
+void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab /*[4 * GROUP_MAX_BLOCKS]*/, const GroupTile& tile);
+size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, const GroupTile& tile);
 size_t predict_group_part_bytes(int Npad, int num_sms, int G);
 int launch_predict_var_grouped(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches);
 // int8 tensor-core variance engine (grouped launch only): exact-integer split of the triangular product

@@ -23,7 +23,7 @@
 // The exponentials are evaluated once per (query, training point): DMMA and DFMA share one
 // FP64 pipe on B200 (profiles/r01_fp64_pipe_probe.txt), so recomputing K* per output block
 // would come straight out of the GEMM's budget.
-#include "apgp_internal.h"
+#include "predict_tile.cuh"
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -93,15 +93,11 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
 
     // ------------------------------------------------------------ phase 1: K* panel + mean
     if (warp < NCONS_WARPS) {
-      for (int e = tid; e < d * BM; e += NCONS) {
-        int i = e / BM, m = e - i * BM;
-        long long q = q0 + m;
-        qs[e] = (q < p.Q) ? p.Xq[q * d + i] * p.qscale[i] : 0.0;
-      }
+      stage_queries<BM, NCONS>(qs, p, d, q0, tid);
       // chunk of training columns staged in the (idle) ring: xs[d][JCH] + alpha[JCH]
       int JCH = (C::RING / (d + 1)) & ~15;
       if (JCH > Npad) JCH = Npad;
-      constexpr int R = BM / (8 * NCW);                // m8 blocks per warp: their exp chains interleave (4R-way ILP)
+      constexpr int R = BM / (8 * NCW);                // m8 blocks per warp
       double mu_part[R] = {};
       for (int j0 = 0; j0 < Npad; j0 += JCH) {
         const int jn = min(JCH, Npad - j0);
@@ -114,44 +110,13 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
         }
         mbar_wait(stagebar, nstaged & 1u);
         ++nstaged;
-        const double* al = ring + d * JCH;
         double macc[R] = {};
-        for (int jb = 0; jb < jn; jb += 16) {           // 4 k4-blocks per trip
-          const int jj = jb + (lane & 3);
-          double s[R][4] = {};
-          for (int i = 0; i < d; ++i) {
-            const double* xr = ring + i * JCH + jj;
-            const double x0 = xr[0], x1 = xr[4], x2 = xr[8], x3 = xr[12];
-#pragma unroll
-            for (int r = 0; r < R; ++r) {
-              const double qv = qs[i * BM + (warp + r * NCONS_WARPS) * 8 + (lane >> 2)];
-              const double d0 = x0 - qv, d1 = x1 - qv, d2 = x2 - qv, d3 = x3 - qv;
-              s[r][0] = fma(d0, d0, s[r][0]); s[r][1] = fma(d1, d1, s[r][1]);
-              s[r][2] = fma(d2, d2, s[r][2]); s[r][3] = fma(d3, d3, s[r][3]);
-            }
-          }
-          const double a0 = al[jj], a1 = al[jj + 4], a2 = al[jj + 8], a3 = al[jj + 12];
-#pragma unroll
-          for (int r = 0; r < R; ++r) {
-            const int mb = warp + r * NCONS_WARPS;
-            const double e0 = exp_neg(s[r][0], etab), e1 = exp_neg(s[r][1], etab);
-            const double e2 = exp_neg(s[r][2], etab), e3 = exp_neg(s[r][3], etab);
-            macc[r] = fma(e0, a0, macc[r]); macc[r] = fma(e1, a1, macc[r]);
-            macc[r] = fma(e2, a2, macc[r]); macc[r] = fma(e3, a3, macc[r]);
-            double* dst = panel + ((size_t)((j0 + jb) >> 2) * (BM / 8) + mb) * 32 + lane;
-            dst[0] = e0; dst[(BM / 8) * 32] = e1; dst[2 * (BM / 8) * 32] = e2; dst[3 * (BM / 8) * 32] = e3;
-          }
-        }
+        panel_columns<BM, NCW>(ring, JCH, ring + d * JCH, jn, qs, d, etab, warp, lane, macc,
+                               [&](int jb, int mb, const double (&e)[4]) { store_dmma_panel<BM>(panel, j0 + jb, mb, lane, e); });
 #pragma unroll
         for (int r = 0; r < R; ++r) mu_part[r] += macc[r];
       }
-#pragma unroll
-      for (int r = 0; r < R; ++r) {
-        double v = mu_part[r];
-        v += __shfl_xor_sync(0xffffffffu, v, 1);
-        v += __shfl_xor_sync(0xffffffffu, v, 2);
-        if ((lane & 3) == 0) mu_s[(warp + r * NCONS_WARPS) * 8 + (lane >> 2)] = v;
-      }
+      store_row_sums<R, NCW>(mu_part, mu_s, warp, lane);
       fence_proxy_async();                             // panel stores -> visible to the TMA reads below
     }
     __syncthreads();
@@ -250,20 +215,7 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
           double tot = 0.0;
 #pragma unroll
           for (int w = 0; w < C::WARPS_N; ++w) tot += ss_s[w * BM + tid];
-          const double mu = p.mean + mu_s[tid];
-          const double var = p.amp - tot;
-          if (p.mu) p.mu[q] = mu;
-          if (p.var) p.var[q] = var;
-          if (p.util) {
-            bool ok = true;
-            if (p.has_box) {
-              for (int i = 0; i < d; ++i) {
-                const double x = p.Xq[q * d + i];
-                ok = ok && (x >= p.lo[i]) && (x <= p.hi[i]);
-              }
-            }
-            p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
-          }
+          write_query(p, d, q, p.mean + mu_s[tid], p.amp - tot);
         }
       }
     }
@@ -291,19 +243,11 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
 // group; against the one-tile-per-CTA kernel the variance agrees to ~1e-15 and the mean to the rounding of a
 // length-N sum (tests/test_gpu_parity.py::test_grouped_variance_kernel_matches_one_tile_per_cta).
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-constexpr int GROUP_MAX_BLOCKS = 128;       // Npad <= 8192 at BN = 64
-
 template <int BM, int BN, int NSTAGE>
 __global__ void __launch_bounds__(8 * 32 + 32, 1)
 predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
   using C = VarCfg<BM, BN, NSTAGE, 8>;
-  constexpr int NCW = 8, NCONS = C::NCONS;
+  constexpr int NCW = 8;
   static_assert(C::WARPS_N == 1, "grouped kernel is written for the 256x64 tiling");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   double* ring = reinterpret_cast<double*>(smem_raw);
@@ -318,20 +262,9 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
   __shared__ double mu_keep[2][BM];                     // my slice's complete means, per buffer
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int d = p.d, Npad = p.Npad, nblk = Npad / BN;
-  const int grp = blockIdx.x / G, rank = blockIdx.x % G;
-  const int gs = min(G, (int)gridDim.x - grp * G);      // ranks in my group
-  const long long ntiles = (p.Q + BM - 1) / BM;
-  // contiguous share of the tiles, proportional to the group's size; rounding up hands the odd tiles to the first
-  // (full-size) groups -- a single-tile call must not land on the smaller last group
-  const long long t_begin = (ntiles * (long long)(grp * G) + gridDim.x - 1) / gridDim.x;
-  const long long t_end = (ntiles * (long long)(grp * G + gs) + gridDim.x - 1) / gridDim.x;
-  const int sl0 = BM * rank / gs, sl1 = BM * (rank + 1) / gs;                                            // my query slice
-  int* arrive = p.grp_arrive + grp;
-  // partial sums are kept per 64-column block (mean) and per block-row (variance) and added in block order by the
-  // finaliser, so a query's result does not depend on which rank -- or how large a group -- computed the pieces
-  double* part_mu = p.grp_part + (size_t)grp * 4 * nblk * BM;       // [2 buffers][nblk][BM]
-  double* part_ss = part_mu + (size_t)2 * nblk * BM;                // [2 buffers][nblk][BM]
+  const int Npad = p.Npad;
+  const GroupCtx<BM, BN> g(p, G);
+  const int nblk = g.nblk, rank = g.rank;
 
   if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
   if (tid == 0) {
@@ -339,139 +272,30 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
     mbar_init(stagebar, 1);
     mbar_fence_init();
   }
-  {   // work split planned on the host (plan_group_split): full groups use table 0, a smaller last group table 1
-    const int* tab = p.grp_plan + (gs == G ? 0 : 2 * GROUP_MAX_BLOCKS);
-    for (int e = tid; e < nblk; e += blockDim.x) owner_s[e] = tab[e];
-    if (tid == 0) {
-      int n = 0;
-      for (int e = 0; e < nblk; ++e) if (tab[GROUP_MAX_BLOCKS + e] == rank) myblk_s[n++] = e;
-      nmine_s = n;
-    }
-  }
+  g.load_plan(p, G, owner_s, myblk_s, &nmine_s);
   __syncthreads();
   const int nmine = nmine_s;
 
   uint32_t it = 0, nstaged = 0;
   int nbar = 0;                                          // group barriers passed so far
 
-  for (long long tile = t_begin; tile <= t_end; ++tile) {
-    const int b = (int)((tile - t_begin) & 1);
-    const long long q0 = tile * BM;
-    const bool live = tile < t_end;                      // the extra trip only finalises the last tile
-    double* panel = p.scratch + ((size_t)grp * 2 + b) * BM * Npad;
+  for (long long tile = g.t_begin; tile <= g.t_end; ++tile) {
+    const int b = (int)((tile - g.t_begin) & 1);
+    const bool live = tile < g.t_end;                    // the extra trip only finalises the last tile
+    double* panel = p.scratch + ((size_t)g.grp * 2 + b) * BM * Npad;
 
     // ------------------------------------------------------------ phase 1: my column blocks of the panel
     if (live && warp < NCW) {
-      for (int e = tid; e < d * BM; e += NCONS) {
-        int i = e / BM, m = e - i * BM;
-        long long q = q0 + m;
-        qs[e] = (q < p.Q) ? p.Xq[q * d + i] * p.qscale[i] : 0.0;
-      }
-      // my 64-column blocks, up to CAPB per staging round (each block: d+1 bulk copies into consecutive ring slots)
-      const int CAPB = min(8, (C::RING / (d + 1)) / BN);
-      const int JCHT = CAPB * BN;                        // ring row stride
-      constexpr int R = BM / (8 * NCW);
-      for (int s0 = 0; s0 < nmine; s0 += CAPB) {
-        const int ns = min(CAPB, nmine - s0);
-        named_bar_sync(1, NCONS);
-        if (tid == 0) {
-          mbar_arrive_expect_tx(stagebar, (uint32_t)((d + 1) * ns * BN * 8));
-          for (int sl = 0; sl < ns; ++sl) {
-            const int j0 = myblk_s[s0 + sl] * BN;
-            for (int i = 0; i < d; ++i) bulk_g2s(ring + i * JCHT + sl * BN, p.Xs + (size_t)i * Npad + j0, BN * 8, stagebar);
-            bulk_g2s(ring + d * JCHT + sl * BN, p.alphaA + j0, BN * 8, stagebar);
-          }
-        }
-        mbar_wait(stagebar, nstaged & 1u);
-        ++nstaged;
-        for (int sl = 0; sl < ns; ++sl) {
-          const int cb = myblk_s[s0 + sl];
-          const int j0 = cb * BN;
-          const double* al = ring + d * JCHT + sl * BN;
-          double macc[R] = {};
-          for (int jb = 0; jb < BN; jb += 16) {
-            const int jj = jb + (lane & 3);
-            double s[R][4] = {};
-            for (int i = 0; i < d; ++i) {
-              const double* xr = ring + i * JCHT + sl * BN + jj;
-              const double x0 = xr[0], x1 = xr[4], x2 = xr[8], x3 = xr[12];
-#pragma unroll
-              for (int r = 0; r < R; ++r) {
-                const double qv = qs[i * BM + (warp + r * NCW) * 8 + (lane >> 2)];
-                const double d0 = x0 - qv, d1 = x1 - qv, d2 = x2 - qv, d3 = x3 - qv;
-                s[r][0] = fma(d0, d0, s[r][0]); s[r][1] = fma(d1, d1, s[r][1]);
-                s[r][2] = fma(d2, d2, s[r][2]); s[r][3] = fma(d3, d3, s[r][3]);
-              }
-            }
-            const double a0 = al[jj], a1 = al[jj + 4], a2 = al[jj + 8], a3 = al[jj + 12];
-#pragma unroll
-            for (int r = 0; r < R; ++r) {
-              const int mb = warp + r * NCW;
-              const double e0 = exp_neg(s[r][0], etab), e1 = exp_neg(s[r][1], etab);
-              const double e2 = exp_neg(s[r][2], etab), e3 = exp_neg(s[r][3], etab);
-              macc[r] = fma(e0, a0, macc[r]); macc[r] = fma(e1, a1, macc[r]);
-              macc[r] = fma(e2, a2, macc[r]); macc[r] = fma(e3, a3, macc[r]);
-              double* dst = panel + ((size_t)((j0 + jb) >> 2) * (BM / 8) + mb) * 32 + lane;
-              dst[0] = e0; dst[(BM / 8) * 32] = e1; dst[2 * (BM / 8) * 32] = e2; dst[3 * (BM / 8) * 32] = e3;
-            }
-          }
-#pragma unroll
-          for (int r = 0; r < R; ++r) {                  // this block's contribution to the means
-            double v = macc[r];
-            v += __shfl_xor_sync(0xffffffffu, v, 1);
-            v += __shfl_xor_sync(0xffffffffu, v, 2);
-            if ((lane & 3) == 0) part_mu[((size_t)b * nblk + cb) * BM + (warp + r * NCW) * 8 + (lane >> 2)] = v;
-          }
-        }
-      }
+      group_phase1<BM, BN, NCW>(p, tile * BM, qs, etab, ring, C::RING, myblk_s, nmine, stagebar, nstaged,
+                                g.part_mu + (size_t)b * nblk * BM, [&](int cb, int jb, int mb, const double (&e)[4]) {
+                                  store_dmma_panel<BM>(panel, cb * BN + jb, mb, lane, e);
+                                });
       __threadfence();                                   // panel + partial means visible GPU-wide before we arrive
     }
     __syncthreads();
 
-    // ------------------------------------------------------------ group barrier (one per tile)
-    if (tid == 0) {
-      ++nbar;
-      __threadfence();                                   // cumulative: everything this CTA wrote before the bar.sync
-      atomicAdd(arrive, 1);
-      const int target = nbar * gs;
-      while (ld_acquire_gpu(arrive) < target) __nanosleep(40);
-      __threadfence();
-    }
-    __syncthreads();
-    fence_proxy_async();                                 // other CTAs' panel stores (generic proxy) -> our TMA reads
-
-    // ------------------------------------------------------------ finalise the previous tile, keep this tile's means
-    if (warp < NCW) {
-      const int m = sl0 + tid;
-      if (tid < sl1 - sl0) {
-        if (live) {
-          double mu = 0.0;
-          for (int cb = 0; cb < nblk; ++cb) mu += __ldcg(part_mu + ((size_t)b * nblk + cb) * BM + m);
-          mu_keep[b][tid] = mu;
-        }
-        if (tile > t_begin) {
-          const long long q = (tile - 1) * BM + m;
-          if (q < p.Q) {
-            double tot = 0.0;
-            for (int ib = 0; ib < nblk; ++ib) tot += __ldcg(part_ss + ((size_t)(b ^ 1) * nblk + ib) * BM + m);
-            const double mu = p.mean + mu_keep[b ^ 1][tid];
-            const double var = p.amp - tot;
-            if (p.mu) p.mu[q] = mu;
-            if (p.var) p.var[q] = var;
-            if (p.util) {
-              bool ok = true;
-              if (p.has_box) {
-                for (int i = 0; i < d; ++i) {
-                  const double x = p.Xq[q * d + i];
-                  ok = ok && (x >= p.lo[i]) && (x <= p.hi[i]);
-                }
-              }
-              p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
-            }
-          }
-        }
-      }
-    }
+    g.barrier(nbar);
+    g.finalise(p, tile, live, b, mu_keep, [&](double, double tot) { return p.amp - tot; });
     if (!live) break;
 
     // ------------------------------------------------------------ phase 2: my block-rows of the triangular GEMM
@@ -552,7 +376,7 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
           }
           sacc += __shfl_xor_sync(0xffffffffu, sacc, 1);
           sacc += __shfl_xor_sync(0xffffffffu, sacc, 2);
-          if ((lane & 3) == 0) part_ss[((size_t)b * nblk + ib) * BM + wm * 32 + mb * 8 + (lane >> 2)] = sacc;
+          if ((lane & 3) == 0) g.part_ss[((size_t)b * nblk + ib) * BM + wm * 32 + mb * 8 + (lane >> 2)] = sacc;
         }
       }
       __threadfence();                                   // partial row sums visible before the next barrier's arrival
@@ -742,14 +566,7 @@ predict_few_kernel(const __grid_constant__ PredictParams p, const double* __rest
     const double mu = __ldcg(mu_ws + q);
     const double var = p.amp - tot;
     count[q] = 0;                                      // re-armed for the next launch on this stream
-    if (p.mu) p.mu[q] = mu;
-    if (p.var) p.var[q] = var;
-    if (p.util) {
-      bool ok = true;
-      if (p.has_box)
-        for (int i = 0; i < d; ++i) { const double x = p.Xq[q * d + i]; ok = ok && (x >= p.lo[i]) && (x <= p.hi[i]); }
-      p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
-    }
+    write_query(p, d, q, mu, var);
   }
 }
 
@@ -818,27 +635,24 @@ int launch_var_t(const PredictParams& p, int num_sms, cudaStream_t st) {
 
 }  // namespace
 
-// variants (BM x BN): 0 = 64x256, 1 = 128x128, 2 = 256x64 (default: B fragments amortised over 8 m8 blocks,
-// smallest diagonal-block waste, no register spills).  Two other schedules (warp-specialised builders, inline
-// builder) were measured slower and are archived with their profiles under profiles/r01_schedules_tried/.
-static inline int variant_bm(int v) { return v == 0 ? 64 : (v == 2 ? 256 : 128); }
-static inline int variant_bn(int v) { return v == 0 ? 256 : (v == 2 ? 64 : 128); }
-int predict_variant_bn(int variant) { return variant_bn(variant); }
+// One tile per CTA: 256x64 (B fragments amortised over 8 m8 blocks, smallest diagonal-block waste, no register
+// spills), or 128x128 from d = 32, where d x 256 staged queries no longer fit beside the 256x64 tile's ring.  Two other
+// schedules (warp-specialised builders, inline builder) were measured slower and are archived with their profiles
+// under profiles/r01_schedules_tried/.
+static int tile_bm(int d) { return d > 31 ? 128 : 256; }
+int predict_tile_bn(int d) { return 256 * 64 / tile_bm(d); }
 
-size_t predict_scratch_bytes(int Npad, int num_sms, int variant) {
-  return (size_t)num_sms * variant_bm(variant) * Npad * 8;
-}
+size_t predict_scratch_bytes(int Npad, int num_sms, int d) { return (size_t)num_sms * tile_bm(d) * Npad * 8; }
 
 // ---- grouped launch (256x64 tiling only) ------------------------------------------------------------
 // Work split inside a group of gs ranks.  Phase 2: block-row ib of L^-1 costs ib + 1 units (one unit = 64 k-columns
 // of DMMA for the 256x64 tile); longest-first onto the least loaded rank.  Phase 1: building one 64-column block of
 // the panel costs (2d + 12)/64 of a unit (exp + distances on the same FP64 pipe); the blocks go, one by one, to the
 // rank with the least combined load, which also evens out what phase 2 could not.  Returns max load / mean load.
-// i8: the int8 engine's unit is one 64-wide k-stage of a 128-query block-row on the int8 pipe; its panel block is
-// estimated at ~0.86 units at d = 5.  The -DAPGP_PROF phase profile (profiles/r04_i8_phases_after.txt, cfg3) measures
-// 3.5 units (a factor of 10 here); that value moves G at many padded sizes that are not powers of two and has not
-// been timed there, so the estimate stays until it has (DESIGN 4.1a)
-double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, bool i8 = false) {
+// Other engines scale that phase-1 cost by their tile's phase1_scale.
+const GroupTile DMMA_GROUP_TILE = {256, 8, 1.0};
+
+double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, const GroupTile& tile) {
   double load[64];
   for (int r = 0; r < gs; ++r) load[r] = 0.0;
   for (int ib = nblk - 1; ib >= 0; --ib) {
@@ -846,7 +660,7 @@ double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, bool 
     for (int r = 1; r < gs; ++r) if (load[r] < load[best]) best = r;
     owner2[ib] = best; load[best] += ib + 1;
   }
-  const double c1 = (2.0 * d + 12.0) / 64.0 * (i8 ? 2.5 : 1.0);
+  const double c1 = (2.0 * d + 12.0) / 64.0 * tile.phase1_scale;
   for (int cb = 0; cb < nblk; ++cb) {
     int best = 0;
     for (int r = 1; r < gs; ++r) if (load[r] < load[best]) best = r;
@@ -857,9 +671,9 @@ double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, bool 
   return mx * gs / tot;
 }
 
-int predict_group_size(int Npad, int num_sms, int variant, int requested, int d, long long Q, bool i8) {
-  if (variant != 2 || Npad / 64 > GROUP_MAX_BLOCKS) return 1;
-  const int BM = i8 ? 128 : 256, EB = i8 ? 7 : 8;      // queries per tile, panel bytes per (query, training point)
+int predict_group_size(int Npad, int num_sms, int requested, int d, long long Q, const GroupTile& tile) {
+  if (Npad / 64 > GROUP_MAX_BLOCKS) return 1;
+  const int BM = tile.bm, EB = tile.panel_bytes;      // queries per tile, panel bytes per (query, training point)
   // the grouped kernel carries 4.6 KB of static shared memory (ownership tables, kept means) on top of the one-tile
   // kernel's dynamic layout: from d = 28 the staged queries no longer fit beside the ring -> one tile per CTA
   if (VarCfg<256, 64, 4, 8>::smem_bytes(d) > 220 * 1024) return 1;
@@ -878,9 +692,9 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
       Gmin = 2;
       while (Gmin < 64 && (size_t)((num_sms + Gmin - 1) / Gmin) * BM * Npad * EB > ((size_t)80 << 20)) ++Gmin;
       for (int g = (Gmin / 2 > 2 ? Gmin / 2 : 2); g <= 64 && 2 * g <= nblk; ++g) {
-        double imb = plan_group_split(nblk, g, d, o2, o1, i8);
+        double imb = plan_group_split(nblk, g, d, o2, o1, tile);
         const int tail = num_sms % g;               // a smaller last group: weigh its imbalance by its share of the SMs
-        if (tail > 1) imb = (imb * (num_sms - tail) + plan_group_split(nblk, tail, d, o2, o1, i8) * tail) / num_sms;
+        if (tail > 1) imb = (imb * (num_sms - tail) + plan_group_split(nblk, tail, d, o2, o1, tile) * tail) / num_sms;
         else if (tail == 1) imb += 1.0 / num_sms;   // a lone CTA does whole tiles: fine, but it cannot share a panel
         const double score = imb + (g < Gmin ? 0.005 : 0.0) + 1e-4 * g;   // L2 fit is worth 0.5 % of balance; then small G
         if (score < bestS) { bestS = score; bestG = g; }
@@ -894,9 +708,9 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
       long long cap = num_sms / ntiles;
       if (cap > 64) cap = 64;
       if (cap > nblk / 2) cap = nblk / 2;
-      int fillG = bestG; double fillS = (bestG > 1) ? plan_group_split(nblk, bestG, d, o2, o1, i8) / bestG : 1.0;
+      int fillG = bestG; double fillS = (bestG > 1) ? plan_group_split(nblk, bestG, d, o2, o1, tile) / bestG : 1.0;
       for (int g = bestG + 1; g <= (int)cap; ++g) {
-        const double t = plan_group_split(nblk, g, d, o2, o1, i8) / g;      // time per tile ~ imbalance / ranks
+        const double t = plan_group_split(nblk, g, d, o2, o1, tile) / g;      // time per tile ~ imbalance / ranks
         if (t < fillS * 0.97) { fillS = t; fillG = g; }
       }
       bestG = fillG;
@@ -908,15 +722,15 @@ int predict_group_size(int Npad, int num_sms, int variant, int requested, int d,
   if (G > 64) G = 64;
   return G < 1 ? 1 : G;
 }
-// work-split tables for the kernel: [full group | last (smaller) group] x [phase-2 owner | phase-1 owner] x 128
-void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab, bool i8) {
+// work-split tables for the kernel: [full group | last (smaller) group] x [phase-2 owner | phase-1 owner] x GROUP_MAX_BLOCKS
+void predict_group_plan(int Npad, int num_sms, int G, int d, int* tab, const GroupTile& tile) {
   const int nblk = Npad / 64, tail = num_sms % G;
   for (int i = 0; i < 4 * GROUP_MAX_BLOCKS; ++i) tab[i] = 0;
-  plan_group_split(nblk, G, d, tab, tab + GROUP_MAX_BLOCKS, i8);
-  plan_group_split(nblk, tail > 0 ? tail : G, d, tab + 2 * GROUP_MAX_BLOCKS, tab + 3 * GROUP_MAX_BLOCKS, i8);
+  plan_group_split(nblk, G, d, tab, tab + GROUP_MAX_BLOCKS, tile);
+  plan_group_split(nblk, tail > 0 ? tail : G, d, tab + 2 * GROUP_MAX_BLOCKS, tab + 3 * GROUP_MAX_BLOCKS, tile);
 }
-size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, bool i8) {
-  return (size_t)2 * ((num_sms + G - 1) / G) * (i8 ? 128 * 7 : 256 * 8) * Npad;
+size_t predict_group_scratch_bytes(int Npad, int num_sms, int G, const GroupTile& tile) {
+  return (size_t)2 * ((num_sms + G - 1) / G) * (tile.bm * tile.panel_bytes) * Npad;
 }
 size_t predict_group_part_bytes(int Npad, int num_sms, int G) { return (size_t)((num_sms + G - 1) / G) * 4 * (Npad / 64) * 256 * 8; }
 
@@ -944,12 +758,11 @@ int launch_predict_var_grouped(const PredictParams& p, int num_sms, int G, cudaS
   return (int)e;
 }
 
-int launch_predict_var(const PredictParams& p, int num_sms, cudaStream_t st, int variant, int* launches) {
+int launch_predict_var(const PredictParams& p, int num_sms, cudaStream_t st, int* launches) {
   if (p.Q <= 0) return 0;
   if (launches) ++*launches;
-  if (variant == 2) return launch_var_t<256, 64, 4>(p, num_sms, st);
-  if (variant == 1) return launch_var_t<128, 128, 5>(p, num_sms, st);
-  return launch_var_t<64, 256, 4>(p, num_sms, st);
+  if (tile_bm(p.d) == 128) return launch_var_t<128, 128, 5>(p, num_sms, st);
+  return launch_var_t<256, 64, 4>(p, num_sms, st);
 }
 
 size_t predict_few_ws_bytes() { return (size_t)PREDICT_FEW_MAX * (FEW_MAX_SPLIT + 1) * 8 + PREDICT_FEW_MAX * sizeof(int); }

@@ -21,7 +21,7 @@
 //
 // Warps: 0-7 build the panel (phase 1) and run the per-block-row epilogue (tcgen05.ld, combine, W^2 row sums);
 // warp 8 lane 0 streams digit tiles with 1-D bulk TMA; warp 9 owns the TMEM allocation and its lane 0 issues MMAs.
-#include "apgp_internal.h"
+#include "predict_tile.cuh"
 #include <stdio.h>
 #include <stdlib.h>
 
@@ -29,7 +29,7 @@ namespace apgp {
 
 namespace {
 
-constexpr int I8_BM = 128, I8_BN = 64, I8_BK = 64, I8_NST = 2, I8_GROUP_MAX_BLOCKS = 128;
+constexpr int I8_BM = 128, I8_BN = 64, I8_BK = 64, I8_NST = 2;
 constexpr int I8_DIG = 7, I8_LEVELS = 8;
 constexpr int I8_A_STAGE = I8_DIG * I8_BM * I8_BK;      // bytes: 57344
 constexpr int I8_B_STAGE = I8_DIG * I8_BN * I8_BK;      // bytes: 28672
@@ -58,12 +58,6 @@ __device__ long long g_i8prof[I8_PROF_CTAS][I8_PROF_SLOTS];
 #endif
 
 size_t i8_smem_bytes(int d) { return (size_t)I8_RING + (size_t)d * I8_BM * 8 + 64 * 8 + 8 * 8 + 128; }
-
-__device__ __forceinline__ int ld_acquire_gpu_i8(const int* p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 
 // no-swizzle K-major shared-memory matrix descriptor (sm_100: version bits 46-48 = 0b001)
 __device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
@@ -158,6 +152,22 @@ __device__ __forceinline__ uint32_t gather_byte(const uint32_t (&lo)[4], const u
   return __byte_perm(__byte_perm(w[0], w[1], sel), __byte_perm(w[2], w[3], sel), 0x5410);
 }
 
+// phase 1's store (panel_columns): the four kernel values of m8 query block mg at columns jb + lane % 4 + {0, 4, 8, 12}
+// of 64-column block cb, as round(E 2^55) in the 7 digit planes of the block's A stage, most significant first; the
+// four values form one 32-bit word of each plane
+__device__ __forceinline__ void store_i8_panel(unsigned char* panel, int cb, int jb, int mg, int lane, const double (&e)[4]) {
+  uint32_t lo[4], hi[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const unsigned long long v = fixed55(e[j]);
+    lo[j] = (uint32_t)v; hi[j] = (uint32_t)(v >> 32);
+  }
+  uint32_t* dst = reinterpret_cast<uint32_t*>(panel + (size_t)cb * I8_A_STAGE + ((size_t)(jb >> 4) * 16 + mg) * 128 +
+                                              (lane >> 2) * 16 + (lane & 3) * 4);
+#pragma unroll
+  for (int pl = 0; pl < I8_DIG; ++pl) dst[pl * (4 * 16 * 128 / 4)] = gather_byte(lo, hi, 6 - pl);
+}
+
 __global__ void __launch_bounds__(I8_NTHREADS, 1)
 predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   constexpr int BM = I8_BM, BN = I8_BN, NCW = 8, NCONS = NCW * 32;
@@ -170,8 +180,8 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   uint64_t* stagebar = empty + I8_NST;
   uint64_t* accfull = stagebar + 1;
   uint64_t* accempty = accfull + 1;
-  __shared__ int owner_s[I8_GROUP_MAX_BLOCKS];
-  __shared__ int myblk_s[I8_GROUP_MAX_BLOCKS];
+  __shared__ int owner_s[GROUP_MAX_BLOCKS];
+  __shared__ int myblk_s[GROUP_MAX_BLOCKS];
   __shared__ int nmine_s;
   __shared__ double mu_keep[2][BM];
   __shared__ double ss_s[BM];
@@ -181,16 +191,9 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   I8P_T(tk);
   I8P_T(tp);
   I8P_T(tm);
-  const int d = p.d, Npad = p.Npad, nblk = Npad / BN;
-  const int grp = blockIdx.x / G, rank = blockIdx.x % G;
-  const int gs = min(G, (int)gridDim.x - grp * G);
-  const long long ntiles = (p.Q + BM - 1) / BM;
-  const long long t_begin = (ntiles * (long long)(grp * G) + gridDim.x - 1) / gridDim.x;
-  const long long t_end = (ntiles * (long long)(grp * G + gs) + gridDim.x - 1) / gridDim.x;
-  const int sl0 = BM * rank / gs, sl1 = BM * (rank + 1) / gs;
-  int* arrive = p.grp_arrive + grp;
-  double* part_mu = p.grp_part + (size_t)grp * 4 * nblk * BM;       // [2 buffers][nblk][BM]
-  double* part_ss = part_mu + (size_t)2 * nblk * BM;                // [2 buffers][nblk][BM]
+  const int Npad = p.Npad;
+  const GroupCtx<BM, BN> g(p, G);
+  const int nblk = g.nblk, rank = g.rank;
   unsigned char* scratch8 = reinterpret_cast<unsigned char*>(p.scratch);
 
   if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
@@ -206,15 +209,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
                  :: "r"(smem_u32(&tmem_base_s)) : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
   }
-  {
-    const int* tab = p.grp_plan + (gs == G ? 0 : 2 * I8_GROUP_MAX_BLOCKS);
-    for (int e = tid; e < nblk; e += blockDim.x) owner_s[e] = tab[e];
-    if (tid == 0) {
-      int n = 0;
-      for (int e = 0; e < nblk; ++e) if (tab[I8_GROUP_MAX_BLOCKS + e] == rank) myblk_s[n++] = e;
-      nmine_s = n;
-    }
-  }
+  g.load_plan(p, G, owner_s, myblk_s, &nmine_s);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -224,137 +219,26 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   uint32_t it = 0, nstaged = 0, nacc = 0;
   int nbar = 0;
 
-  for (long long tile = t_begin; tile <= t_end; ++tile) {
-    const int b = (int)((tile - t_begin) & 1);
-    const long long q0 = tile * BM;
-    const bool live = tile < t_end;
-    unsigned char* panel = scratch8 + ((size_t)grp * 2 + b) * BM * (size_t)Npad * I8_DIG;
+  for (long long tile = g.t_begin; tile <= g.t_end; ++tile) {
+    const int b = (int)((tile - g.t_begin) & 1);
+    const bool live = tile < g.t_end;
+    unsigned char* panel = scratch8 + ((size_t)g.grp * 2 + b) * BM * (size_t)Npad * I8_DIG;
     if (tid == 0 && live) { I8P_CNT(9, 1); I8P_CNT(10, nmine); }
 
     // ------------------------------------------------------------ phase 1: my column blocks of the digit panel
     if (live && warp < NCW) {
-      for (int e = tid; e < d * BM; e += NCONS) {
-        int i = e / BM, m = e - i * BM;
-        long long q = q0 + m;
-        qs[e] = (q < p.Q) ? p.Xq[q * d + i] * p.qscale[i] : 0.0;
-      }
-      double* stg = reinterpret_cast<double*>(ring);
-      const int CAPB = min(8, (I8_RING / 8 / (d + 1)) / BN);
-      const int JCHT = CAPB * BN;
-      constexpr int R = BM / (8 * NCW);
-      const int l = lane & 3, row = lane >> 2;
-      for (int s0 = 0; s0 < nmine; s0 += CAPB) {
-        const int ns = min(CAPB, nmine - s0);
-        named_bar_sync(1, NCONS);
-        if (tid == 0) {
-          mbar_arrive_expect_tx(stagebar, (uint32_t)((d + 1) * ns * BN * 8));
-          for (int sl = 0; sl < ns; ++sl) {
-            const int j0 = myblk_s[s0 + sl] * BN;
-            for (int i = 0; i < d; ++i) bulk_g2s(stg + i * JCHT + sl * BN, p.Xs + (size_t)i * Npad + j0, BN * 8, stagebar);
-            bulk_g2s(stg + d * JCHT + sl * BN, p.alphaA + j0, BN * 8, stagebar);
-          }
-        }
-        mbar_wait(stagebar, nstaged & 1u);
-        ++nstaged;
-        for (int sl = 0; sl < ns; ++sl) {
-          const int cb = myblk_s[s0 + sl];
-          const double* al = stg + d * JCHT + sl * BN;
-          unsigned char* pstage = panel + (size_t)cb * I8_A_STAGE;
-          double macc[R] = {};
-          for (int jb = 0; jb < BN; jb += 16) {
-            const int jj = jb + l;
-            double s[R][4] = {};
-            for (int i = 0; i < d; ++i) {
-              const double* xr = stg + i * JCHT + sl * BN + jj;
-              const double x0 = xr[0], x1 = xr[4], x2 = xr[8], x3 = xr[12];
-#pragma unroll
-              for (int r = 0; r < R; ++r) {
-                const double qv = qs[i * BM + (warp + r * NCW) * 8 + row];
-                const double d0 = x0 - qv, d1 = x1 - qv, d2 = x2 - qv, d3 = x3 - qv;
-                s[r][0] = fma(d0, d0, s[r][0]); s[r][1] = fma(d1, d1, s[r][1]);
-                s[r][2] = fma(d2, d2, s[r][2]); s[r][3] = fma(d3, d3, s[r][3]);
-              }
-            }
-            const double a0 = al[jj], a1 = al[jj + 4], a2 = al[jj + 8], a3 = al[jj + 12];
-#pragma unroll
-            for (int r = 0; r < R; ++r) {
-              const int mg = warp + r * NCW;
-              double ev[4];
-              ev[0] = exp_neg(s[r][0], etab); ev[1] = exp_neg(s[r][1], etab);
-              ev[2] = exp_neg(s[r][2], etab); ev[3] = exp_neg(s[r][3], etab);
-              macc[r] = fma(ev[0], a0, macc[r]); macc[r] = fma(ev[1], a1, macc[r]);
-              macc[r] = fma(ev[2], a2, macc[r]); macc[r] = fma(ev[3], a3, macc[r]);
-              uint32_t lo[4], hi[4];
-#pragma unroll
-              for (int j = 0; j < 4; ++j) {
-                const unsigned long long v = fixed55(ev[j]);
-                lo[j] = (uint32_t)v; hi[j] = (uint32_t)(v >> 32);
-              }
-              uint32_t* dst = reinterpret_cast<uint32_t*>(pstage + ((size_t)(jb >> 4) * 16 + mg) * 128 + row * 16 + l * 4);
-#pragma unroll
-              for (int pl = 0; pl < I8_DIG; ++pl) dst[pl * (4 * 16 * 128 / 4)] = gather_byte(lo, hi, 6 - pl);
-            }
-          }
-#pragma unroll
-          for (int r = 0; r < R; ++r) {
-            double v = macc[r];
-            v += __shfl_xor_sync(0xffffffffu, v, 1);
-            v += __shfl_xor_sync(0xffffffffu, v, 2);
-            if (l == 0) part_mu[((size_t)b * nblk + cb) * BM + (warp + r * NCW) * 8 + row] = v;
-          }
-        }
-      }
+      group_phase1<BM, BN, NCW>(p, tile * BM, qs, etab, reinterpret_cast<double*>(ring), I8_RING / 8, myblk_s, nmine,
+                                stagebar, nstaged, g.part_mu + (size_t)b * nblk * BM,
+                                [&](int cb, int jb, int mg, const double (&e)[4]) { store_i8_panel(panel, cb, jb, mg, lane, e); });
       __threadfence();
     }
     __syncthreads();
     if (tid == 0) I8P_ADD(0, tp);
 
-    // ------------------------------------------------------------ group barrier (one per tile)
-    if (tid == 0) {
-      ++nbar;
-      __threadfence();
-      atomicAdd(arrive, 1);
-      const int target = nbar * gs;
-      while (ld_acquire_gpu_i8(arrive) < target) __nanosleep(40);
-      __threadfence();
-      I8P_ADD(1, tp);
-    }
-    __syncthreads();
-    fence_proxy_async();
-
-    // ------------------------------------------------------------ finalise the previous tile, keep this tile's means
-    if (warp < NCW) {
-      const int m = sl0 + tid;
-      if (tid < sl1 - sl0) {
-        if (live) {
-          double mu = 0.0;
-          for (int cb = 0; cb < nblk; ++cb) mu += __ldcg(part_mu + ((size_t)b * nblk + cb) * BM + m);
-          mu_keep[b][tid] = mu;
-        }
-        if (tile > t_begin) {
-          const long long q = (tile - 1) * BM + m;
-          if (q < p.Q) {
-            double tot = 0.0;
-            for (int ib = 0; ib < nblk; ++ib) tot += __ldcg(part_ss + ((size_t)(b ^ 1) * nblk + ib) * BM + m);
-            const double mu = p.mean + mu_keep[b ^ 1][tid];
-            // a NaN query has NaN kernel values, which reach the mean but not the panel (fixed55 has no NaN digits)
-            const double var = isnan(mu) ? mu : p.amp - tot;
-            if (p.mu) p.mu[q] = mu;
-            if (p.var) p.var[q] = var;
-            if (p.util) {
-              bool ok = true;
-              if (p.has_box) {
-                for (int i = 0; i < d; ++i) {
-                  const double x = p.Xq[q * d + i];
-                  ok = ok && (x >= p.lo[i]) && (x <= p.hi[i]);
-                }
-              }
-              p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
-            }
-          }
-        }
-      }
-    }
+    g.barrier(nbar);
+    if (tid == 0) I8P_ADD(1, tp);
+    // a NaN query has NaN kernel values, which reach the mean but not the panel (fixed55 has no NaN digits)
+    g.finalise(p, tile, live, b, mu_keep, [&](double mu, double tot) { return isnan(mu) ? mu : p.amp - tot; });
     if (tid == 0) I8P_ADD(2, tp);
     if (!live) break;
 
@@ -444,7 +328,7 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
         tc_fence_before();
         if (half == 1) ss_s[m] = ss;
         named_bar_sync(1, NCONS);
-        if (half == 0) part_ss[((size_t)b * nblk + ib) * BM + m] = ss + ss_s[m];
+        if (half == 0) g.part_ss[((size_t)b * nblk + ib) * BM + m] = ss + ss_s[m];
         mbar_arrive(accempty);
       }
       __threadfence();
@@ -505,6 +389,12 @@ pack_linv_i8_kernel(const double* __restrict__ Linv, int ld, int N, double amp, 
 
 }  // namespace
 
+// The planner's unit for this engine is one 64-wide k-stage of a 128-query block-row on the int8 pipe; a panel block is
+// estimated at ~0.86 units at d = 5 (2.5 times the DMMA tile's estimate).  The -DAPGP_PROF phase profile
+// (profiles/r04_i8_phases_after.txt, cfg3) measures 3.5 units (a factor of 10); that value moves G at many padded
+// sizes that are not powers of two and has not been timed there, so the estimate stays until it has (DESIGN 4.1a)
+const GroupTile I8_GROUP_TILE = {I8_BM, I8_DIG, 2.5};
+
 size_t linv_i8_bytes(int Npad) {
   const size_t nblk = (size_t)Npad / I8_BN;
   return nblk * (nblk + 1) / 2 * I8_B_STAGE;
@@ -517,7 +407,7 @@ int launch_pack_linv_i8(const double* Linv, int ld, int N, int Npad, double amp,
 }
 
 bool predict_i8_fits(int Npad, int d) {
-  return Npad % I8_BN == 0 && Npad / I8_BN <= I8_GROUP_MAX_BLOCKS && i8_smem_bytes(d) <= 200 * 1024;
+  return Npad % I8_BN == 0 && Npad / I8_BN <= GROUP_MAX_BLOCKS && i8_smem_bytes(d) <= 200 * 1024;
 }
 
 int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches) {

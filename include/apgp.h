@@ -230,9 +230,6 @@ int apgp_debug_i8_operands(apgp_handle* h, unsigned char* linv_i8, double* rowsc
 int apgp_debug_pack_linv_i8(apgp_handle* h, const double* M, int n, double amp, unsigned char* out, double* rowscale);
 /* profiling builds (-DAPGP_PROF): read and reset 16 per-phase SM-cycle counters of the log-likelihood objective */
 int apgp_debug_read_prof(long long* out16);
-/* select the variance-kernel tiling (queries x L^-1 rows per CTA tile): 0 = 64x256, 1 = 128x128,
- * 2 = 256x64 (default).  Call before factorize. */
-int apgp_set_variant(apgp_handle* h, int variant);
 /* CTAs that share one query tile in the 256x64 variance kernel (their K* panels then stay in L2 instead of streaming
  * through HBM): 0 = one tile per CTA, -1 = automatic (by training-set size, and by the number of query tiles of the
  * call: a few-tile call is spread over more CTAs for latency), 2..64 = fixed group size.  Default -1. */
