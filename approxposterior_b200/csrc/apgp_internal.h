@@ -68,6 +68,7 @@ struct GroupTile {
   int bm;                  // queries per tile
   int panel_bytes;         // panel bytes per (query, training point)
   double phase1_scale;     // cost of building a 64-column panel block, relative to the DMMA tile's (plan_group_split)
+  int max_d;               // largest input dimension the kernel takes
 };
 extern const GroupTile DMMA_GROUP_TILE;   // predict_var_group_kernel, 256 x 64 (predict.cu)
 extern const GroupTile I8_GROUP_TILE;     // predict_var_i8_kernel, 128 x 64 (predict_i8.cu)

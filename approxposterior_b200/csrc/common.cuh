@@ -67,12 +67,10 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
 
 // ---------------------------------------------------------------------------------
 // Fragment-tiled storage of A * L^{-1} for the predict GEMM  W = K* . (A L^{-1})^T
-//   block-row ib (BN rows) x k-step kb (16 columns), only kb*16 < (ib+1)*BN stored.
+//   block-row ib (BN rows) x k-step kb (16 columns), only kb*16 < (ib+1)*BN stored: tile (ib, kb) is tile
+//   (BN/16) ib(ib+1)/2 + kb (stream_operands, pack_linv_kernel).
 //   inside a tile: [k4 (4)][n8 (BN/8)][lane (32)],  lane <-> (n = n8*8 + lane/4, k = k4*4 + lane%4)
 // ---------------------------------------------------------------------------------
-__host__ __device__ __forceinline__ long linvf_tile_index(int ib, int kb, int BN) {
-  return (long)(BN / 16) * ((long)ib * (ib + 1) / 2) + kb;
-}
 __host__ __device__ __forceinline__ long linvf_total_tiles(int Npad, int BN) {
   int nb = Npad / BN;
   return (long)(BN / 16) * ((long)nb * (nb + 1) / 2);

@@ -33,42 +33,116 @@ namespace {
 
 constexpr int BK = 16;
 
-// NCW consumer warps (warp tile 32x64) + 1 TMA producer warp.  NCW = 8: one CTA per SM (all shipped tilings).
-// NCW = 4 (two co-resident 128x64 CTAs per SM, so one CTA's panel phase overlaps the other's DMMA phase) was
-// measured: identical results, 0-2 % slower at every N (profiles/r01_schedules_tried/README.md).
-template <int BM, int BN, int NSTAGE, int NCW = 8>
+// 8 consumer warps (warp tile 32x64) + 1 TMA producer warp, one CTA per SM.  Four consumer warps (two co-resident
+// 128x64 CTAs per SM, so one CTA's panel phase overlaps the other's DMMA phase) were measured: identical results,
+// 0-2 % slower at every N (profiles/r01_schedules_tried/README.md).
+template <int BM, int BN, int NSTAGE>
 struct VarCfg {
-  static constexpr int NCONS_WARPS = NCW;
-  static constexpr int NCONS = NCW * 32;
+  static constexpr int NCONS_WARPS = 8;
+  static constexpr int NCONS = NCONS_WARPS * 32;
   static constexpr int NTHREADS = NCONS + 32;
-  static constexpr int CTAS_PER_SM = (NCW == 4) ? 2 : 1;
   static constexpr int WARPS_M = BM / 32;
   static constexpr int WARPS_N = BN / 64;
-  static_assert(WARPS_M * WARPS_N == NCW, "consumer warps x warp tile 32x64 must cover the CTA tile");
+  static_assert(WARPS_M * WARPS_N == NCONS_WARPS, "consumer warps x warp tile 32x64 must cover the CTA tile");
   static constexpr int A_TILE = BM * BK;                 // doubles
   static constexpr int B_TILE = BN * BK;
   static constexpr int STAGE = A_TILE + B_TILE;
   static constexpr int RING = NSTAGE * STAGE;            // doubles, reused as the phase-1 staging area
-  static size_t smem_bytes(int d) {
-    return (size_t)RING * 8 + (size_t)d * BM * 8 /*qs*/ + (size_t)BM * 8 /*mu_s*/ +
-           (size_t)WARPS_N * BM * 8 /*ss_s*/ + 64 * 8 /*exp table*/ + (2 * NSTAGE + 1) * 8 /*barriers*/ + 128;
+};
+
+// The DMMA kernels' dynamic shared memory, in this order: the operand ring, the scaled queries qs[d][BM], the tile's
+// means mu_s[BM] and per-column-warp row sums ss_s[WARPS_N][BM] (used by the one-tile kernel only), the 2^(j/64) table
+// etab[64] of exp_neg, the ring's full[NSTAGE] and empty[NSTAGE] mbarriers and phase 1's stagebar.
+template <int BM, int BN, int NSTAGE>
+struct VarSmem {
+  using C = VarCfg<BM, BN, NSTAGE>;
+  double *ring, *qs, *mu_s, *ss_s, *etab;
+  uint64_t *full, *empty, *stagebar;
+  __device__ __forceinline__ VarSmem(unsigned char* raw, int d)
+      : ring(reinterpret_cast<double*>(raw)), qs(ring + C::RING), mu_s(qs + (size_t)d * BM), ss_s(mu_s + BM),
+        etab(ss_s + C::WARPS_N * BM), full(reinterpret_cast<uint64_t*>(etab + 64)), empty(full + NSTAGE),
+        stagebar(empty + NSTAGE) {}
+  // the carve-up above in bytes, and 128 to spare
+  static constexpr size_t bytes(int d) {
+    return ((size_t)C::RING + (size_t)d * BM + BM + C::WARPS_N * BM + 64) * 8 + (2 * NSTAGE + 1) * 8 + 128;
   }
 };
 
-template <int BM, int BN, int NSTAGE, int NCW>
-__global__ void __launch_bounds__(NCW * 32 + 32, (NCW == 4) ? 2 : 1)
+// One block-row ib of phase 2 on the DMMA pipe: consume its (ib + 1) BN/16 k-stages from the ring, arriving on
+// empty[s] once per warp, into the 32x64 tile of W of warp (wm, wn) of the WARPS_M x WARPS_N consumer warps (the n8
+// fragments are interleaved over the column warps so that the diagonal block's zero skipping stays balanced), and
+// return in ss[mb] the sum of W^2 over this lane's fragments of m8 block mb.
+template <int BM, int BN, int NSTAGE>
+__device__ __forceinline__ void dmma_block_row(const double* ring, uint64_t* full, uint64_t* empty, uint32_t& it,
+                                               int ib, int wm, int wn, int lane, double (&ss)[4]) {
+  using C = VarCfg<BM, BN, NSTAGE>;
+  double acc[4][8][2];
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int b = 0; b < 8; ++b) { acc[a][b][0] = 0.0; acc[a][b][1] = 0.0; }
+  const int nk = (ib + 1) * (BN / BK);
+  const int kdiag = ib * (BN / BK);
+  for (int kb = 0; kb < nk; ++kb, ++it) {
+    const int s = it % NSTAGE;
+    const uint32_t ph = (it / NSTAGE) & 1u;
+    mbar_wait(&full[s], ph);
+    const double* As = ring + (size_t)s * C::STAGE + (wm * 4) * 32 + lane;
+    const double* Bs = ring + (size_t)s * C::STAGE + C::A_TILE + wn * 32 + lane;
+    if (kb < kdiag) {
+#pragma unroll
+      for (int k4 = 0; k4 < 4; ++k4) {
+        double a[4], b[8];
+#pragma unroll
+        for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
+#pragma unroll
+        for (int nb = 0; nb < 8; ++nb) b[nb] = Bs[(k4 * (BN / 8) + nb * C::WARPS_N) * 32];
+#pragma unroll
+        for (int mb = 0; mb < 4; ++mb)
+#pragma unroll
+          for (int nb = 0; nb < 8; ++nb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], b[nb]);
+      }
+    } else {
+      // diagonal block: n8 fragment (columns n0..n0+7 of W) only sees k <= n
+      const int kloc = (kb - kdiag) * BK;              // k offset inside the diagonal block
+#pragma unroll
+      for (int k4 = 0; k4 < 4; ++k4) {
+        double a[4];
+#pragma unroll
+        for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
+#pragma unroll
+        for (int nb = 0; nb < 8; ++nb) {
+          const int n0 = (nb * C::WARPS_N + wn) * 8;
+          if (kloc + k4 * 4 <= n0 + 7) {
+            const double b = Bs[(k4 * (BN / 8) + nb * C::WARPS_N) * 32];
+#pragma unroll
+            for (int mb = 0; mb < 4; ++mb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], b);
+          }
+        }
+      }
+    }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&empty[s]);
+  }
+#pragma unroll
+  for (int mb = 0; mb < 4; ++mb) {
+    double sacc = 0.0;
+#pragma unroll
+    for (int nb = 0; nb < 8; ++nb) {
+      sacc = fma(acc[mb][nb][0], acc[mb][nb][0], sacc);
+      sacc = fma(acc[mb][nb][1], acc[mb][nb][1], sacc);
+    }
+    ss[mb] = sacc;
+  }
+}
+
+template <int BM, int BN, int NSTAGE>
+__global__ void __launch_bounds__(VarCfg<BM, BN, NSTAGE>::NTHREADS, 1)
 predict_var_kernel(const __grid_constant__ PredictParams p) {
-  using C = VarCfg<BM, BN, NSTAGE, NCW>;
+  using C = VarCfg<BM, BN, NSTAGE>;
   constexpr int NCONS_WARPS = C::NCONS_WARPS, NCONS = C::NCONS;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  double* ring = reinterpret_cast<double*>(smem_raw);
-  double* qs = ring + C::RING;                          // [d][BM] scaled queries
-  double* mu_s = qs + (size_t)p.d * BM;                 // [BM]
-  double* ss_s = mu_s + BM;                             // [WARPS_N][BM]
-  double* etab = ss_s + C::WARPS_N * BM;                // [64] 2^(j/64) for exp_neg
-  uint64_t* full = reinterpret_cast<uint64_t*>(etab + 64);
-  uint64_t* empty = full + NSTAGE;
-  uint64_t* stagebar = empty + NSTAGE;                  // training-set staging (phase 1) completion
+  const VarSmem<BM, BN, NSTAGE> sm(smem_raw, p.d);
 
   const int tid = threadIdx.x;
   const int warp = tid >> 5, lane = tid & 31;
@@ -76,13 +150,7 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
   const int nblk = Npad / BN;
   const long long ntiles = (p.Q + BM - 1) / BM;
   double* panel = p.scratch + (size_t)blockIdx.x * BM * Npad;
-  if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
-
-  if (tid == 0) {
-    for (int s = 0; s < NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], NCONS_WARPS); }
-    mbar_init(stagebar, 1);
-    mbar_fence_init();
-  }
+  init_tile_smem<NSTAGE>(sm.etab, sm.full, sm.empty, sm.stagebar, NCONS_WARPS);
   __syncthreads();
 
   uint32_t it = 0;   // ring position, identical sequence in producer and consumers
@@ -93,120 +161,54 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
 
     // ------------------------------------------------------------ phase 1: K* panel + mean
     if (warp < NCONS_WARPS) {
-      stage_queries<BM, NCONS>(qs, p, d, q0, tid);
+      stage_queries<BM, NCONS>(sm.qs, p, d, q0, tid);
       // chunk of training columns staged in the (idle) ring: xs[d][JCH] + alpha[JCH]
       int JCH = (C::RING / (d + 1)) & ~15;
       if (JCH > Npad) JCH = Npad;
-      constexpr int R = BM / (8 * NCW);                // m8 blocks per warp
+      constexpr int R = BM / (8 * NCONS_WARPS);        // m8 blocks per warp
       double mu_part[R] = {};
       for (int j0 = 0; j0 < Npad; j0 += JCH) {
         const int jn = min(JCH, Npad - j0);
         named_bar_sync(1, NCONS);                      // previous chunk fully consumed / qs visible
         // TMA-staged training set: d rows of the scaled SoA inputs + the alpha row, one bulk copy each
         if (tid == 0) {
-          mbar_arrive_expect_tx(stagebar, (uint32_t)((d + 1) * jn * 8));
-          for (int i = 0; i < d; ++i) bulk_g2s(ring + i * JCH, p.Xs + (size_t)i * Npad + j0, jn * 8, stagebar);
-          bulk_g2s(ring + d * JCH, p.alphaA + j0, jn * 8, stagebar);
+          mbar_arrive_expect_tx(sm.stagebar, (uint32_t)((d + 1) * jn * 8));
+          for (int i = 0; i < d; ++i) bulk_g2s(sm.ring + i * JCH, p.Xs + (size_t)i * Npad + j0, jn * 8, sm.stagebar);
+          bulk_g2s(sm.ring + d * JCH, p.alphaA + j0, jn * 8, sm.stagebar);
         }
-        mbar_wait(stagebar, nstaged & 1u);
+        mbar_wait(sm.stagebar, nstaged & 1u);
         ++nstaged;
         double macc[R] = {};
-        panel_columns<BM, NCW>(ring, JCH, ring + d * JCH, jn, qs, d, etab, warp, lane, macc,
-                               [&](int jb, int mb, const double (&e)[4]) { store_dmma_panel<BM>(panel, j0 + jb, mb, lane, e); });
+        panel_columns<BM, NCONS_WARPS>(sm.ring, JCH, sm.ring + d * JCH, jn, sm.qs, d, sm.etab, warp, lane, macc,
+                                       [&](int jb, int mb, const double (&e)[4]) { store_dmma_panel<BM>(panel, j0 + jb, mb, lane, e); });
 #pragma unroll
         for (int r = 0; r < R; ++r) mu_part[r] += macc[r];
       }
-      store_row_sums<R, NCW>(mu_part, mu_s, warp, lane);
+      store_row_sums<R, NCONS_WARPS>(mu_part, sm.mu_s, warp, lane);
       fence_proxy_async();                             // panel stores -> visible to the TMA reads below
     }
     __syncthreads();
 
     // ------------------------------------------------------------ phase 2: triangular DMMA GEMM
     if (warp == NCONS_WARPS) {
-      if (lane == 0) {
-        for (int ib = 0; ib < nblk; ++ib) {
-          const int nk = (ib + 1) * (BN / BK);
-          const double* bsrc = p.LinvF + (size_t)linvf_tile_index(ib, 0, BN) * C::B_TILE;
-          for (int kb = 0; kb < nk; ++kb, ++it) {
-            const int s = it % NSTAGE;
-            const uint32_t ph = (it / NSTAGE) & 1u;
-            mbar_wait(&empty[s], ph ^ 1u);
-            double* dstA = ring + (size_t)s * C::STAGE;
-            mbar_arrive_expect_tx(&full[s], C::STAGE * 8);
-            bulk_g2s(dstA, panel + (size_t)kb * C::A_TILE, C::A_TILE * 8, &full[s]);
-            bulk_g2s(dstA + C::A_TILE, bsrc + (size_t)kb * C::B_TILE, C::B_TILE * 8, &full[s]);
-          }
-        }
-      }
+      if (lane == 0)
+        stream_operands<NSTAGE, C::A_TILE * 8, C::B_TILE * 8, BN / BK>(sm.ring, panel, p.LinvF, nblk, sm.full, sm.empty,
+                                                                        it, [](int) { return true; });
     } else {
       const int wm = warp / C::WARPS_N, wn = warp % C::WARPS_N;
       double rowss[4] = {0.0, 0.0, 0.0, 0.0};
       for (int ib = 0; ib < nblk; ++ib) {
-        double acc[4][8][2];
+        double ss[4];
+        dmma_block_row<BM, BN, NSTAGE>(sm.ring, sm.full, sm.empty, it, ib, wm, wn, lane, ss);
 #pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-          for (int b = 0; b < 8; ++b) { acc[a][b][0] = 0.0; acc[a][b][1] = 0.0; }
-        const int nk = (ib + 1) * (BN / BK);
-        const int kdiag = ib * (BN / BK);
-        for (int kb = 0; kb < nk; ++kb, ++it) {
-          const int s = it % NSTAGE;
-          const uint32_t ph = (it / NSTAGE) & 1u;
-          mbar_wait(&full[s], ph);
-          const double* As = ring + (size_t)s * C::STAGE + (wm * 4) * 32 + lane;
-          const double* Bs = ring + (size_t)s * C::STAGE + C::A_TILE + wn * 32 + lane;
-          if (kb < kdiag) {
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              double a[4], b[8];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
-#pragma unroll
-              for (int nb = 0; nb < 8; ++nb) b[nb] = Bs[(k4 * (BN / 8) + nb * C::WARPS_N) * 32];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb)
-#pragma unroll
-                for (int nb = 0; nb < 8; ++nb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], b[nb]);
-            }
-          } else {
-            // diagonal block: n8 fragment (columns n0..n0+7 of W) only sees k <= n
-            const int kloc = (kb - kdiag) * BK;          // k offset inside the diagonal block
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              double a[4];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
-#pragma unroll
-              for (int nb = 0; nb < 8; ++nb) {
-                const int n0 = (nb * C::WARPS_N + wn) * 8;
-                if (kloc + k4 * 4 <= n0 + 7) {
-                  const double b = Bs[(k4 * (BN / 8) + nb * C::WARPS_N) * 32];
-#pragma unroll
-                  for (int mb = 0; mb < 4; ++mb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], b);
-                }
-              }
-            }
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&empty[s]);
-        }
-#pragma unroll
-        for (int mb = 0; mb < 4; ++mb) {
-          double sacc = 0.0;
-#pragma unroll
-          for (int nb = 0; nb < 8; ++nb) {
-            sacc = fma(acc[mb][nb][0], acc[mb][nb][0], sacc);
-            sacc = fma(acc[mb][nb][1], acc[mb][nb][1], sacc);
-          }
-          rowss[mb] += sacc;
-        }
+        for (int mb = 0; mb < 4; ++mb) rowss[mb] += ss[mb];
       }
 #pragma unroll
       for (int mb = 0; mb < 4; ++mb) {
         double v = rowss[mb];
         v += __shfl_xor_sync(0xffffffffu, v, 1);
         v += __shfl_xor_sync(0xffffffffu, v, 2);
-        if ((lane & 3) == 0) ss_s[wn * BM + wm * 32 + mb * 8 + (lane >> 2)] = v;
+        if ((lane & 3) == 0) sm.ss_s[wn * BM + wm * 32 + mb * 8 + (lane >> 2)] = v;
       }
       named_bar_sync(1, NCONS);
       if (tid < BM) {
@@ -214,8 +216,8 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
         if (q < p.Q) {
           double tot = 0.0;
 #pragma unroll
-          for (int w = 0; w < C::WARPS_N; ++w) tot += ss_s[w * BM + tid];
-          write_query(p, d, q, p.mean + mu_s[tid], p.amp - tot);
+          for (int w = 0; w < C::WARPS_N; ++w) tot += sm.ss_s[w * BM + tid];
+          write_query(p, d, q, p.mean + sm.mu_s[tid], p.amp - tot);
         }
       }
     }
@@ -244,18 +246,13 @@ predict_var_kernel(const __grid_constant__ PredictParams p) {
 // length-N sum (tests/test_gpu_parity.py::test_grouped_variance_kernel_matches_one_tile_per_cta).
 // ---------------------------------------------------------------------------------------------
 template <int BM, int BN, int NSTAGE>
-__global__ void __launch_bounds__(8 * 32 + 32, 1)
+__global__ void __launch_bounds__(VarCfg<BM, BN, NSTAGE>::NTHREADS, 1)
 predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
-  using C = VarCfg<BM, BN, NSTAGE, 8>;
-  constexpr int NCW = 8;
+  using C = VarCfg<BM, BN, NSTAGE>;
+  constexpr int NCW = C::NCONS_WARPS;
   static_assert(C::WARPS_N == 1, "grouped kernel is written for the 256x64 tiling");
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  double* ring = reinterpret_cast<double*>(smem_raw);
-  double* qs = ring + C::RING;                          // [d][BM] scaled queries
-  double* etab = qs + (size_t)p.d * BM + 2 * BM;        // [64] (same carve-up as predict_var_kernel: VarCfg::smem_bytes)
-  uint64_t* full = reinterpret_cast<uint64_t*>(etab + 64);
-  uint64_t* empty = full + NSTAGE;
-  uint64_t* stagebar = empty + NSTAGE;
+  const VarSmem<BM, BN, NSTAGE> sm(smem_raw, p.d);
   __shared__ int owner_s[GROUP_MAX_BLOCKS];             // block-row of L^-1 (phase 2) -> rank
   __shared__ int myblk_s[GROUP_MAX_BLOCKS];             // the 64-column blocks of the panel this rank builds (phase 1)
   __shared__ int nmine_s;
@@ -266,12 +263,7 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
   const GroupCtx<BM, BN> g(p, G);
   const int nblk = g.nblk, rank = g.rank;
 
-  if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
-  if (tid == 0) {
-    for (int s = 0; s < NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], NCW); }
-    mbar_init(stagebar, 1);
-    mbar_fence_init();
-  }
+  init_tile_smem<NSTAGE>(sm.etab, sm.full, sm.empty, sm.stagebar, NCW);
   g.load_plan(p, G, owner_s, myblk_s, &nmine_s);
   __syncthreads();
   const int nmine = nmine_s;
@@ -286,7 +278,7 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
 
     // ------------------------------------------------------------ phase 1: my column blocks of the panel
     if (live && warp < NCW) {
-      group_phase1<BM, BN, NCW>(p, tile * BM, qs, etab, ring, C::RING, myblk_s, nmine, stagebar, nstaged,
+      group_phase1<BM, BN, NCW>(p, tile * BM, sm.qs, sm.etab, sm.ring, C::RING, myblk_s, nmine, sm.stagebar, nstaged,
                                 g.part_mu + (size_t)b * nblk * BM, [&](int cb, int jb, int mb, const double (&e)[4]) {
                                   store_dmma_panel<BM>(panel, cb * BN + jb, mb, lane, e);
                                 });
@@ -300,83 +292,20 @@ predict_var_group_kernel(const __grid_constant__ PredictParams p, const int G) {
 
     // ------------------------------------------------------------ phase 2: my block-rows of the triangular GEMM
     if (warp == NCW) {
-      if (lane == 0) {
-        for (int ib = 0; ib < nblk; ++ib) {
-          if (owner_s[ib] != rank) continue;
-          const int nk = (ib + 1) * (BN / BK);
-          const double* bsrc = p.LinvF + (size_t)linvf_tile_index(ib, 0, BN) * C::B_TILE;
-          for (int kb = 0; kb < nk; ++kb, ++it) {
-            const int s = it % NSTAGE;
-            const uint32_t ph = (it / NSTAGE) & 1u;
-            mbar_wait(&empty[s], ph ^ 1u);
-            double* dstA = ring + (size_t)s * C::STAGE;
-            mbar_arrive_expect_tx(&full[s], C::STAGE * 8);
-            bulk_g2s(dstA, panel + (size_t)kb * C::A_TILE, C::A_TILE * 8, &full[s]);
-            bulk_g2s(dstA + C::A_TILE, bsrc + (size_t)kb * C::B_TILE, C::B_TILE * 8, &full[s]);
-          }
-        }
-      }
+      if (lane == 0)
+        stream_operands<NSTAGE, C::A_TILE * 8, C::B_TILE * 8, BN / BK>(sm.ring, panel, p.LinvF, nblk, sm.full, sm.empty,
+                                                                        it, [&](int ib) { return owner_s[ib] == rank; });
     } else {
-      const int wm = warp;
       for (int ib = 0; ib < nblk; ++ib) {
         if (owner_s[ib] != rank) continue;
-        double acc[4][8][2];
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-          for (int c = 0; c < 8; ++c) { acc[a][c][0] = 0.0; acc[a][c][1] = 0.0; }
-        const int nk = (ib + 1) * (BN / BK);
-        const int kdiag = ib * (BN / BK);
-        for (int kb = 0; kb < nk; ++kb, ++it) {
-          const int s = it % NSTAGE;
-          const uint32_t ph = (it / NSTAGE) & 1u;
-          mbar_wait(&full[s], ph);
-          const double* As = ring + (size_t)s * C::STAGE + (wm * 4) * 32 + lane;
-          const double* Bs = ring + (size_t)s * C::STAGE + C::A_TILE + lane;
-          if (kb < kdiag) {
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              double a[4], bb[8];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
-#pragma unroll
-              for (int nb = 0; nb < 8; ++nb) bb[nb] = Bs[(k4 * (BN / 8) + nb) * 32];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb)
-#pragma unroll
-                for (int nb = 0; nb < 8; ++nb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], bb[nb]);
-            }
-          } else {
-            const int kloc = (kb - kdiag) * BK;
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              double a[4];
-#pragma unroll
-              for (int mb = 0; mb < 4; ++mb) a[mb] = As[(k4 * (BM / 8) + mb) * 32];
-#pragma unroll
-              for (int nb = 0; nb < 8; ++nb) {
-                if (kloc + k4 * 4 <= nb * 8 + 7) {
-                  const double bv = Bs[(k4 * (BN / 8) + nb) * 32];
-#pragma unroll
-                  for (int mb = 0; mb < 4; ++mb) dmma884(acc[mb][nb][0], acc[mb][nb][1], a[mb], bv);
-                }
-              }
-            }
-          }
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&empty[s]);
-        }
+        double ss[4];
+        dmma_block_row<BM, BN, NSTAGE>(sm.ring, sm.full, sm.empty, it, ib, warp, 0, lane, ss);
 #pragma unroll
         for (int mb = 0; mb < 4; ++mb) {                 // this block-row's contribution to rowsum(W^2)
-          double sacc = 0.0;
-#pragma unroll
-          for (int nb = 0; nb < 8; ++nb) {
-            sacc = fma(acc[mb][nb][0], acc[mb][nb][0], sacc);
-            sacc = fma(acc[mb][nb][1], acc[mb][nb][1], sacc);
-          }
-          sacc += __shfl_xor_sync(0xffffffffu, sacc, 1);
-          sacc += __shfl_xor_sync(0xffffffffu, sacc, 2);
-          if ((lane & 3) == 0) g.part_ss[((size_t)b * nblk + ib) * BM + wm * 32 + mb * 8 + (lane >> 2)] = sacc;
+          double v = ss[mb];
+          v += __shfl_xor_sync(0xffffffffu, v, 1);
+          v += __shfl_xor_sync(0xffffffffu, v, 2);
+          if ((lane & 3) == 0) g.part_ss[((size_t)b * nblk + ib) * BM + warp * 32 + mb * 8 + (lane >> 2)] = v;
         }
       }
       __threadfence();                                   // partial row sums visible before the next barrier's arrival
@@ -614,24 +543,25 @@ __global__ void exp_neg_test_kernel(const double* __restrict__ s, int n, double*
     out[i] = variant ? exp_neg256(s[i], tab) : exp_neg(s[i], tab);
 }
 
-template <int BM, int BN, int NSTAGE, int NCW = 8>
+template <int BM, int BN, int NSTAGE>
 int launch_var_t(const PredictParams& p, int num_sms, cudaStream_t st) {
-  using C = VarCfg<BM, BN, NSTAGE, NCW>;
-  const size_t smem = C::smem_bytes(p.d);
+  const size_t smem = VarSmem<BM, BN, NSTAGE>::bytes(p.d);
   static PerDeviceOnce attr;
   if (attr.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(predict_var_kernel<BM, BN, NSTAGE, NCW>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 / C::CTAS_PER_SM);
+    cudaError_t e = cudaFuncSetAttribute(predict_var_kernel<BM, BN, NSTAGE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         227 * 1024);
     if (e != cudaSuccess) return (int)e;
     attr.mark();
   }
   long long ntiles = (p.Q + BM - 1) / BM;
-  const long long cap = (long long)num_sms * C::CTAS_PER_SM;
-  int grid = (int)(ntiles < cap ? ntiles : cap);
+  int grid = (int)(ntiles < num_sms ? ntiles : num_sms);
   if (grid < 1) return 0;
-  predict_var_kernel<BM, BN, NSTAGE, NCW><<<grid, C::NTHREADS, smem, st>>>(p);
+  predict_var_kernel<BM, BN, NSTAGE><<<grid, VarCfg<BM, BN, NSTAGE>::NTHREADS, smem, st>>>(p);
   return (int)cudaGetLastError();
 }
+
+// the grouped kernel's dynamic shared memory opt-in; its 4.6 KB of static tables (ownership, kept means) come on top
+constexpr int GROUP_SMEM = 220 * 1024;
 
 }  // namespace
 
@@ -650,7 +580,13 @@ size_t predict_scratch_bytes(int Npad, int num_sms, int d) { return (size_t)num_
 // the panel costs (2d + 12)/64 of a unit (exp + distances on the same FP64 pipe); the blocks go, one by one, to the
 // rank with the least combined load, which also evens out what phase 2 could not.  Returns max load / mean load.
 // Other engines scale that phase-1 cost by their tile's phase1_scale.
-const GroupTile DMMA_GROUP_TILE = {256, 8, 1.0};
+// The grouped kernel takes d up to 27: from d = 28 the staged queries no longer fit beside the ring in GROUP_SMEM.
+constexpr int dmma_group_max_d() {
+  int d = 1;
+  while (VarSmem<256, 64, 4>::bytes(d + 1) <= GROUP_SMEM) ++d;
+  return d;
+}
+const GroupTile DMMA_GROUP_TILE = {256, 8, 1.0, dmma_group_max_d()};
 
 double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, const GroupTile& tile) {
   double load[64];
@@ -673,10 +609,8 @@ double plan_group_split(int nblk, int gs, int d, int* owner2, int* owner1, const
 
 int predict_group_size(int Npad, int num_sms, int requested, int d, long long Q, const GroupTile& tile) {
   if (Npad / 64 > GROUP_MAX_BLOCKS) return 1;
+  if (d > tile.max_d) return 1;
   const int BM = tile.bm, EB = tile.panel_bytes;      // queries per tile, panel bytes per (query, training point)
-  // the grouped kernel carries 4.6 KB of static shared memory (ownership tables, kept means) on top of the one-tile
-  // kernel's dynamic layout: from d = 28 the staged queries no longer fit beside the ring -> one tile per CTA
-  if (VarCfg<256, 64, 4, 8>::smem_bytes(d) > 220 * 1024) return 1;
   const int nblk = Npad / 64;
   int G = requested;
   if (G < 0) {
@@ -736,26 +670,15 @@ size_t predict_group_part_bytes(int Npad, int num_sms, int G) { return (size_t)(
 
 int launch_predict_var_grouped(const PredictParams& p, int num_sms, int G, cudaStream_t st, int* launches) {
   if (p.Q <= 0) return 0;
-  using C = VarCfg<256, 64, 4, 8>;
-  const size_t smem = C::smem_bytes(p.d);
   static PerDeviceOnce attr;
   if (attr.needed()) {
-    cudaError_t e = cudaFuncSetAttribute(predict_var_group_kernel<256, 64, 4>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(predict_var_group_kernel<256, 64, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         GROUP_SMEM);
     if (e != cudaSuccess) return (int)e;
     attr.mark();
   }
-  const int ngroups = (num_sms + G - 1) / G;
-  cudaError_t e = cudaMemsetAsync(p.grp_arrive, 0, sizeof(int) * ngroups, st);
-  if (e != cudaSuccess) return (int)e;
-  // the group barrier spins: every CTA of the grid must be resident at once -> cooperative launch (one CTA per SM)
-  PredictParams pc = p;
-  int Gc = G;
-  void* args[] = {(void*)&pc, (void*)&Gc};
-  e = cudaLaunchCooperativeKernel((const void*)predict_var_group_kernel<256, 64, 4>, dim3(num_sms), dim3(C::NTHREADS),
-                                  args, smem, st);
-  if (launches) ++*launches;
-  return (int)e;
+  return launch_grouped((const void*)predict_var_group_kernel<256, 64, 4>, p, num_sms, G, VarCfg<256, 64, 4>::NTHREADS,
+                        VarSmem<256, 64, 4>::bytes(p.d), st, launches);
 }
 
 int launch_predict_var(const PredictParams& p, int num_sms, cudaStream_t st, int* launches) {

@@ -196,14 +196,11 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
   const int nblk = g.nblk, rank = g.rank;
   unsigned char* scratch8 = reinterpret_cast<unsigned char*>(p.scratch);
 
-  if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
-  if (tid == 0) {
-    for (int s = 0; s < I8_NST; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    mbar_init(stagebar, 1);
+  if (tid == 0) {                                        // before init_tile_smem, whose fence covers these too
     mbar_init(accfull, 1);
     mbar_init(accempty, NCONS);
-    mbar_fence_init();
   }
+  init_tile_smem<I8_NST>(etab, full, empty, stagebar, 1);   // empty[s]: one tcgen05.commit per stage
   if (warp == 9) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;\n"
                  :: "r"(smem_u32(&tmem_base_s)) : "memory");
@@ -244,21 +241,9 @@ predict_var_i8_kernel(const __grid_constant__ PredictParams p, const int G) {
 
     // ------------------------------------------------------------ phase 2: my block-rows on the int8 tensor cores
     if (warp == NCW) {
-      if (lane == 0) {
-        for (int ib = 0; ib < nblk; ++ib) {
-          if (owner_s[ib] != rank) continue;
-          const unsigned char* bsrc = p.LinvI8 + ((size_t)ib * (ib + 1) / 2) * I8_B_STAGE;
-          for (int kb = 0; kb <= ib; ++kb, ++it) {
-            const int s = it % I8_NST;
-            const uint32_t ph = (it / I8_NST) & 1u;
-            mbar_wait(&empty[s], ph ^ 1u);
-            unsigned char* dst = ring + (size_t)s * I8_STAGE;
-            mbar_arrive_expect_tx(&full[s], I8_STAGE);
-            bulk_g2s(dst, panel + (size_t)kb * I8_A_STAGE, I8_A_STAGE, &full[s]);
-            bulk_g2s(dst + I8_A_STAGE, bsrc + (size_t)kb * I8_B_STAGE, I8_B_STAGE, &full[s]);
-          }
-        }
-      }
+      if (lane == 0)
+        stream_operands<I8_NST, I8_A_STAGE, I8_B_STAGE, 1>(ring, panel, p.LinvI8, nblk, full, empty, it,
+                                                           [&](int ib) { return owner_s[ib] == rank; });
     } else if (warp == NCW + 1) {
       if (lane == 0) {
         I8P_SET(tm);
@@ -393,7 +378,9 @@ pack_linv_i8_kernel(const double* __restrict__ Linv, int ld, int N, double amp, 
 // estimated at ~0.86 units at d = 5 (2.5 times the DMMA tile's estimate).  The -DAPGP_PROF phase profile
 // (profiles/r04_i8_phases_after.txt, cfg3) measures 3.5 units (a factor of 10); that value moves G at many padded
 // sizes that are not powers of two and has not been timed there, so the estimate stays until it has (DESIGN 4.1a)
-const GroupTile I8_GROUP_TILE = {I8_BM, I8_DIG, 2.5};
+// The largest d is the DMMA tile's 27, the engine's range since it was introduced: its own shared memory would take d up
+// to 31 (predict_i8_fits), but the engine has not been tested or timed beyond 27.
+const GroupTile I8_GROUP_TILE = {I8_BM, I8_DIG, 2.5, 27};
 
 size_t linv_i8_bytes(int Npad) {
   const size_t nblk = (size_t)Npad / I8_BN;
@@ -420,14 +407,7 @@ int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream
     if (e != cudaSuccess) return (int)e;
     attr.mark();
   }
-  const int ngroups = (num_sms + G - 1) / G;
-  cudaError_t e = cudaMemsetAsync(p.grp_arrive, 0, sizeof(int) * ngroups, st);
-  if (e != cudaSuccess) return (int)e;
-  PredictParams pc = p;
-  int Gc = G;
-  void* args[] = {(void*)&pc, (void*)&Gc};
-  e = cudaLaunchCooperativeKernel((const void*)predict_var_i8_kernel, dim3(num_sms), dim3(I8_NTHREADS), args, smem, st);
-  if (launches) ++*launches;
+  const int e = launch_grouped((const void*)predict_var_i8_kernel, p, num_sms, G, I8_NTHREADS, smem, st, launches);
 #ifdef APGP_PROF
   if (getenv("APGP_PROF_PRINT")) {
     cudaStreamSynchronize(st);
@@ -442,7 +422,7 @@ int launch_predict_var_i8(const PredictParams& p, int num_sms, int G, cudaStream
     cudaMemcpyToSymbol(g_i8prof, z, sizeof(z));
   }
 #endif
-  return (int)e;
+  return e;
 }
 
 }  // namespace apgp

@@ -4,7 +4,10 @@
 // Phase 1 -- the kernel values E[q,j] of a query tile, their contribution to the mean, and the panel that phase 2
 // multiplies -- is written once here.  The kernels differ only in how they store the panel (a store functor), so
 // all three compute the same E and the same mean in the same order: the int8 engine's mean is the DMMA engine's mean
-// by construction.  The grouped kernels also share their group scaffold (GroupCtx) and the per-query output.
+// by construction.  Phase 2's operand stream (stream_operands: panel and B operand through the mbarrier ring) is
+// shared too; the kernels differ in the stage sizes and in how they consume a stage (the two DMMA kernels share one
+// block-row, dmma_block_row in predict.cu).  The grouped kernels also share their group scaffold (GroupCtx, and
+// launch_grouped on the host) and the per-query output.
 #pragma once
 #include "apgp_internal.h"
 
@@ -89,6 +92,46 @@ __device__ __forceinline__ void write_query(const PredictParams& p, int d, long 
       }
     }
     p.util[q] = ok ? utility_eval(p.utility_kind, mu, var, p.ybest, p.zeta) : INFINITY;
+  }
+}
+
+// The prologue every tiled kernel shares: the 2^(j/64) table of exp_neg, and the mbarriers of the NSTAGE operand ring
+// (full: the producer's expect_tx; empty: ncons consumer arrivals) and of phase 1's training-set staging.  The fence
+// also covers barriers the caller initialised before it.  The caller synchronises the CTA afterwards.
+template <int NSTAGE>
+__device__ __forceinline__ void init_tile_smem(double* etab, uint64_t* full, uint64_t* empty, uint64_t* stagebar,
+                                               uint32_t ncons) {
+  const int tid = threadIdx.x;
+  if (tid < 64) etab[tid] = exp2((double)tid * (1.0 / 64.0));
+  if (tid == 0) {
+    for (int s = 0; s < NSTAGE; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], ncons); }
+    mbar_init(stagebar, 1);
+    mbar_fence_init();
+  }
+}
+
+// Phase 2's operand stream, run by the producer lane: for every block-row ib with mine(ib), its (ib + 1) KPB k-stages
+// (KPB per block-row height) through the NSTAGE ring, each one A_BYTES of the panel a followed by B_BYTES of the
+// block-row's B operand, which starts KPB ib(ib + 1)/2 stages into b.  it: the ring position, advanced in the same
+// sequence by the consumers.
+template <int NSTAGE, int A_BYTES, int B_BYTES, int KPB, class Mine>
+__device__ __forceinline__ void stream_operands(void* ring, const void* a, const void* b, int nblk, uint64_t* full,
+                                                uint64_t* empty, uint32_t& it, Mine&& mine) {
+  unsigned char* const ring8 = static_cast<unsigned char*>(ring);
+  const unsigned char* const a8 = static_cast<const unsigned char*>(a);
+  for (int ib = 0; ib < nblk; ++ib) {
+    if (!mine(ib)) continue;
+    const int nk = (ib + 1) * KPB;
+    const unsigned char* bsrc = static_cast<const unsigned char*>(b) + (size_t)KPB * ((size_t)ib * (ib + 1) / 2) * B_BYTES;
+    for (int kb = 0; kb < nk; ++kb, ++it) {
+      const int s = it % NSTAGE;
+      const uint32_t ph = (it / NSTAGE) & 1u;
+      mbar_wait(&empty[s], ph ^ 1u);
+      unsigned char* dst = ring8 + (size_t)s * (A_BYTES + B_BYTES);
+      mbar_arrive_expect_tx(&full[s], A_BYTES + B_BYTES);
+      bulk_g2s(dst, a8 + (size_t)kb * A_BYTES, A_BYTES, &full[s]);
+      bulk_g2s(dst + A_BYTES, bsrc + (size_t)kb * B_BYTES, B_BYTES, &full[s]);
+    }
   }
 }
 
@@ -216,6 +259,22 @@ __device__ __forceinline__ void group_phase1(const PredictParams& p, long long q
       store_row_sums<R, NCW>(macc, part_mu + (size_t)cb * BM, warp, lane);   // this block's contribution to the means
     }
   }
+}
+
+// Host side of the group scaffold: zero the groups' barrier counters and launch kernel(p, G) with one CTA per SM.  The
+// group barrier spins, so every CTA of the grid must be resident at once: a cooperative launch, which is refused
+// rather than left to deadlock when they cannot be.
+inline int launch_grouped(const void* kernel, const PredictParams& p, int num_sms, int G, int nthreads, size_t smem,
+                          cudaStream_t st, int* launches) {
+  const int ngroups = (num_sms + G - 1) / G;
+  cudaError_t e = cudaMemsetAsync(p.grp_arrive, 0, sizeof(int) * ngroups, st);
+  if (e != cudaSuccess) return (int)e;
+  PredictParams pc = p;
+  int Gc = G;
+  void* args[] = {(void*)&pc, (void*)&Gc};
+  e = cudaLaunchCooperativeKernel(kernel, dim3(num_sms), dim3(nthreads), args, smem, st);
+  if (launches) ++*launches;
+  return (int)e;
 }
 
 }  // namespace apgp
