@@ -84,6 +84,7 @@ _SIGNATURES = {
     "apgp_debug_read_prof": (C.c_int, [C.c_void_p]),
     "apgp_debug_group_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]),
     "apgp_debug_last_var_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
+    "apgp_debug_last_loglik_path": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "apgp_debug_i8_operands": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),
     "apgp_debug_pack_linv_i8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_void_p, C.c_void_p]),
 }

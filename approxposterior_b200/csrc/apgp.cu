@@ -78,6 +78,7 @@ struct apgp_handle {
   int plan_Npad = -1, plan_G = -1, plan_d = -1, plan_i8 = -1;   // what g_plan currently holds
   DevBuf LinvI8, i8scale;              // int8 engine operands (pack_linv_i8)
   int last_var_path = 0;               // VarPath of the last variance launch (apgp_debug_last_var_path)
+  int last_loglik_path = 0;            // LoglikPath of the last apgp_loglik_batch call (apgp_debug_last_loglik_path)
 };
 
 namespace {
@@ -102,6 +103,24 @@ void read_env_knobs(apgp_handle* h) {
 void fill_hyper_row(double* row, double mean, double amp, double wn, const double* logM, int d) {
   row[0] = mean; row[1] = amp; row[2] = exp(wn) + TINY2;
   for (int i = 0; i < d; ++i) row[3 + i] = exp(-logM[i]);
+}
+
+// apgp_loglik_batch's kernels, as apgp_debug_last_loglik_path reports them
+enum LoglikPath { LL_SMALL = 1, LL_GROUP = 2, LL_TILED = 3 };
+// One restart per CTA while the small evaluator fits one CTA's shared memory (N <= ~224), else one CLUSTER per restart
+// (fused single launch, chol_group.cuh) -- except a handful of large matrices, which the multi-launch tiled sequence
+// spreads over the whole GPU where a cluster is at most 16 SMs (measured, R = 1: N = 1024 0.51 ms fused vs 0.71 ms tiled,
+// N = 2048 1.85 vs 1.48 ms; R = 8, N = 2048: 2.87 vs 2.73).  APGP_LOGLIK_PATH = small | group | tiled overrides (small
+// only where it fits).
+int choose_loglik_path(const apgp_handle* h, int R) {
+  const bool fits = loglik_small_smem(h->N, h->d) <= 220 * 1024;
+  if (const char* v = getenv("APGP_LOGLIK_PATH")) {
+    if (!strcmp(v, "small") && fits) return LL_SMALL;
+    if (!strcmp(v, "group")) return LL_GROUP;
+    if (!strcmp(v, "tiled")) return LL_TILED;
+  }
+  if (fits) return LL_SMALL;
+  return (h->Np >= 2048 && R <= 8) ? LL_TILED : LL_GROUP;
 }
 
 }  // namespace
@@ -169,6 +188,7 @@ int apgp_reset(apgp_handle* h) {
   h->plan_Npad = h->plan_G = h->plan_d = h->plan_i8 = -1;
   h->i8_packed = false;
   h->last_var_path = 0;
+  h->last_loglik_path = 0;
   h->group = -1; h->predict_few = true; h->var_i8 = true;   // tuning knobs back to their defaults (as apgp_create)
   read_env_knobs(h);
   if (h->comm) { comm_destroy(h->comm); h->comm = nullptr; h->comm_rank = 0; h->comm_world = 1; }
@@ -593,26 +613,17 @@ int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fi
   const int d = h->d, N = h->N, Np = h->Np;
   if (P != 1 + (fit_amp ? 1 : 0) + d) return fail(APGP_ERR_ARG, "apgp_loglik_batch: P != 1 + fit_amp + d");
   if (R < 1) return APGP_OK;
+  const int path = choose_loglik_path(h, R);
+  if (grad_host && path != LL_SMALL) return APGP_NEEDS_HOST;    // batched gradients come from the small kernel only
+  h->last_loglik_path = path;
   Guard g(h->device);
-  // three paths: one restart per CTA in shared memory (N <= ~224); one CLUSTER per restart with the matrix in L2
-  // (fused single launch, chol_group.cuh); the multi-launch tiled sequence (APGP_LOGLIK_PATH=tiled, kept for A/B runs)
-  const char* pathv = getenv("APGP_LOGLIK_PATH");
-  const bool force_tiled = getenv("APGP_LOGLIK_TILED") || (pathv && !strcmp(pathv, "tiled"));
-  const bool force_group = pathv && !strcmp(pathv, "group");
-  const bool small = loglik_small_smem(N, d) <= 220 * 1024 && !force_tiled && !force_group;
-  // a handful of large matrices: the multi-launch tiled sequence spreads each one over the whole GPU, a cluster is at most
-  // 16 SMs (measured, R = 1: N = 1024 0.51 ms fused vs 0.71 ms tiled, N = 2048 1.85 vs 1.48 ms; R = 8, N = 2048: 2.87 vs 2.73)
-  const bool few_large = Np >= 2048 && R <= 8 && !force_group;
-  const bool group = !small && !force_tiled && !few_large;
-  if (grad_host && !small)
-    return fail(APGP_ERR_ARG, "apgp_loglik_batch: batched gradients need the shared-memory path (N <= ~224); "
-                              "use apgp_grad_log_likelihood per vector");
+  const double noise = exp(white_noise) + TINY2;
   // chunk the restart axis so the tiled path's workspace stays below ~4 GiB
   size_t per = (size_t)Np * Np * 8;
-  int Rc = small ? R : (int)((4ull << 30) / per); if (Rc < 1) Rc = 1; if (Rc > R) Rc = R;
-  if (group) {
+  int Rc = (path == LL_SMALL) ? R : (int)((4ull << 30) / per); if (Rc < 1) Rc = 1; if (Rc > R) Rc = R;
+  if (path == LL_GROUP) {
     CUI(h->gws.reserve(chol_group_ws_bytes(Np, Rc)));
-  } else if (!small) {
+  } else if (path == LL_TILED) {
     CUI(h->bK.reserve(per * Rc));
     CUI(h->bDinv.reserve((size_t)Rc * Np * 64 * 8));
     CUI(h->br.reserve((size_t)Rc * Np * 8));
@@ -623,35 +634,35 @@ int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fi
   CUI(h->bll.reserve((size_t)Rc * 8));
   if (grad_host) CUI(h->bgrad.reserve((size_t)Rc * (2 + d) * 8));
   std::vector<double> gtmp(grad_host ? (size_t)Rc * (2 + d) : 0);
-  std::vector<double> rows((size_t)Rc * (3 + d));
-  std::vector<char> bad(R, 0);
+  std::vector<double> rows(path == LL_TILED ? (size_t)Rc * (3 + d) : 0);
   for (int r0 = 0; r0 < R; r0 += Rc) {
     const int rc = (R - r0 < Rc) ? (R - r0) : Rc;
-    for (int r = 0; r < rc; ++r) {
-      const double* p = P_host + (size_t)(r0 + r) * P;
-      bool fin = true;
-      for (int i = 0; i < P; ++i) fin = fin && isfinite(p[i]);
-      bad[r0 + r] = fin ? 0 : 1;
-      double amp = fit_amp ? d * exp(p[1]) : 1.0;
-      const double* lm = p + 1 + (fit_amp ? 1 : 0);
-      double* row = rows.data() + (size_t)r * (3 + d);
-      if (fin) fill_hyper_row(row, p[0], amp, white_noise, lm, d);
-      else { row[0] = 0; row[1] = 1; row[2] = 1; for (int i = 0; i < d; ++i) row[3 + i] = 1; }
+    // the small and group kernels take the parameter vectors; the tiled sequence takes hyper rows (a vector that is not
+    // finite is set to -inf below)
+    const double* src = P_host + (size_t)r0 * P;
+    size_t row_len = P;
+    if (path == LL_TILED) {
+      for (int r = 0; r < rc; ++r) {
+        const double* p = src + (size_t)r * P;
+        fill_hyper_row(rows.data() + (size_t)r * (3 + d), p[0], fit_amp ? d * exp(p[1]) : 1.0, white_noise,
+                       p + 1 + (fit_amp ? 1 : 0), d);
+      }
+      src = rows.data();
+      row_len = 3 + d;
     }
-    const bool pin_ok = (size_t)rc * (3 + d) <= apgp_handle::PIN_DOUBLES / 2 && (size_t)rc <= apgp_handle::PIN_DOUBLES / 2;
-    const double* rsrc = rows.data();
-    if (pin_ok) { memcpy(h->pin, rows.data(), (size_t)rc * (3 + d) * 8); rsrc = h->pin; }
-    CU(cudaMemcpyAsync(h->bhyper.p, rsrc, (size_t)rc * (3 + d) * 8, cudaMemcpyHostToDevice, h->stream));
+    const bool pin_ok = (size_t)rc * row_len <= apgp_handle::PIN_DOUBLES / 2 && (size_t)rc <= apgp_handle::PIN_DOUBLES / 2;
+    if (pin_ok) { memcpy(h->pin, src, (size_t)rc * row_len * 8); src = h->pin; }
+    CU(cudaMemcpyAsync(h->bhyper.p, src, (size_t)rc * row_len * 8, cudaMemcpyHostToDevice, h->stream));
     int nl = 0;
-    if (small) {
+    if (path == LL_SMALL) {
       // one restart per CTA, everything in shared memory: a single launch per optimiser round
-      CUI(launch_loglik_small(h->X.as<double>(), h->y.as<double>(), N, d, h->bhyper.as<double>(), rc,
+      CUI(launch_loglik_small(h->X.as<double>(), h->y.as<double>(), N, d, h->bhyper.as<double>(), fit_amp, noise, rc,
                               h->bll.as<double>(), grad_host ? h->bgrad.as<double>() : nullptr, h->stream)); ++nl;
       if (grad_host)
         CU(cudaMemcpyAsync(gtmp.data(), h->bgrad.p, (size_t)rc * (2 + d) * 8, cudaMemcpyDeviceToHost, h->stream));
-    } else if (group) {
-      CUI(launch_loglik_group(h->X.as<double>(), h->y.as<double>(), N, d, Np, h->bhyper.as<double>(), rc, h->num_sms,
-                              h->gws.p, h->bll.as<double>(), h->stream)); ++nl;
+    } else if (path == LL_GROUP) {
+      CUI(launch_loglik_group(h->X.as<double>(), h->y.as<double>(), N, d, Np, h->bhyper.as<double>(), fit_amp, noise, rc,
+                              h->num_sms, h->gws.p, h->bll.as<double>(), h->stream)); ++nl;
     } else {
       FactorBatch fb{rc, N, Np, h->bK.as<double>(), h->bDinv.as<double>(), h->br.as<double>(), h->bscal.as<double>(),
                      h->binfo.as<int>()};
@@ -664,19 +675,23 @@ int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fi
     CU(cudaStreamSynchronize(h->stream));
     if (pin_ok) memcpy(ll_host + r0, lldst, (size_t)rc * 8);
     h->launches += nl;
-    if (grad_host) {                         // [sum alpha, d/dlog_c, d/dlogM..] -> george order, amplitude slot optional
-      for (int r = 0; r < rc; ++r) {
-        const double* g = gtmp.data() + (size_t)r * (2 + d);
+    for (int r = 0; r < rc; ++r) {
+      const double* p = P_host + (size_t)(r0 + r) * P;
+      bool fin = true;
+      for (int i = 0; i < P; ++i) fin = fin && isfinite(p[i]);
+      double& ll = ll_host[r0 + r];
+      if (!fin || !isfinite(ll)) ll = -INFINITY;
+      if (grad_host) {                       // [sum alpha, d/dlog_c, d/dlogM..] -> george order, amplitude slot optional
+        const double* gr = gtmp.data() + (size_t)r * (2 + d);
         double* o = grad_host + (size_t)(r0 + r) * P;
         int k = 0;
-        o[k++] = g[0];
-        if (fit_amp) o[k++] = g[1];
-        for (int i = 0; i < d; ++i) o[k++] = g[2 + i];
-        if (bad[r0 + r] || !isfinite(ll_host[r0 + r])) for (int i = 0; i < P; ++i) o[i] = 0.0;
+        o[k++] = gr[0];
+        if (fit_amp) o[k++] = gr[1];
+        for (int i = 0; i < d; ++i) o[k++] = gr[2 + i];
+        if (ll == -INFINITY) for (int i = 0; i < P; ++i) o[i] = 0.0;
       }
     }
   }
-  for (int r = 0; r < R; ++r) if (bad[r] || !isfinite(ll_host[r])) ll_host[r] = -INFINITY;
   return APGP_OK;
 }
 
@@ -1101,6 +1116,12 @@ int apgp_get_chol(apgp_handle* h, double* L) { return get_square(h, h->K, L); }
 int apgp_debug_last_var_path(const apgp_handle* h, int* path) {
   if (!h || !path) return fail(APGP_ERR_ARG, "apgp_debug_last_var_path");
   *path = h->last_var_path;
+  return APGP_OK;
+}
+
+int apgp_debug_last_loglik_path(const apgp_handle* h, int* path) {
+  if (!h || !path) return fail(APGP_ERR_ARG, "apgp_debug_last_loglik_path");
+  *path = h->last_loglik_path;
   return APGP_OK;
 }
 

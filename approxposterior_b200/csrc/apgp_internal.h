@@ -115,15 +115,17 @@ int launch_refine_alpha(const double* X, const double* y, int N, int d, int Np, 
 int launch_append_point(const double* X, int N, int d, int Np, const double* xnew_dev, const double* hyper_dev, double kappa,
                         double rnew, double* L, double* Linv, double* z, double* alpha, double* kvec, double* lvec,
                         double* uvec, double* scal, int* status, cudaStream_t st, int* launches);
-// fused one-restart-per-CTA path (everything in shared memory); usable when loglik_small_smem(N,d) <= 220 KB
+// batched log-likelihood of P [R][1 + fit_amp + d] (george order; noise = e^{white_noise} + TINY^2) by the evaluators of
+// loglik.cuh, the same bits as the device optimisers' objective.  Small: one restart per CTA, everything in shared memory,
+// usable when loglik_small_smem(N, d) <= 220 KB
 size_t loglik_small_smem(int N, int d);
-int launch_loglik_small(const double* X, const double* y, int N, int d, const double* hyper, int R, double* ll,
-                        double* grad /*[R][2+d] or null*/, cudaStream_t st);
-// fused one-CLUSTER-per-restart path for larger N (chol_group.cuh): the matrix lives in L2-resident global workspace
+int launch_loglik_small(const double* X, const double* y, int N, int d, const double* P, int fit_amp, double noise, int R,
+                        double* ll, double* grad /*[R][2+d] or null*/, cudaStream_t st);
+// group: one CLUSTER per restart for larger N (chol_group.cuh), the matrix in L2-resident global workspace
 int chol_group_cluster(int Np, int R, int num_sms);
 size_t chol_group_ws_bytes(int Np, int R);
-int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* hyper, int R, int num_sms,
-                        void* ws_bytes, double* ll, cudaStream_t st);
+int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp, double noise,
+                        int R, int num_sms, void* ws_bytes, double* ll, cudaStream_t st);
 // gradient pieces: Kinv = Linv^T Linv (lower), then tr-products; grad_dev needs grad_loglik_doubles(Np, d) doubles
 size_t grad_loglik_doubles(int Np, int d);
 int launch_grad_loglik(const double* X, int N, int d, int Np, const double* Linv, const double* alpha,

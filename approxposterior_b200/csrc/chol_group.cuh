@@ -36,6 +36,8 @@
 // The flags only ever grow (epoch-based targets), so repeated evaluations by the same cluster -- the device
 // optimisers call this once per objective evaluation -- need no reset.  All partial sums are added in block order:
 // every CTA of the cluster returns the SAME bits, which the replicated optimiser state relies on.
+// Every multiply-add is explicit (fma, or __dmul_rn / __dadd_rn / __dsub_rn where none is fused), so the routine rounds
+// the same in translation units compiled with and without -fmad (loglik.cuh).
 #pragma once
 #include <cuda_runtime.h>
 #include <math.h>
@@ -515,8 +517,8 @@ __device__ double chol_group_loglik(const CholGroup& g, const double* hyp, doubl
               const int rr = rbase + u, gi = ci * CG_T + rr;
               double v;
               if (gi < g.N && gj < g.N) {
-                v = amp * exp_neg(s16[u], etab);
-                if (gi == gj) v += noise;
+                v = __dmul_rn(amp, exp_neg(s16[u], etab));
+                if (gi == gj) v = __dadd_rn(v, noise);
               } else {
                 v = (gi == gj) ? 1.0 : 0.0;
               }
@@ -581,7 +583,7 @@ __device__ double chol_group_loglik(const CholGroup& g, const double* hyp, doubl
         }
       }
       if (tid < 32) {                                                          // block partials, fixed order
-        double zz = R[tid] * R[tid] + R[tid + 32] * R[tid + 32];
+        double zz = __dadd_rn(__dmul_rn(R[tid], R[tid]), __dmul_rn(R[tid + 32], R[tid + 32]));
         double lg = log(dg[tid]) + log(dg[tid + 32]);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) { zz += __shfl_xor_sync(0xffffffffu, zz, o); lg += __shfl_xor_sync(0xffffffffu, lg, o); }
@@ -624,7 +626,7 @@ __device__ double chol_group_loglik(const CholGroup& g, const double* hyp, doubl
   if (C > 1) cg_wait_ge(g.flagA, baseA + nb);
   double zz = 0.0, lg = 0.0, bad = 0.0;
   for (int k = 0; k < nb; ++k) { zz += __ldcg(part + k * 4); lg += __ldcg(part + k * 4 + 1); bad += __ldcg(part + k * 4 + 2); }
-  double ll = -0.5 * zz - lg - 0.5 * g.N * 1.8378770664093454836;
+  double ll = __dsub_rn(__dsub_rn(__dmul_rn(-0.5, zz), lg), __dmul_rn(__dmul_rn(0.5, (double)g.N), 1.8378770664093454836));
   if (bad != 0.0 || !(ll == ll) || !(fabs(ll) < INFINITY)) ll = -INFINITY;
   __syncthreads();
   CGP_ADD(9, t_ph);

@@ -3,6 +3,7 @@
 //     mma.sync f64 shape lowers to it -- see profiles/r01_fp64_pipe_probe.txt)
 //   * mbarrier + 1-D bulk TMA (cp.async.bulk -> SASS UBLKCP) wrappers
 //   * fragment-order index helpers shared by the packers and the consumers
+//   * fixed-order CTA sum
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -18,6 +19,20 @@ namespace apgp {
 __device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
                : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
+}
+
+// fixed-order sum over a CTA of NT threads, the same bits in every thread; red: NT / 32 doubles of shared memory
+template <int NT>
+__device__ __forceinline__ double cta_sum(double v, double* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();                      // red free to overwrite
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  double t = 0.0;
+#pragma unroll
+  for (int w = 0; w < NT / 32; ++w) t += red[w];
+  return t;
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

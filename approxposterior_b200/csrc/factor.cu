@@ -13,8 +13,7 @@
 // Padding: N is padded to Np (multiple of 64) with an identity block, so L and L^{-1} pad with
 // the identity and the rhs with zeros; nothing downstream needs edge handling.
 #include "apgp_internal.h"
-#include "chol_small.cuh"
-#include "chol_group.cuh"
+#include "loglik.cuh"
 #include <math.h>
 #include <stdlib.h>
 #include <stdio.h>
@@ -417,62 +416,35 @@ __global__ void grad_finish_kernel(const double* __restrict__ part, int ntiles, 
 }
 
 
-// ---- one restart per CTA: covariance build + Cholesky + forward solve + log-likelihood, all in shared
-//      memory (packed lower triangle).  Used when N(N+1)/2 + N(d+2) doubles fit in 220 KB (N <= ~224 < 256 threads).
-//      Replaces one gpUtils._nll evaluation (gpUtils.py:46-80) per CTA.
+// ---- one restart per CTA: the small evaluator of loglik.cuh (N <= ~224), one parameter vector of P [R][1 + fit_amp + d]
+//      per CTA.  Replaces one gpUtils._nll evaluation (gpUtils.py:46-80) per CTA; a vector that is not finite gives -inf
+//      without being factorised.
 //      With grad_out != nullptr the CTA goes on to alpha = L^{-T} z, inverts L in place, forms K^{-1} pair by pair
 //      and reduces  dl/dp = 1/2 tr[(alpha alpha^T - K^{-1}) dK/dp]  (george.GP.grad_log_likelihood, gpUtils.py:110):
 //      grad_out[r] = [ sum(alpha), d/dlog_constant, d/dlog M_0 .. ]   (the host drops the amplitude slot if unused).
-__global__ void __launch_bounds__(256, 1) loglik_small_kernel(const double* __restrict__ X, const double* __restrict__ y,
-                                                           int N, int d, const double* __restrict__ hyper,
-                                                           double* __restrict__ ll_out, double* __restrict__ grad_out) {
+__global__ void __launch_bounds__(LL_NT, 1) loglik_small_kernel(const double* __restrict__ X, const double* __restrict__ y,
+                                                              int N, int d, const double* __restrict__ Pv, int fit_amp,
+                                                              double noise, double* __restrict__ ll_out,
+                                                              double* __restrict__ grad_out) {
   extern __shared__ __align__(16) double sm[];
-  double* K = sm;                                   // packed lower: K[i(i+1)/2 + j], j <= i
-  double* xs = K + (size_t)N * (N + 1) / 2;         // [N][d]
-  double* r = xs + (size_t)N * d;                   // [N] residual -> z
-  double* col = r + N;                              // [N] current column of L
+  const SmallLL L = SmallLL::carve(sm, N, d);
   __shared__ double red[256];
-  __shared__ int bad;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const double* h = hyper + (size_t)blockIdx.x * (3 + d);
-  const double mean = h[0], amp = h[1], noise = h[2];
-  if (tid == 0) bad = 0;
-  for (int e = tid; e < N * d; e += 256) xs[e] = X[e];
-  for (int i = tid; i < N; i += 256) r[i] = y[i] - mean;
-  __syncthreads();
-  // covariance, row i handled by one warp at a time
-  for (int i = warp; i < N; i += 8) {
-    double* Ki = K + (size_t)i * (i + 1) / 2;
-    for (int j = lane; j <= i; j += 32) {
-      double s = 0.0;
-      for (int c = 0; c < d; ++c) { double df = xs[i * d + c] - xs[j * d + c]; s += df * df * h[3 + c]; }
-      double v = amp * exp(-0.5 * s);
-      if (i == j) v += noise;
-      Ki[j] = v;
-    }
-  }
-  __syncthreads();
-  // blocked Cholesky, forward substitution riding along (chol_small.cuh): r <- z, col <- diag(L)
-  chol_packed_blocked<256>(K, r, col, N, &bad, grad_out != nullptr);
-  double part = 0.0, lpart = 0.0;
-  for (int i = tid; i < N; i += 256) { part = fma(r[i], r[i], part); lpart += log(col[i]); }
-  red[tid] = lpart;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) { if (tid < o) red[tid] += red[tid + o]; __syncthreads(); }
-  const double logdet = red[0];
-  __syncthreads();
-  red[tid] = part;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) { if (tid < o) red[tid] += red[tid + o]; __syncthreads(); }
-  if (tid == 0) {
-    double v = -0.5 * red[0] - logdet - 0.5 * N * 1.8378770664093454836;
-    if (bad || !(v == v) || v == INFINITY || v == -INFINITY) v = -INFINITY;
-    ll_out[blockIdx.x] = v;
-  }
+  const int tid = threadIdx.x;
+  const int P = 1 + fit_amp + d;
+  const double* p = Pv + (size_t)blockIdx.x * P;
+  if (!nll_row_finite(p, P)) { if (tid == 0) ll_out[blockIdx.x] = -INFINITY; return; }
+  for (int e = tid; e < N * d; e += LL_NT) L.X[e] = X[e];
+  for (int i = tid; i < N; i += LL_NT) L.y[i] = y[i];
+  nll_hyp(p, d, fit_amp, noise, L.hyp);
+  const double ll = loglik_small(L, N, d, grad_out != nullptr);      // L in K, z in r, diag(L) in col
+  if (tid == 0) ll_out[blockIdx.x] = ll;
+  double* K = L.K; double* r = L.r; double* col = L.col;
+  const double* xs = L.X; const double* h = L.hyp;
+  const double amp = h[1];
   if (grad_out == nullptr) return;
   double* g_out = grad_out + (size_t)blockIdx.x * (2 + d);
   __syncthreads();
-  if (bad) {                                          // quiet=True convention: zeros when the factorisation failed
+  if (*L.bad) {                                       // quiet=True convention: zeros when the factorisation failed
     for (int c = tid; c < 2 + d; c += 256) g_out[c] = 0.0;
     return;
   }
@@ -610,16 +582,19 @@ __global__ void __launch_bounds__(256) append_finish_kernel(double* __restrict__
 //      (chol_group.cuh).  grid = R * C CTAs, cluster dimension C; ws = per-restart workspace described by GroupWs.
 __global__ void __launch_bounds__(CG_THREADS, 1) loglik_group_kernel(const double* __restrict__ X, const double* __restrict__ y,
                                                                      int N, int d, int Np, int C,
-                                                                     const double* __restrict__ hyper, GroupWs ws,
-                                                                     double* __restrict__ ll_out) {
+                                                                     const double* __restrict__ Pv, int fit_amp, double noise,
+                                                                     GroupWs ws, double* __restrict__ ll_out) {
   extern __shared__ __align__(16) double gsm[];
   __shared__ double hyp[3 + APGP_MAXD];
-  const int rr = blockIdx.x / C;
-  if (threadIdx.x < 3 + d) hyp[threadIdx.x] = hyper[(size_t)rr * (3 + d) + threadIdx.x];
+  const int rr = blockIdx.x / C, rank = (C > 1) ? cg_cluster_ctarank() : 0;
+  const int P = 1 + fit_amp + d;
+  const double* p = Pv + (size_t)rr * P;
+  if (!nll_row_finite(p, P)) { if (rank == 0 && threadIdx.x == 0) ll_out[rr] = -INFINITY; return; }   // uniform in the cluster
+  nll_hyp(p, d, fit_amp, noise, hyp);
   __syncthreads();
-  const CholGroup g = cg_make(ws, rr, N, Np, d, C, (C > 1) ? cg_cluster_ctarank() : 0, X, y);
+  const CholGroup g = cg_make(ws, rr, N, Np, d, C, rank, X, y);
   const double ll = chol_group_loglik<true>(g, hyp, gsm, 0ull);
-  if (g.rank == 0 && threadIdx.x == 0) ll_out[rr] = ll;
+  if (rank == 0 && threadIdx.x == 0) ll_out[rr] = ll;
 }
 
 PerDeviceOnce g_attr_done;
@@ -691,12 +666,12 @@ int launch_tri_inverse(const double* L, const double* Dinv, int Np, double* Linv
   return (int)cudaGetLastError();
 }
 
-size_t loglik_small_smem(int N, int d) { return ((size_t)N * (N + 1) / 2 + (size_t)N * (d + 2)) * sizeof(double); }
+size_t loglik_small_smem(int N, int d) { return SmallLL::doubles(N, d) * sizeof(double); }
 
-int launch_loglik_small(const double* X, const double* y, int N, int d, const double* hyper, int R, double* ll,
-                        double* grad, cudaStream_t st) {
+int launch_loglik_small(const double* X, const double* y, int N, int d, const double* P, int fit_amp, double noise, int R,
+                        double* ll, double* grad, cudaStream_t st) {
   int e = ensure_attrs(); if (e) return e;
-  loglik_small_kernel<<<R, 256, loglik_small_smem(N, d), st>>>(X, y, N, d, hyper, ll, grad);
+  loglik_small_kernel<<<R, LL_NT, loglik_small_smem(N, d), st>>>(X, y, N, d, P, fit_amp, noise, ll, grad);
   return (int)cudaGetLastError();
 }
 
@@ -713,9 +688,9 @@ int chol_group_cluster(int Np, int R, int num_sms) {
   return C;
 }
 size_t chol_group_ws_bytes(int Np, int R) { return cg_ws_bytes(Np, R); }
-// ws: chol_group_ws_bytes(Np, R) bytes.  hyper [R][3 + d] as for launch_build_K.  One launch for all R vectors.
-int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* hyper, int R, int num_sms,
-                        void* ws_bytes, double* ll, cudaStream_t st) {
+// ws: chol_group_ws_bytes(Np, R) bytes.  P [R][1 + fit_amp + d] as for launch_loglik_small.  One launch for all R vectors.
+int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp, double noise,
+                        int R, int num_sms, void* ws_bytes, double* ll, cudaStream_t st) {
   int e = ensure_attrs(); if (e) return e;
   GroupWs ws = cg_ws_carve(ws_bytes, Np, R);
   cudaError_t ce = cudaMemsetAsync(ws.flags, 0, (size_t)R * 16, st);
@@ -729,7 +704,7 @@ int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, 
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    ce = cudaLaunchKernelEx(&cfg, loglik_group_kernel, X, y, N, d, Np, C, hyper, ws, ll);
+    ce = cudaLaunchKernelEx(&cfg, loglik_group_kernel, X, y, N, d, Np, C, P, fit_amp, noise, ws, ll);
     if (ce == cudaSuccess || C == 1) break;
     (void)cudaGetLastError();                // the cluster could not be scheduled: halve it (C = 1 always can)
     C >>= 1;

@@ -28,10 +28,8 @@
 // may be used to endorse or promote products derived from this software without specific prior written permission.
 // THIS SOFTWARE IS PROVIDED "AS IS", WITHOUT WARRANTIES OF ANY KIND.
 #include "apgp_internal.h"
-#include "chol_small.cuh"
-#include "chol_group.cuh"
+#include "loglik.cuh"
 #include <math.h>
-#include <type_traits>
 #include <stdlib.h>
 
 namespace apgp {
@@ -39,21 +37,6 @@ namespace {
 
 constexpr int OT = 256;                 // threads per CTA
 constexpr int OW = OT / 32;
-constexpr double LOG_2PI = 1.8378770664093454836;
-
-// fixed-order CTA sum, identical result in every thread
-__device__ __forceinline__ double cta_sum(double v, double* red /*[OW]*/) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  __syncthreads();                      // red free to overwrite
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-  __syncthreads();
-  double t = 0.0;
-#pragma unroll
-  for (int w = 0; w < OW; ++w) t += red[w];
-  return t;
-}
-
 // The objectives are __noinline__ on purpose: the optimisers call them from ~20 places, and inlining every copy
 // made 600 KB of SASS per kernel (37 600 instructions; 6 400 now, +11 % speed: profiles/r01_optimizers.md).
 // A non-inlined member cannot see that the struct's pointers are shared-memory addresses, so the structs carry
@@ -98,7 +81,7 @@ struct UtilObj {
       E[j] = e;
       part = fma(e, alphaA[j], part);
     }
-    const double mu = mean + cta_sum(part, red);         // (its barriers also publish E)
+    const double mu = mean + cta_sum<OT>(part, red);         // (its barriers also publish E)
     if (kind == 4) return -mu;                           // findMAP objective: -(GP mean)
     double acc = 0.0;
     for (int i = warp; i < N; i += OW) {
@@ -124,94 +107,23 @@ struct UtilObj {
 };
 
 // ------------------------------------------------------------------------------------------------------
-// Objective 2: negative log-likelihood at one hyper-parameter vector (gpUtils._nll): covariance build,
-// Cholesky with the forward substitution riding along, all in shared memory (packed lower triangle).
+// Objective 2: negative log-likelihood at one hyper-parameter vector (gpUtils._nll) behind defaultHyperPrior:
+// the small evaluator of loglik.cuh, everything in this CTA's shared memory.
 // ------------------------------------------------------------------------------------------------------
 struct NllObj {
   int N, d, P, fit_amp, default_prior;
   double noise;            // exp(white_noise) + TINY^2
-  int oX, oY, oK, oR, oCol, oInvM, oRed, oBad;   // shared: X [N][d], y [N], packed K, r [N], diag(L) [N], invM [d], red, flag
 
   __device__ __noinline__ double eval(int ox) const {
     extern __shared__ __align__(16) double smem_dyn[];
-    const int tid = threadIdx.x;
     const double* p = smem_dyn + ox;
-    const double* X = smem_dyn + oX; const double* y = smem_dyn + oY;
-    double* K = smem_dyn + oK; double* r = smem_dyn + oR; double* col = smem_dyn + oCol;
-    double* invM = smem_dyn + oInvM; double* red = smem_dyn + oRed;
-    int* badflag = reinterpret_cast<int*>(smem_dyn + oBad);
-    PROF_T(t_e0);
+    const SmallLL L = SmallLL::carve(smem_dyn, N, d);
     __syncthreads();
-    bool fin = true;
-    for (int k = 0; k < P; ++k) { const double v = p[k]; fin = fin && (v == v) && (fabs(v) < INFINITY); }
-    if (!fin) return INFINITY;
+    if (!nll_row_finite(p, P)) return INFINITY;
     if (default_prior)                                   // gpUtils.defaultHyperPrior: |p[1:]| <= 20
       for (int k = 1; k < P; ++k) if (fabs(p[k]) > 20.0) return INFINITY;
-    const double mean = p[0];
-    const double amp = fit_amp ? (double)d * exp(p[1]) : 1.0;
-    if (tid < d) invM[tid] = exp(-p[1 + fit_amp + tid]);
-    if (tid == 0) *badflag = 0;
-    for (int i = tid; i < N; i += OT) r[i] = y[i] - mean;
-    __syncthreads();
-    PROF_ADD(6, t_e0);
-    PROF_T(t_b0);
-    // covariance: the packed triangle is one linear array, so element e = i(i+1)/2 + j goes to thread e mod OT
-    // ((i, j) recovered with a float sqrt + integer fix-up); two or four elements are in flight per thread so their
-    // distance and exp chains overlap
-    {
-      const int total = N * (N + 1) / 2;
-      auto build = [&](auto uc) {
-        constexpr int U = decltype(uc)::value;
-        for (int e0 = tid; e0 < total; e0 += U * OT) {
-          int ii[U], jj[U];
-          bool on[U];
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            const int e = e0 + u * OT;
-            on[u] = e < total;
-            int i = (int)((sqrtf(8.0f * (float)e + 1.0f) - 1.0f) * 0.5f);
-            if ((i + 1) * (i + 2) / 2 <= e) ++i;
-            if (i * (i + 1) / 2 > e) --i;
-            if (!on[u]) i = 0;
-            ii[u] = i;
-            jj[u] = on[u] ? e - i * (i + 1) / 2 : 0;
-          }
-          double sv[U];
-#pragma unroll
-          for (int u = 0; u < U; ++u) sv[u] = 0.0;
-          for (int c = 0; c < d; ++c) {
-            const double m = invM[c];
-#pragma unroll
-            for (int u = 0; u < U; ++u) {
-              const double da = X[ii[u] * d + c] - X[jj[u] * d + c];
-              sv[u] = fma(da * da, m, sv[u]);
-            }
-          }
-#pragma unroll
-          for (int u = 0; u < U; ++u) {
-            double v = amp * exp(-0.5 * sv[u]);
-            if (ii[u] == jj[u]) v += noise;
-            if (on[u]) K[e0 + u * OT] = v;
-          }
-        }
-      };
-      // measured (cycles per evaluation, 2 -> 4 in flight): N = 50 +1000, 70 +800, 90 -700, 200 -7000, N = 200 / d = 10 -26000
-      if (total > 12 * OT) build(std::integral_constant<int, 4>{}); else build(std::integral_constant<int, 2>{});
-    }
-    PROF_ADD(7, t_b0);
-    __syncthreads();
-    PROF_ADD(2, t_e0);                                            // prologue + covariance build
-    chol_packed_blocked<OT>(K, r, col, N, badflag, false);      // r <- z = L^{-1}(y - m), col <- diag(L)
-    PROF_T(t_e1);
-    double zpart = 0.0, lpart = 0.0;
-    for (int i = tid; i < N; i += OT) { zpart = fma(r[i], r[i], zpart); lpart += log(col[i]); }
-    const double ssq = cta_sum(zpart, red);
-    const double logdet = cta_sum(lpart, red);
-    const bool bad = (*badflag != 0);
-    PROF_ADD(3, t_e1);                                            // log-det + |z|^2 reductions
-    const double ll = -0.5 * ssq - logdet - 0.5 * N * LOG_2PI;
-    if (bad || !(ll == ll) || !(fabs(ll) < INFINITY)) return INFINITY;
-    return -ll;
+    nll_hyp(p, d, fit_amp, noise, L.hyp);
+    return -loglik_small(L, N, d, false);
   }
 };
 
@@ -230,21 +142,16 @@ struct NllGroupObj {
 
   __device__ __noinline__ double eval(int ox) {
     extern __shared__ __align__(16) double smem_dyn[];
-    const int tid = threadIdx.x;
     const double* p = smem_dyn + ox;
     double* hyp = smem_dyn + oHyp;
     __syncthreads();
-    bool fin = true;
-    for (int k = 0; k < P; ++k) { const double v = p[k]; fin = fin && (v == v) && (fabs(v) < INFINITY); }
-    if (!fin) return INFINITY;
+    if (!nll_row_finite(p, P)) return INFINITY;
     if (default_prior)                                   // gpUtils.defaultHyperPrior: |p[1:]| <= 20
       for (int k = 1; k < P; ++k) if (fabs(p[k]) > 20.0) return INFINITY;
-    if (tid == 0) { hyp[0] = p[0]; hyp[1] = fit_amp ? (double)d * exp(p[1]) : 1.0; hyp[2] = noise; }
-    if (tid < d) hyp[3 + tid] = exp(-p[1 + fit_amp + tid]);
+    nll_hyp(p, d, fit_amp, noise, hyp);
     __syncthreads();
     const double ll = chol_group_loglik<true>(g, hyp, smem_dyn + oTiles, epoch);
     ++epoch;
-    if (!(ll == ll) || !(fabs(ll) < INFINITY)) return INFINITY;
     return -ll;
   }
 };
@@ -700,20 +607,11 @@ struct NllKernelParams {
 __global__ void __launch_bounds__(OT, 1) minimize_nll_kernel(const __grid_constant__ NllKernelParams p) {
   extern __shared__ __align__(16) double sm[];
   const int tid = threadIdx.x, n = p.P;
-  double* cur = sm;
-  double* K = cur; cur += (size_t)p.N * (p.N + 1) / 2;
-  double* X = cur; cur += (size_t)p.N * p.d;
-  double* y = cur; cur += p.N;
-  double* r = cur; cur += p.N;
-  double* col = cur; cur += p.N;
-  double* invM = cur; cur += p.d;
-  double* red = cur; cur += OW;
-  int* badflag = reinterpret_cast<int*>(cur); cur += 1;
-  OptWork w; w.carve(cur, n); w.base = sm;
-  for (int e = tid; e < p.N * p.d; e += OT) X[e] = p.X[e];
-  for (int e = tid; e < p.N; e += OT) y[e] = p.y[e];
-  NllObj f{p.N, p.d, p.P, p.fit_amp, p.default_prior, p.noise, (int)(X - sm), (int)(y - sm), (int)(K - sm), (int)(r - sm),
-           (int)(col - sm), (int)(invM - sm), (int)(red - sm), (int)(reinterpret_cast<double*>(badflag) - sm)};
+  const SmallLL L = SmallLL::carve(sm, p.N, p.d);
+  OptWork w; w.carve(sm + SmallLL::doubles(p.N, p.d), n); w.base = sm;
+  for (int e = tid; e < p.N * p.d; e += OT) L.X[e] = p.X[e];
+  for (int e = tid; e < p.N; e += OT) L.y[e] = p.y[e];
+  NllObj f{p.N, p.d, p.P, p.fit_amp, p.default_prior, p.noise};
   const double* x0 = p.p0 + (size_t)blockIdx.x * n;
   double* start = (p.opt.method == 1 && p.mode == 1) ? w.v0 : w.sim;
   if (tid < n) start[tid] = x0[tid];
@@ -805,7 +703,7 @@ void fill_opt(OptOpts& o, const OptimizeParams& q, int n) {
 }  // namespace
 
 size_t minimize_nll_smem(int N, int d, int P) {
-  return ((size_t)N * (N + 1) / 2 + (size_t)N * (d + 3) + d + OW + 1 + OptWork::doubles(P)) * sizeof(double);
+  return (SmallLL::doubles(N, d) + OptWork::doubles(P)) * sizeof(double);
 }
 bool minimize_nll_fits(int N, int d, int P) { return minimize_nll_smem(N, d, P) <= SMEM_CAP && P + 1 <= OT && N < OT; }
 

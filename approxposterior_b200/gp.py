@@ -355,10 +355,11 @@ class GP(object):
         Pfull = P if self.fit_mean else np.ascontiguousarray(np.hstack([np.full((P.shape[0], 1), self.mean), P]))
         ll = np.empty(Pfull.shape[0])
         grad = np.empty_like(Pfull) if return_grad else None
-        N, d = self._x.shape
-        fused = (N * (N + 1) // 2 + N * (d + 2)) * 8 <= 220 * 1024
-        if return_grad and not fused:
-            # large N: one factorisation per vector on the single-GP path (explicit inverse + trace products)
+        st = _lib.check(self._lib.apgp_loglik_batch(self._h, _lib.ptr(Pfull), Pfull.shape[0], Pfull.shape[1], fit_amp,
+                                                    self.white_noise, _lib.ptr(ll), _lib.ptr(grad)), "apgp_loglik_batch")
+        if st == _lib.APGP_NEEDS_HOST:
+            # batched gradients come from the one-restart-per-CTA kernel only: one factorisation per vector on the
+            # single-GP path (explicit inverse + trace products)
             keep = self.get_parameter_vector()
             for r in range(P.shape[0]):
                 self.set_parameter_vector(P[r])
@@ -367,10 +368,6 @@ class GP(object):
                 grad[r] = g if self.fit_mean else np.concatenate([[0.0], g])
             self.set_parameter_vector(keep)
             self.recompute(quiet=True)
-        else:
-            _lib.check(self._lib.apgp_loglik_batch(self._h, _lib.ptr(Pfull), Pfull.shape[0], Pfull.shape[1], fit_amp,
-                                                   self.white_noise, _lib.ptr(ll), _lib.ptr(grad)),
-                       "apgp_loglik_batch")
         if not return_grad:
             return ll
         return ll, (grad if self.fit_mean else grad[:, 1:])

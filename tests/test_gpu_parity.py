@@ -204,13 +204,13 @@ def test_loglik_batch_gradients(N, fit_amp):
 
 def test_loglik_batch_fused_and_tiled_paths_agree(monkeypatch):
     """N small enough for the one-restart-per-CTA shared-memory kernel: it must agree with the tiled
-    multi-launch path (forced with APGP_LOGLIK_TILED) and with the oracle."""
+    multi-launch path (forced with APGP_LOGLIK_PATH=tiled) and with the oracle."""
     theta, y = rosenbrock_training(150)
     gp, orc = make_pair(theta, y, np.zeros(2), amp=float(np.var(y)))
     rng = np.random.default_rng(5)
     P = np.column_stack([np.full(20, np.median(y)), rng.standard_normal((20, 3))])
     ll_small = gp.log_likelihood_batch(P, y)
-    monkeypatch.setenv("APGP_LOGLIK_TILED", "1")
+    monkeypatch.setenv("APGP_LOGLIK_PATH", "tiled")
     ll_tiled = gp.log_likelihood_batch(P, y)
     np.testing.assert_allclose(ll_small, ll_tiled, rtol=1e-10)
     for r in range(0, 20, 5):

@@ -42,9 +42,9 @@ for N, d, amp in ((70, 2, None), (200, 3, 2.0), (300, 5, None)):
         gp.minimize_nll(P[:3], y2, evaluate_only=True)
         gp.minimize_nll(P[:3], y2, method="powell", options={"maxfev": 25})
         gp.minimize_nll(P[:3], y2, method="nelder-mead", options={"maxfev": 25})
-    os.environ["APGP_LOGLIK_TILED"] = "1"
+    os.environ["APGP_LOGLIK_PATH"] = "tiled"
     gp.log_likelihood_batch(P, y2)
-    del os.environ["APGP_LOGLIK_TILED"]
+    del os.environ["APGP_LOGLIK_PATH"]
 # grouped variance kernel (G CTAs per query tile, cooperative launch): N >= 1024 selects it automatically
 N, d = 1100, 3
 X = rng.uniform(-5, 5, size=(N, d)); y = np.sin(X).sum(axis=1)

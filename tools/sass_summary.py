@@ -11,7 +11,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-COLS = ("DMMA", "UBLKCP", "SYNCS", "BAR", "DFMA", "LDS", "STS", "MUFU", "CGABAR", "ATOM", "RED")
+COLS = ("DMMA", "UBLKCP", "SYNCS", "BAR", "DFMA", "DMUL", "DADD", "LDS", "STS", "MUFU", "CGABAR", "ATOM", "RED")
 
 
 def demangle(names):
