@@ -106,20 +106,24 @@ void fill_hyper_row(double* row, double mean, double amp, double wn, const doubl
 }
 
 // apgp_loglik_batch's kernels, as apgp_debug_last_loglik_path reports them
-enum LoglikPath { LL_SMALL = 1, LL_GROUP = 2, LL_TILED = 3 };
+enum LoglikPath { LL_SMALL = 1, LL_GROUP = 2, LL_TILED = 3, LL_GROUP_GRAD = 4 };
 // One restart per CTA while the small evaluator fits one CTA's shared memory (N <= ~224), else one CLUSTER per restart
 // (fused single launch, chol_group.cuh) -- except a handful of large matrices, which the multi-launch tiled sequence
 // spreads over the whole GPU where a cluster is at most 16 SMs (measured, R = 1: N = 1024 0.51 ms fused vs 0.71 ms tiled,
-// N = 2048 1.85 vs 1.48 ms; R = 8, N = 2048: 2.87 vs 2.73).  APGP_LOGLIK_PATH = small | group | tiled overrides (small
-// only where it fits).
-int choose_loglik_path(const apgp_handle* h, int R) {
+// N = 2048 1.85 vs 1.48 ms; R = 8, N = 2048: 2.87 vs 2.73).  With gradients (grad) everything above the small class takes
+// the cluster kernel with gradients, loglik_grad_group_kernel, few large matrices included.  APGP_LOGLIK_PATH = small |
+// group | tiled forces a value kernel (small only where it fits); forced group or tiled has no gradients (the caller gets
+// APGP_NEEDS_HOST).  APGP_LOGLIK_PATH = group_grad forces the cluster kernel with gradients at any N (group for values).
+int choose_loglik_path(const apgp_handle* h, int R, bool grad) {
   const bool fits = loglik_small_smem(h->N, h->d) <= 220 * 1024;
   if (const char* v = getenv("APGP_LOGLIK_PATH")) {
     if (!strcmp(v, "small") && fits) return LL_SMALL;
     if (!strcmp(v, "group")) return LL_GROUP;
     if (!strcmp(v, "tiled")) return LL_TILED;
+    if (!strcmp(v, "group_grad")) return grad ? LL_GROUP_GRAD : LL_GROUP;
   }
   if (fits) return LL_SMALL;
+  if (grad) return LL_GROUP_GRAD;
   return (h->Np >= 2048 && R <= 8) ? LL_TILED : LL_GROUP;
 }
 
@@ -613,16 +617,19 @@ int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fi
   const int d = h->d, N = h->N, Np = h->Np;
   if (P != 1 + (fit_amp ? 1 : 0) + d) return fail(APGP_ERR_ARG, "apgp_loglik_batch: P != 1 + fit_amp + d");
   if (R < 1) return APGP_OK;
-  const int path = choose_loglik_path(h, R);
-  if (grad_host && path != LL_SMALL) return APGP_NEEDS_HOST;    // batched gradients come from the small kernel only
+  const int path = choose_loglik_path(h, R, grad_host != nullptr);
+  // gradients come from the small kernel and the cluster kernel with gradients, not from a forced value-only kernel
+  if (grad_host && path != LL_SMALL && path != LL_GROUP_GRAD) return APGP_NEEDS_HOST;
   h->last_loglik_path = path;
   Guard g(h->device);
   const double noise = exp(white_noise) + TINY2;
-  // chunk the restart axis so the tiled path's workspace stays below ~4 GiB
-  size_t per = (size_t)Np * Np * 8;
+  // chunk the restart axis so the workspace stays below ~4 GiB (the gradient kernel keeps L and its inverse per restart)
+  size_t per = (path == LL_GROUP_GRAD) ? loglik_grad_group_ws_bytes(Np, d, 1) : (size_t)Np * Np * 8;
   int Rc = (path == LL_SMALL) ? R : (int)((4ull << 30) / per); if (Rc < 1) Rc = 1; if (Rc > R) Rc = R;
   if (path == LL_GROUP) {
     CUI(h->gws.reserve(chol_group_ws_bytes(Np, Rc)));
+  } else if (path == LL_GROUP_GRAD) {
+    CUI(h->gws.reserve(loglik_grad_group_ws_bytes(Np, d, Rc)));
   } else if (path == LL_TILED) {
     CUI(h->bK.reserve(per * Rc));
     CUI(h->bDinv.reserve((size_t)Rc * Np * 64 * 8));
@@ -663,6 +670,11 @@ int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fi
     } else if (path == LL_GROUP) {
       CUI(launch_loglik_group(h->X.as<double>(), h->y.as<double>(), N, d, Np, h->bhyper.as<double>(), fit_amp, noise, rc,
                               h->num_sms, h->gws.p, h->bll.as<double>(), h->stream)); ++nl;
+    } else if (path == LL_GROUP_GRAD) {
+      // one cluster per restart: factorisation, inverse and trace products in a single launch
+      CUI(launch_loglik_grad_group(h->X.as<double>(), h->y.as<double>(), N, d, Np, h->bhyper.as<double>(), fit_amp, noise,
+                                   rc, h->num_sms, h->gws.p, h->bll.as<double>(), h->bgrad.as<double>(), h->stream)); ++nl;
+      CU(cudaMemcpyAsync(gtmp.data(), h->bgrad.p, (size_t)rc * (2 + d) * 8, cudaMemcpyDeviceToHost, h->stream));
     } else {
       FactorBatch fb{rc, N, Np, h->bK.as<double>(), h->bDinv.as<double>(), h->br.as<double>(), h->bscal.as<double>(),
                      h->binfo.as<int>()};

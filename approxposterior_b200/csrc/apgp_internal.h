@@ -126,6 +126,11 @@ int chol_group_cluster(int Np, int R, int num_sms);
 size_t chol_group_ws_bytes(int Np, int R);
 int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp, double noise,
                         int R, int num_sms, void* ws_bytes, double* ll, cudaStream_t st);
+// the same with gradients (loglik_grad_group_kernel): grad [R][2 + d] = [sum alpha, d/dlog_constant, d/dlog M_0 ..], zeros
+// where ll is -inf; the workspace adds the transposed inverse of L, alpha and the per-tile partials to the factorisation's
+size_t loglik_grad_group_ws_bytes(int Np, int d, int R);
+int launch_loglik_grad_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp,
+                             double noise, int R, int num_sms, void* ws_bytes, double* ll, double* grad, cudaStream_t st);
 // gradient pieces: Kinv = Linv^T Linv (lower), then tr-products; grad_dev needs grad_loglik_doubles(Np, d) doubles
 size_t grad_loglik_doubles(int Np, int d);
 int launch_grad_loglik(const double* X, int N, int d, int Np, const double* Linv, const double* alpha,

@@ -597,6 +597,306 @@ __global__ void __launch_bounds__(CG_THREADS, 1) loglik_group_kernel(const doubl
   if (rank == 0 && threadIdx.x == 0) ll_out[rr] = ll;
 }
 
+// ---- the same cluster class with gradients (loglik_grad_group_kernel): after chol_group_loglik, per restart
+//        W = L^{-1}                     column block by column block, each column block by one CTA of the cluster
+//        alpha = W^T z                  by the owner of the column block, on the way
+//        K^{-1}_ab = sum_{k >= a} W_ka^T W_kb   one lower tile at a time, reduced at once into the trace products
+//      dl/dp = 1/2 tr[(alpha alpha^T - K^{-1}) dK/dp] (george.GP.grad_log_likelihood, gpUtils.py:110), as grad_reduce_kernel.
+//      W is kept TRANSPOSED, tile-major in a second triangle next to L: tile (i, j), i >= j, holds T_ij = W_ij^T.  In that
+//      form every product is  A B^T  of two row-major tiles -- the operand form of cg_update_phase -- and the triangular
+//      step is the panel solve of the factorisation (cg_trsm_dmma, X = P L_ii^{-T}) with the diagonal block's inverted 8x8
+//      blocks the factorisation left in Dinv:
+//        T_jj = I L_jj^{-T},   T_ij = -(sum_{j <= k < i} T_kj L_ik^T) L_ii^{-T}   (i > j),
+//        K^{-1}_ab = sum_{k >= a} T_ka T_kb^T,   alpha_a = sum_{k >= a} T_ka z_k.
+struct GradWs {
+  double* T; double* alpha; double* part;  // per restart: transposed inverse (nb(nb+1)/2 tiles), alpha [Np], [ntiles][2 + d]
+  size_t sT, sA, sPart;
+};
+size_t gg_restart_bytes(int Np, int d) {
+  const size_t nb = Np / CG_T, nt = nb * (nb + 1) / 2;
+  return (nt * CG_TILE + Np + nt * (2 + d)) * sizeof(double);
+}
+size_t gg_ws_bytes(int Np, int d, int R) { return (cg_ws_bytes(Np, R) + 255) / 256 * 256 + (size_t)R * gg_restart_bytes(Np, d); }
+GradWs gg_ws_carve(void* ws_bytes, int Np, int d, int R) {
+  const size_t nb = Np / CG_T, nt = nb * (nb + 1) / 2;
+  GradWs w;
+  char* base = static_cast<char*>(ws_bytes) + (cg_ws_bytes(Np, R) + 255) / 256 * 256;
+  w.T = reinterpret_cast<double*>(base); w.sT = nt * CG_TILE; base += (size_t)R * w.sT * 8;
+  w.alpha = reinterpret_cast<double*>(base); w.sA = Np; base += (size_t)R * w.sA * 8;
+  w.part = reinterpret_cast<double*>(base); w.sPart = nt * (2 + d);
+  return w;
+}
+
+// dynamic shared memory of the gradient phases: two operand pairs of the product pipeline, the tile being solved, L_ii,
+// the inverted 8x8 diagonal blocks of L_ii and z_i.  The factorisation (CG_SMEM_DOUBLES) runs in the same allocation.
+constexpr int GG_P = 4 * CG_TILE, GG_L = 5 * CG_TILE, GG_AUX = 6 * CG_TILE, GG_Z = GG_AUX + 8 * 64;
+constexpr size_t GG_SMEM_DOUBLES = GG_Z + CG_T;
+static_assert(GG_SMEM_DOUBLES >= CG_SMEM_DOUBLES, "the factorisation runs in the gradient kernel's shared memory");
+static_assert(GG_SMEM_DOUBLES * 8 <= 227 * 1024, "one CTA per SM");
+static_assert(2 * APGP_MAXD * CG_T + 2 * CG_T <= CG_TILE, "inputs and alpha of a tile pair fit the solve tile");
+static_assert((1 + APGP_MAXD) * 8 <= CG_TILE, "warp partials fit the L_ii tile");
+
+__device__ __forceinline__ double* gg_tile(double* base, int i, int j) { return base + (size_t)(i * (i + 1) / 2 + j) * CG_TILE; }
+// column blocks of W dealt out in snake order (0, 1, .., C-1, C-1, .., 0, 0, ..): column j costs ~(nb - j)^2 / 2 products
+__device__ __forceinline__ int gg_col_owner(int j, int C) { const int r = j % C; return ((j / C) & 1) ? C - 1 - r : r; }
+
+// acc = sum_{t < cnt} A_t B_t^T over 64x64 tiles of global memory (tile-major [64][CG_LD]; tiles(t, A_t, B_t) names them),
+// by all 8 warps, warp tile 32x16 as in cg_update_phase.  The operand pair of product t + 1 arrives by bulk TMA while
+// product t is multiplied; `used` counts the products this CTA has taken through the two slots (slot used & 1, mbarrier
+// phase (used >> 1) & 1), identical in every thread.  The products are added in t order: the bits do not depend on the CTA.
+template <class F>
+__device__ __forceinline__ void gg_chain(double* sm, uint64_t* full, uint32_t& used, int cnt, F tiles, double (&acc)[4][2][2]) {
+  const int tid = threadIdx.x, w8 = tid >> 5, lane = tid & 31, wm = w8 >> 2, wn = w8 & 3;
+#pragma unroll
+  for (int a = 0; a < 4; ++a)
+#pragma unroll
+    for (int b = 0; b < 2; ++b) { acc[a][b][0] = 0.0; acc[a][b][1] = 0.0; }
+  if (cnt == 0) return;
+  auto issue = [&](int t, uint32_t slot) {
+    const double* A; const double* B;
+    tiles(t, A, B);
+    mbar_arrive_expect_tx(&full[slot], 2u * CG_TILE * 8u);
+    bulk_g2s(sm + (size_t)slot * 2 * CG_TILE, A, CG_TILE * 8, &full[slot]);
+    bulk_g2s(sm + (size_t)slot * 2 * CG_TILE + CG_TILE, B, CG_TILE * 8, &full[slot]);
+  };
+  fence_proxy_async();                                 // tiles this CTA stored through the generic proxy -> bulk copies
+  __syncthreads();
+  if (tid == 0) issue(0, used & 1u);
+  for (int t = 0; t < cnt; ++t, ++used) {
+    const uint32_t slot = used & 1u;
+    mbar_wait(&full[slot], (used >> 1) & 1u);
+    __syncthreads();                                   // everyone is done with product t - 1: its slot can be refilled
+    if (tid == 0 && t + 1 < cnt) issue(t + 1, slot ^ 1u);
+    const double* As = sm + (size_t)slot * 2 * CG_TILE;
+    const double* ap = As + (wm * 32 + (lane >> 2)) * CG_LD + (lane & 3);
+    const double* bp = As + CG_TILE + (wn * 16 + (lane >> 2)) * CG_LD + (lane & 3);
+#pragma unroll 4
+    for (int k4 = 0; k4 < CG_T / 4; ++k4) {
+      double av[4], bv[2];
+#pragma unroll
+      for (int a = 0; a < 4; ++a) av[a] = ap[a * 8 * CG_LD + k4 * 4];
+#pragma unroll
+      for (int b = 0; b < 2; ++b) bv[b] = bp[b * 8 * CG_LD + k4 * 4];
+#pragma unroll
+      for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b) dmma884(acc[a][b][0], acc[a][b][1], av[a], bv[b]);
+    }
+  }
+}
+
+// all CTAs of the cluster (or the CTA when C = 1) have finished their global writes; they are visible to every one of them
+__device__ __forceinline__ void gg_cluster_sync(int C) {
+  __threadfence();
+  if (C > 1) asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;\n" ::: "memory");
+  else __syncthreads();
+}
+
+// this CTA's column blocks of T = W^T (and alpha on those rows)
+__device__ __forceinline__ void gg_inverse_phase(const CholGroup& g, double* T, double* alpha, double* sm, uint64_t* full,
+                                                 uint64_t* lbar, uint32_t& used, uint32_t& lused) {
+  const int tid = threadIdx.x, w8 = tid >> 5, lane = tid & 31, wm = w8 >> 2, wn = w8 & 3;
+  const int nb = g.nb, row = w8 * 8 + (lane >> 2), q = lane & 3;
+  double* const Ps = sm + GG_P;
+  double* const Ls = sm + GG_L;
+  double* const aux = sm + GG_AUX;
+  double* const zb = sm + GG_Z;
+  for (int j = 0; j < nb; ++j) {
+    if (gg_col_owner(j, g.C) != g.rank) continue;
+    double al = 0.0;                                   // alpha_{64 j + row}: sum over i of (T_ij z_i)[row], i ascending
+    for (int i = j; i < nb; ++i) {
+      fence_proxy_async();
+      __syncthreads();                                 // the previous step is done with Ls, Ps, aux, zb
+      if (tid == 0) {
+        mbar_arrive_expect_tx(lbar, CG_TILE * 8u);
+        bulk_g2s(Ls, cg_tile_ptr(g, i, i), CG_TILE * 8, lbar);
+      }
+      const double* Dg = g.Dinv + (size_t)i * CG_T * CG_T + CG_T;
+      for (int e = tid; e < 8 * 64; e += CG_THREADS) aux[e] = __ldcg(Dg + e);
+      if (tid < CG_T) zb[tid] = __ldcg(g.r + i * CG_T + tid);
+      double acc[4][2][2];
+      gg_chain(sm, full, used, i - j, [&](int t, const double*& A, const double*& B) {
+        A = gg_tile(T, j + t, j); B = cg_tile_ptr(g, i, j + t);
+      }, acc);
+#pragma unroll
+      for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b) {
+          const int r = wm * 32 + a * 8 + (lane >> 2), c = wn * 16 + b * 8 + 2 * q;
+          double2 o;
+          if (i == j) { o.x = (r == c) ? 1.0 : 0.0; o.y = (r == c + 1) ? 1.0 : 0.0; }
+          else { o.x = -acc[a][b][0]; o.y = -acc[a][b][1]; }
+          *reinterpret_cast<double2*>(Ps + r * CG_LD + c) = o;
+        }
+      __syncthreads();
+      mbar_wait(lbar, lused & 1u); ++lused;
+      double* const Ts[1] = {Ps};
+      cg_trsm_dmma<1>(Ts, Ls, aux, w8, lane);          // warp w8 solves rows 8 w8 .. 8 w8 + 7: T_ij
+      const double* xr = Ps + row * CG_LD;
+      double s = 0.0;
+#pragma unroll
+      for (int m = 0; m < CG_T / 4; ++m) s = fma(xr[q + 4 * m], zb[q + 4 * m], s);
+      s += __shfl_xor_sync(0xffffffffu, s, 1);
+      s += __shfl_xor_sync(0xffffffffu, s, 2);
+      al += s;
+      double* Tij = gg_tile(T, i, j);
+#pragma unroll
+      for (int rr = 0; rr < 8; ++rr) {
+        const int off = (w8 * 8 + rr) * CG_LD + 2 * lane;
+        *reinterpret_cast<double2*>(Tij + off) = *reinterpret_cast<const double2*>(Ps + off);
+      }
+    }
+    if (q == 0) alpha[j * CG_T + row] = al;
+  }
+}
+
+// this CTA's lower tiles of K^{-1} (tile t = a(a+1)/2 + b belongs to CTA t mod C), each reduced at once into
+// part[t] = [t == 0 ? sum alpha : 0, 1/2 sum G Kk, 1/2 sum G Kk (1/2 D_c^2 / M_c) ..]; padding rows and columns excluded
+__device__ __forceinline__ void gg_reduce_phase(const CholGroup& g, double* T, const double* alpha, double* part,
+                                                const double* hyp, double* sm, uint64_t* full, uint32_t& used) {
+  const int tid = threadIdx.x, w8 = tid >> 5, lane = tid & 31, wm = w8 >> 2, wn = w8 & 3;
+  const int nb = g.nb, N = g.N, d = g.d, C = g.C, me = g.rank;
+  double* const Xa = sm + GG_P;                        // [d][64] inputs of the tile's row block, then of its column block
+  double* const Xb = Xa + APGP_MAXD * CG_T;
+  double* const aa_ = Xb + APGP_MAXD * CG_T;           // alpha of the row block, then of the column block
+  double* const ab_ = aa_ + CG_T;
+  double* const wred = sm + GG_L;                      // [1 + d][8] warp partials
+  const double amp = hyp[1];
+  if (me == 0) {                                       // tile 0 is rank 0's: sum alpha in a fixed order
+    double sa = 0.0;
+    for (int i = tid; i < N; i += CG_THREADS) sa += __ldcg(alpha + i);
+    sa = cta_sum<CG_THREADS>(sa, wred);
+    if (tid == 0) part[0] = sa;
+  }
+  int t = -1;
+  for (int a = 0; a < nb; ++a)
+    for (int b = 0; b <= a; ++b) {
+      if (++t % C != me) continue;
+      double acc[4][2][2];
+      gg_chain(sm, full, used, nb - a, [&](int s, const double*& A, const double*& B) {
+        A = gg_tile(T, a + s, a); B = gg_tile(T, a + s, b);
+      }, acc);
+      __syncthreads();                                 // the previous tile's reduction is done with Xa .. wred
+      for (int e = tid; e < CG_T * d; e += CG_THREADS) {
+        const int r = e / d, c = e - r * d;
+        const int ga = a * CG_T + r, gb = b * CG_T + r;
+        Xa[c * CG_T + r] = (ga < N) ? g.X[(size_t)ga * d + c] : 0.0;
+        Xb[c * CG_T + r] = (gb < N) ? g.X[(size_t)gb * d + c] : 0.0;
+      }
+      if (tid < CG_T) { aa_[tid] = __ldcg(alpha + a * CG_T + tid); ab_[tid] = __ldcg(alpha + b * CG_T + tid); }
+      __syncthreads();
+      // this thread's 16 entries, in the accumulator layout: rows wm*32 + 8 u + lane/4, columns wn*16 + 8 v + 2 (lane%4) + h
+      double gk[4][2][2];
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int v = 0; v < 2; ++v) { gk[u][v][0] = 0.0; gk[u][v][1] = 0.0; }
+      const int r0 = wm * 32 + (lane >> 2), c0 = wn * 16 + 2 * (lane & 3);
+      for (int c = 0; c < d; ++c) {
+        const double im = hyp[3 + c];
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+#pragma unroll
+          for (int v = 0; v < 2; ++v)
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+              const double df = Xa[c * CG_T + r0 + 8 * u] - Xb[c * CG_T + c0 + 8 * v + h];
+              gk[u][v][h] += 0.5 * df * df * im;       // sum_c of 1/2 D_c^2 / M_c
+            }
+      }
+      double v0 = 0.0;
+#pragma unroll
+      for (int u = 0; u < 4; ++u)
+#pragma unroll
+        for (int v = 0; v < 2; ++v)
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            const int pl = r0 + 8 * u, ql = c0 + 8 * v + h, p = a * CG_T + pl, qq = b * CG_T + ql;
+            const double kk = amp * exp(-gk[u][v][h]);
+            const double G = aa_[pl] * ab_[ql] - acc[u][v][h];
+            const double w = (p == qq) ? 0.5 : 1.0;    // off-diagonal pairs appear twice in the full trace
+            const bool on = p < N && qq < N && (a != b || ql <= pl);
+            gk[u][v][h] = on ? w * G * kk : 0.0;
+            v0 += gk[u][v][h];
+          }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v0 += __shfl_xor_sync(0xffffffffu, v0, o);
+      if (lane == 0) wred[w8] = v0;
+      for (int c = 0; c < d; ++c) {
+        const double im = hyp[3 + c];
+        double vc = 0.0;
+#pragma unroll
+        for (int u = 0; u < 4; ++u)
+#pragma unroll
+          for (int v = 0; v < 2; ++v)
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+              const double df = Xa[c * CG_T + r0 + 8 * u] - Xb[c * CG_T + c0 + 8 * v + h];
+              vc += gk[u][v][h] * (0.5 * df * df * im);
+            }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) vc += __shfl_xor_sync(0xffffffffu, vc, o);
+        if (lane == 0) wred[(1 + c) * 8 + w8] = vc;
+      }
+      __syncthreads();
+      double* pt = part + (size_t)t * (2 + d);
+      if (tid <= d) {
+        double s = 0.0;
+#pragma unroll
+        for (int w = 0; w < 8; ++w) s += wred[tid * 8 + w];
+        pt[1 + tid] = s;
+      }
+      if (tid == 0 && t != 0) pt[0] = 0.0;
+    }
+}
+
+// grid = R * C CTAs, cluster dimension C, as loglik_group_kernel (whose ll it returns bit for bit); grad_out [R][2 + d]:
+// [sum alpha, d/dlog_constant, d/dlog M_0 ..] (loglik_small_kernel's layout), zeros where ll is -inf.
+__global__ void __launch_bounds__(CG_THREADS, 1) loglik_grad_group_kernel(const double* __restrict__ X, const double* __restrict__ y,
+                                                                          int N, int d, int Np, int C,
+                                                                          const double* __restrict__ Pv, int fit_amp, double noise,
+                                                                          GroupWs ws, GradWs gw, double* __restrict__ ll_out,
+                                                                          double* __restrict__ grad_out) {
+  extern __shared__ __align__(16) double gsm[];
+  __shared__ double hyp[3 + APGP_MAXD];
+  __shared__ __align__(8) uint64_t bars[3];            // operand slots 0 / 1 of gg_chain, L_ii
+  const int tid = threadIdx.x;
+  const int rr = blockIdx.x / C, rank = (C > 1) ? cg_cluster_ctarank() : 0;
+  const int P = 1 + fit_amp + d;
+  const double* p = Pv + (size_t)rr * P;
+  double* gout = grad_out + (size_t)rr * (2 + d);
+  if (!nll_row_finite(p, P)) {                         // uniform in the cluster
+    if (rank == 0) { if (tid == 0) ll_out[rr] = -INFINITY; if (tid < 2 + d) gout[tid] = 0.0; }
+    return;
+  }
+  nll_hyp(p, d, fit_amp, noise, hyp);
+  __syncthreads();
+  const CholGroup g = cg_make(ws, rr, N, Np, d, C, rank, X, y);
+  const double ll = chol_group_loglik<true>(g, hyp, gsm, 0ull);
+  if (rank == 0 && tid == 0) ll_out[rr] = ll;
+  if (ll == -INFINITY) {                               // the same bits in every CTA: the whole cluster leaves
+    if (rank == 0 && tid < 2 + d) gout[tid] = 0.0;
+    return;
+  }
+  // every CTA has acquired flag A of the last block (C > 1) inside chol_group_loglik: all of L, Dinv and z are visible
+  if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); mbar_init(&bars[2], 1); mbar_fence_init(); }
+  __syncthreads();
+  double* T = gw.T + rr * gw.sT;
+  double* alpha = gw.alpha + rr * gw.sA;
+  double* part = gw.part + rr * gw.sPart;
+  uint32_t used = 0, lused = 0;
+  gg_inverse_phase(g, T, alpha, gsm, bars, &bars[2], used, lused);
+  gg_cluster_sync(C);
+  gg_reduce_phase(g, T, alpha, part, hyp, gsm, bars, used);
+  gg_cluster_sync(C);
+  if (rank == 0 && tid < 2 + d) {                      // per-tile partials in tile order, whichever CTA owned each tile
+    const int nt = g.nb * (g.nb + 1) / 2;
+    double s = 0.0;
+    for (int t = 0; t < nt; ++t) s += __ldcg(part + (size_t)t * (2 + d) + tid);
+    gout[tid] = s;
+  }
+}
+
 PerDeviceOnce g_attr_done;
 int ensure_attrs() {
   if (!g_attr_done.needed()) return 0;
@@ -608,6 +908,8 @@ int ensure_attrs() {
   e = cudaFuncSetAttribute(loglik_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024); if (e) return (int)e;
   e = cudaFuncSetAttribute(loglik_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CG_SMEM_DOUBLES * 8)); if (e) return (int)e;
   e = cudaFuncSetAttribute(loglik_group_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1); if (e) return (int)e;
+  e = cudaFuncSetAttribute(loglik_grad_group_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(GG_SMEM_DOUBLES * 8)); if (e) return (int)e;
+  e = cudaFuncSetAttribute(loglik_grad_group_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1); if (e) return (int)e;
   g_attr_done.mark();
   return 0;
 }
@@ -688,6 +990,39 @@ int chol_group_cluster(int Np, int R, int num_sms) {
   return C;
 }
 size_t chol_group_ws_bytes(int Np, int R) { return cg_ws_bytes(Np, R); }
+// R clusters of C CTAs (CG_THREADS each): launch(cfg, C); a cluster size that cannot be scheduled is halved (C = 1 always
+// can), C returns the size that ran
+template <class F>
+static cudaError_t launch_clusters(int& C, int R, size_t smem, cudaStream_t st, F launch) {
+  for (;;) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(R * C)); cfg.blockDim = dim3(CG_THREADS);
+    cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    const cudaError_t ce = launch(cfg, C);
+    if (ce == cudaSuccess || C == 1) return ce;
+    (void)cudaGetLastError();
+    C >>= 1;
+  }
+}
+size_t loglik_grad_group_ws_bytes(int Np, int d, int R) { return gg_ws_bytes(Np, d, R); }
+// ws: loglik_grad_group_ws_bytes(Np, d, R) bytes; grad [R][2 + d].  One launch for all R vectors.
+int launch_loglik_grad_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp,
+                             double noise, int R, int num_sms, void* ws_bytes, double* ll, double* grad, cudaStream_t st) {
+  int e = ensure_attrs(); if (e) return e;
+  GroupWs ws = cg_ws_carve(ws_bytes, Np, R);
+  GradWs gw = gg_ws_carve(ws_bytes, Np, d, R);
+  cudaError_t ce = cudaMemsetAsync(ws.flags, 0, (size_t)R * 16, st);
+  if (ce != cudaSuccess) return (int)ce;
+  int C = chol_group_cluster(Np, R, num_sms);
+  ce = launch_clusters(C, R, GG_SMEM_DOUBLES * 8, st, [&](const cudaLaunchConfig_t& cfg, int c) {
+    return cudaLaunchKernelEx(&cfg, loglik_grad_group_kernel, X, y, N, d, Np, c, P, fit_amp, noise, ws, gw, ll, grad);
+  });
+  return (int)ce;
+}
 // ws: chol_group_ws_bytes(Np, R) bytes.  P [R][1 + fit_amp + d] as for launch_loglik_small.  One launch for all R vectors.
 int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, const double* P, int fit_amp, double noise,
                         int R, int num_sms, void* ws_bytes, double* ll, cudaStream_t st) {
@@ -696,19 +1031,9 @@ int launch_loglik_group(const double* X, const double* y, int N, int d, int Np, 
   cudaError_t ce = cudaMemsetAsync(ws.flags, 0, (size_t)R * 16, st);
   if (ce != cudaSuccess) return (int)ce;
   int C = chol_group_cluster(Np, R, num_sms);
-  for (;;) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(R * C)); cfg.blockDim = dim3(CG_THREADS);
-    cfg.dynamicSmemBytes = CG_SMEM_DOUBLES * 8; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    ce = cudaLaunchKernelEx(&cfg, loglik_group_kernel, X, y, N, d, Np, C, P, fit_amp, noise, ws, ll);
-    if (ce == cudaSuccess || C == 1) break;
-    (void)cudaGetLastError();                // the cluster could not be scheduled: halve it (C = 1 always can)
-    C >>= 1;
-  }
+  ce = launch_clusters(C, R, CG_SMEM_DOUBLES * 8, st, [&](const cudaLaunchConfig_t& cfg, int c) {
+    return cudaLaunchKernelEx(&cfg, loglik_group_kernel, X, y, N, d, Np, c, P, fit_amp, noise, ws, ll);
+  });
 #ifdef APGP_PROF_CG
   if (getenv("APGP_PROF_PRINT")) {
     cudaStreamSynchronize(st);

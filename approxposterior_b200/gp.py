@@ -343,8 +343,10 @@ class GP(object):
         """log-likelihood of ``y`` for every row of ``P`` (george parameter-vector layout) in one
         batched device pass; ``-inf`` where the covariance is not positive definite
         (the quiet=True convention of gpUtils._nll, gpUtils.py:78-79).  ``return_grad`` adds the
-        gradients (rows of zeros where the likelihood is -inf, as grad_log_likelihood(quiet=True)).
-        Leaves the GP's own hyper-parameters untouched."""
+        gradients (rows of zeros where the likelihood is -inf, as grad_log_likelihood(quiet=True)), from the
+        same single launch at every N: the one-restart-per-CTA kernel while the training set fits one CTA's
+        shared memory, the cluster-per-vector kernel with gradients beyond.  Leaves the GP's own
+        hyper-parameters untouched."""
         P = np.ascontiguousarray(np.atleast_2d(np.asarray(P, dtype=np.float64)))
         if P.shape[1] != len(self):
             raise ValueError("dimension mismatch")
@@ -358,8 +360,8 @@ class GP(object):
         st = _lib.check(self._lib.apgp_loglik_batch(self._h, _lib.ptr(Pfull), Pfull.shape[0], Pfull.shape[1], fit_amp,
                                                     self.white_noise, _lib.ptr(ll), _lib.ptr(grad)), "apgp_loglik_batch")
         if st == _lib.APGP_NEEDS_HOST:
-            # batched gradients come from the one-restart-per-CTA kernel only: one factorisation per vector on the
-            # single-GP path (explicit inverse + trace products)
+            # gradients requested under a forced value-only kernel (APGP_LOGLIK_PATH=group|tiled): one factorisation
+            # per vector on the single-GP path (explicit inverse + trace products)
             keep = self.get_parameter_vector()
             for r in range(P.shape[0]):
                 self.set_parameter_vector(P[r])

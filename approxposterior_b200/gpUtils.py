@@ -112,7 +112,8 @@ def optimizeGP(gp, theta, y, seed=None, nGPRestarts=1, method="powell", options=
     Cholesky inside the objective -- so the whole multistart fit is a single launch.
     ``engine="lockstep"`` / larger N: the restarts advance in lock step on the host and every round of
     objective calls is one ``log_likelihood_batch`` launch -- for gradient methods the same launch also
-    returns the gradients (fused one-restart-per-CTA kernel while the training set fits in shared memory).
+    returns the gradients, at every N (one restart per CTA while the training set fits one CTA's shared
+    memory, one thread-block cluster per restart beyond).
     """
     y = np.asarray(y, dtype=np.float64)
     npar = len(gp.get_parameter_vector())

@@ -29,7 +29,8 @@ extern "C" {
 #define APGP_NOT_COMPUTED 2      /* predict/log-likelihood before a successful factorisation */
 #define APGP_NEEDS_REFACTOR 3    /* apgp_append_point: padded buffers are full, call set_training + factorize */
 #define APGP_NEEDS_HOST 4        /* apgp_integrated_time: chain longer than one CTA's shared memory / window beyond 4096 lags;
-                                    apgp_loglik_batch: batched gradients beyond the one-restart-per-CTA kernel */
+                                    apgp_loglik_batch: gradients requested under a forced value-only kernel
+                                    (APGP_LOGLIK_PATH = group | tiled) */
 #define APGP_ERR_ARG (-1)
 #define APGP_ERR_CUDA (-2)
 #define APGP_ERR_NOMEM (-3)
@@ -113,8 +114,12 @@ int apgp_grad_log_likelihood(apgp_handle* h, int fit_amp, double* grad);
  * N(N+1)/2 + N(d+3) + d + 12 doubles fit 220 KB (N <= ~224); beyond, ONE launch of the fused cluster-per-vector kernel
  * (covariance build, look-ahead blocked Cholesky, reductions; csrc/chol_group.cuh), or for at most 8 vectors of
  * N > 1984 the multi-launch tiled sequence.  The first two return exactly -f of apgp_minimize_nll(default_prior=0).
- * APGP_LOGLIK_PATH = small | group | tiled overrides the choice.  Batched gradients need the one-restart-per-CTA kernel:
- * elsewhere the call returns APGP_NEEDS_HOST (use apgp_grad_log_likelihood per vector).
+ * With grad_host: the one-restart-per-CTA kernel while it fits, else ONE launch of the cluster-per-vector kernel with
+ * gradients (the same factorisation, then L^-1, alpha and the trace products; its ll is the value kernel's bit for bit)
+ * for every larger N, few large matrices included.
+ * APGP_LOGLIK_PATH = small | group | tiled overrides the choice of value kernel; group_grad forces the cluster kernel with
+ * gradients at any N (group for value-only calls).  Gradients under a forced group or tiled kernel return
+ * APGP_NEEDS_HOST (use apgp_grad_log_likelihood per vector).
  * Does not disturb the handle's current factorisation. */
 int apgp_loglik_batch(apgp_handle* h, const double* P_host, int R, int P, int fit_amp, double white_noise,
                       double* ll_host, double* grad_host);
@@ -223,8 +228,9 @@ int apgp_debug_group_plan(int N, int num_sms, int d, long long Q, int requested,
 /* kernel of the handle's last predict call with variances: 0 none yet, 1 few-query kernel, 2 one-tile DMMA kernel (also
  * the fallback when the cooperative grouped launch does not fit), 3 grouped DMMA kernel, 4 grouped int8 kernel */
 int apgp_debug_last_var_path(const apgp_handle* h, int* path);
-/* kernel of the handle's last apgp_loglik_batch call: 0 none yet, 1 one restart per CTA, 2 one cluster per restart,
- * 3 multi-launch tiled sequence */
+/* kernel of the handle's last apgp_loglik_batch call: 0 none yet, 1 one restart per CTA (with or without gradients),
+ * 2 one cluster per restart, 3 multi-launch tiled sequence, 4 one cluster per restart with gradients (every batched
+ * gradient call above the one-CTA class; a call that returned APGP_NEEDS_HOST leaves the previous value) */
 int apgp_debug_last_loglik_path(const apgp_handle* h, int* path);
 /* the int8 engine's operands as the kernel reads them (host outputs, each may be NULL): linv_i8 the digit planes of
  * amp * L^-1 (nblk (nblk + 1) / 2 * 28672 bytes, nblk = Npad / 64), rowscale the Npad row scales 2^(ex_i - 38) (0 for
